@@ -22,6 +22,11 @@ writes for the same input (tests/golden/fullsize.json) before anything is timed.
 
 `--impl reference` times the reference's own CPU tools (oracle/_ref, built from the unmodified
 sources; else the oracle port) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the device-resident path returned in its last timed step, the
+forward and the inverse output of every block, as DIR/<workload>_<block>_{forward,inverse}.npy
+(float32, 48 MiB in all; a longer block is sampled at fixed, seeded positions).  The inputs come
+from a seeded generator, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import hashlib
@@ -54,6 +59,7 @@ WORKLOADS = {
 }
 C5_BLOCKS = 8
 MULTI = ("C5", "C5S")
+DUMP_BYTES = 48 << 20  # --dump-outputs: all arrays of a run together, as float32
 INVERSE_CLASSES = ("inv_tile_hist", "inv_lf_rank", "inv_walk", "inv_jump", "inv_scan", "inv_place")
 
 
@@ -422,6 +428,24 @@ def device_resident(torch, ctx, blocks, stream, flush, steps, warmup, golden, ag
     return total_ms, fwd_ms, inv_ms, launches, last_f, last_i, checked
 
 
+def dump_outputs(torch, blocks, names, out_dir, per_array):
+    """--dump-outputs: d_mid (forward output) and d_back (inverse output) of every block as float32 .npy files.
+    A block longer than `per_array` bytes is sampled: one byte out of every n // per_array, at an offset inside
+    that stretch drawn from a fixed seed, so that every run of the same arguments reads the same positions."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for b, name in zip(blocks.items, names):
+        n, idx = b["n"], None
+        if n > per_array:
+            stride = n // per_array
+            pos = np.arange(per_array, dtype=np.int64) * stride + np.random.default_rng(0).integers(0, stride, per_array)
+            idx = torch.from_numpy(pos).to(b["d_mid"].device)
+        for what, t in (("forward", b["d_mid"]), ("inverse", b["d_back"])):
+            np.save(out / f"{name}_{what}.npy", (t if idx is None else t[idx]).float().cpu().numpy())
+    log(f"wrote {2 * len(names)} output array(s) to {out}")
+
+
 def host_buffers(torch, ctx, blocks, steps, warmup):
     """the host-buffer C-ABI calls on pinned memory, one block at a time; returns (wall ms, device ms) per step"""
     copies = {"h2d_ms": 0.0, "d2h_ms": 0.0, "bytes": 0}
@@ -481,8 +505,9 @@ def blocks_call(torch, bwts, items, devices, steps, warmup, golden, pinned=True)
     return sum(w for w, _ in res) / steps, sum(f for _, f in res) / steps, checked
 
 
-def cli_round_trip(data, n):
-    """wall seconds of `bin/mk_bwts in out` and `bin/unbwts out back` on /dev/shm files"""
+def cli_round_trip(data, n, steps):
+    """wall seconds of `bin/mk_bwts in out` and `bin/unbwts out back` on /dev/shm files: the best of `steps`
+    timed round trips after one untimed one"""
     bindir = REPO / "bijective-bwt_b200" / "bin"
     d = "/dev/shm" if os.path.isdir("/dev/shm") else None
     with tempfile.TemporaryDirectory(dir=d) as td:
@@ -490,13 +515,13 @@ def cli_round_trip(data, n):
         src.write_bytes(data)
         env = dict(os.environ)
         best = None
-        for _ in range(2):  # the first run pages the binaries and the CUDA libraries in
+        for i in range(1 + steps):  # the untimed first run pages the binaries and the CUDA libraries in
             t0 = time.perf_counter()
             subprocess.check_call([str(bindir / "mk_bwts"), str(src), str(mid)], env=env)
             t1 = time.perf_counter()
             subprocess.check_call([str(bindir / "unbwts"), str(mid), str(back)], env=env)
             t2 = time.perf_counter()
-            if best is None or t2 - t0 < best[0] + best[1]:
+            if i > 0 and (best is None or t2 - t0 < best[0] + best[1]):
                 best = (t1 - t0, t2 - t1)
         ok = back.read_bytes() == data
         fwd_sha = hashlib.sha256(mid.read_bytes()).hexdigest()
@@ -610,6 +635,10 @@ def run_gpu_arm(args, rank, local_rank, world):
         barrier()
         pipe_ms, _, _ = blocks_call(torch, bwts, blocks.items, [local_rank], args.steps, min(args.warmup, 1), golden)
     clocks = sampler.stop()  # sampled across the timed regions (device-resident and end-to-end)
+    if args.dump_outputs:  # d_mid / d_back still hold the last device-resident step
+        names = [f"{args.workload}_{s_ - seed if args.workload in MULTI else rank}" for _, s_, _, _ in plan]
+        per_array = DUMP_BYTES // 4 // (2 * total_blocks(args.workload, world))
+        dump_outputs(torch, blocks, names, args.dump_outputs, per_array)
     barrier()
 
     # ---- max over ranks (times), sum over ranks (bytes)
@@ -636,7 +665,7 @@ def run_gpu_arm(args, rank, local_rank, world):
             allplan.sort(key=lambda p: p[1])  # file order = block order = seed order
             items = [{"host_in": torch.frombuffer(bytearray(d), dtype=torch.uint8), "n": p[2], "golden": p[3]}
                      for p, d in zip(allplan, make_inputs(allplan))]
-            d_ms, d_fwd_ms, d_checked = blocks_call(torch, bwts, items, list(range(world)), max(1, min(args.steps, 3)), 1, golden)
+            d_ms, d_fwd_ms, d_checked = blocks_call(torch, bwts, items, list(range(world)), args.steps, 1, golden)
             fb = sum(b["n"] for b in items)
             dealer = {"value": fb / MB / (d_ms * 1e-3), "unit": "MB/s", "devices": world, "ms": d_ms, "forward_ms": d_fwd_ms,
                       "bytes": fb, "golden_checked": d_checked,
@@ -699,14 +728,15 @@ def run_gpu_arm(args, rank, local_rank, world):
             ctx.close()  # the tools are separate processes with their own workspace: give the HBM back first
             b0 = blocks.items[0]
             data0 = b0["host_in"].numpy().tobytes()
-            tf, ti, fwd_sha = cli_round_trip(data0, b0["n"])
+            tf, ti, fwd_sha = cli_round_trip(data0, b0["n"], args.steps)
             g = golden.get(b0["golden"]) if b0["golden"] else None
             if g and g["n"] == b0["n"]:
                 assert fwd_sha == g["fwd_sha256"], "CLI forward output differs from the reference's"
             line["e2e_cli"] = {"value": b0["n"] / MB / (tf + ti), "unit": "MB/s", "forward_s": tf, "inverse_s": ti,
                                "how": "wall clock of `bin/mk_bwts in mid` + `bin/unbwts mid back` on /dev/shm files: process "
                                       "start, CUDA context, workspace allocation, map_file input, transform, fwrite output "
-                                      "(/root/reference/map_file.c:16-46 -> mk_bwts_sa.c:60, unbwts.c:173); best of 2 runs"}
+                                      f"(map_file.c:16-46 -> mk_bwts_sa.c:60, unbwts.c:173); best of {args.steps} runs "
+                                      "after one untimed run"}
             del data0
         if world == 1 and not args.no_cpu:
             kind = ref_kind()
@@ -735,14 +765,14 @@ def run_gpu_arm(args, rank, local_rank, world):
         ctx = bwts.Context(local_rank)
         mplan = plan_blocks("C5", 0, 1)
         mb = Blocks(torch, dev, mplan)
-        ms_total, mf, mi, _, _, _, mchecked = device_resident(torch, ctx, mb, stream, flush, 2, 1, golden)
-        p_ms, _, pchecked = blocks_call(torch, bwts, mb.items, [local_rank], 2, 1, golden)
+        ms_total, mf, mi, _, _, _, mchecked = device_resident(torch, ctx, mb, stream, flush, args.steps, 1, golden)
+        p_ms, _, pchecked = blocks_call(torch, bwts, mb.items, [local_rank], args.steps, 1, golden)
         line["multi_block"] = {
             "workload": WORKLOADS["C5"][3] + ", all 8 blocks on this one GPU",
-            "value": mb.bytes / MB / (ms_total / 2 * 1e-3), "unit": "MB/s", "forward_ms": mf, "inverse_ms": mi,
+            "value": mb.bytes / MB / (ms_total / args.steps * 1e-3), "unit": "MB/s", "forward_ms": mf, "inverse_ms": mi,
             "e2e_value": mb.bytes / MB / (p_ms * 1e-3), "golden_checked": sorted(set(mchecked) | set(pchecked)),
-            "how": "value: device-resident, CUDA events, 1 warm-up + 2 steps; e2e_value: bwts_b200_*_blocks pipeline on "
-                   "pinned host buffers, host clock"}
+            "how": f"value: device-resident, CUDA events, 1 warm-up + {args.steps} steps; e2e_value: bwts_b200_*_blocks "
+                   "pipeline on pinned host buffers, host clock"}
     if rank == 0:
         emit_json(line)
     ctx.close()
@@ -766,7 +796,13 @@ def main():
     ap.add_argument("--no-multi-block", dest="multi_block", action="store_false",
                     help="N = 1: skip the C5-on-one-GPU leg")
     ap.add_argument("--tune", action="append", default=[], help="key:value for bwts_b200_tune (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the forward and inverse outputs of the last timed step to DIR/*.npy (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm; --impl reference has none to write")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -675,7 +675,10 @@ def test_timings_use_the_reference_phase_labels(gen, tmp_path):
     assert p.returncode == 0, p.stderr
     pat = re.compile(r"^([A-Z][A-Za-z ]+) time (\d+\.\d{3})$")
     labels = [m.group(1) for m in (pat.match(ln) for ln in p.stderr.splitlines()) if m]
-    want = ["Suffix sort", "Compute ISA", "Fix sort order", "Generate BWTS", "Write BWTS"]
+    stored = json.loads((Path(__file__).parent / "golden" / "reference_checks.json").read_text())["timed"]
+    assert (stored["kind"], stored["seed"], stored["n"]) == ("dna", 77, len(x)) and helpers.sha256(x) == stored["input_sha256"]
+    want = stored["labels"]
+    assert helpers.sha256(dst.read_bytes()) == stored["fwd_sha256"], "differs from the reference's output"
     ref_timed = helpers.REF_DIR / "mk_bwts_timed"
     if ref_timed.exists():
         r = subprocess.run([str(ref_timed), str(src), str(tmp_path / "ref_out")], capture_output=True, text=True)
