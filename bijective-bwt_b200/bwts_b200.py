@@ -26,6 +26,9 @@ EXPORTS = [
     "bwts_b200_inverse_device", "bwts_b200_get_stats", "bwts_b200_class_name", "bwts_b200_set_profile",
     "bwts_b200_strerror", "bwts_b200_last_cuda_error", "bwts_b200_version", "bwts_b200_tune",
     "bwts_b200_divsufsort", "bwts_b200_phase_name",
+    "bwts_b200_bwt_forward", "bwts_b200_bwt_inverse", "bwts_b200_bwt_forward_host", "bwts_b200_bwt_inverse_host",
+    "bwts_b200_bwt_forward_device", "bwts_b200_bwt_inverse_device", "bwts_b200_bwt_forward_blocks",
+    "bwts_b200_bwt_inverse_blocks",
 ]
 
 
@@ -91,6 +94,14 @@ def lib():
     L.bwts_b200_version.restype = ctypes.c_char_p
     L.bwts_b200_tune.argtypes = [ci, cl]
     L.bwts_b200_divsufsort.argtypes = [vp, vp, ci, ci]
+    L.bwts_b200_bwt_forward.argtypes = [vp, cl, vp, vp, ci]
+    L.bwts_b200_bwt_inverse.argtypes = [vp, cl, cl, vp, ci]
+    L.bwts_b200_bwt_forward_host.argtypes = [vp, vp, cl, vp, vp]
+    L.bwts_b200_bwt_inverse_host.argtypes = [vp, vp, cl, cl, vp]
+    L.bwts_b200_bwt_forward_device.argtypes = [vp, vp, cl, vp, vp, vp]
+    L.bwts_b200_bwt_inverse_device.argtypes = [vp, vp, cl, cl, vp, vp]
+    L.bwts_b200_bwt_forward_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
+    L.bwts_b200_bwt_inverse_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
     _lib = L
     return L
 
@@ -159,6 +170,67 @@ def blocks_ptr(direction, in_ptr, length, block_len, out_ptr, devices=(0,)):
     _check(fn(in_ptr, length, block_len, out_ptr, devs, len(devices)), "bwts_b200_*_blocks")
 
 
+def bwt_forward(data, device=0):
+    """bwts_b200_bwt_forward: classic BWT of `data` -> (bytes, primary index), host buffers."""
+    src = _as_u8(data)
+    out = np.empty(len(src), dtype=np.uint8)
+    primary = ctypes.c_long(-1)
+    _check(lib().bwts_b200_bwt_forward(src.ctypes.data if len(src) else None, len(src),
+                                       out.ctypes.data if len(src) else None, ctypes.byref(primary), device),
+           "bwts_b200_bwt_forward")
+    return out.tobytes(), primary.value
+
+
+def bwt_inverse(data, primary, device=0):
+    """bwts_b200_bwt_inverse: inverse classic BWT of (`data`, `primary`) -> bytes, host buffers."""
+    src = _as_u8(data)
+    out = np.empty(len(src), dtype=np.uint8)
+    _check(lib().bwts_b200_bwt_inverse(src.ctypes.data if len(src) else None, len(src), primary,
+                                       out.ctypes.data if len(src) else None, device), "bwts_b200_bwt_inverse")
+    return out.tobytes()
+
+
+def _nblocks(length, block_len):
+    return 1 if block_len <= 0 or block_len >= length else -(-length // block_len)
+
+
+def bwt_forward_blocks(data, block_len, devices=(0,)):
+    """bwts_b200_bwt_forward_blocks -> (bytes, [primary index of each block])"""
+    src = _as_u8(data)
+    out = np.empty(len(src), dtype=np.uint8)
+    primary = np.full(_nblocks(len(src), block_len), -1, dtype=np.int64)
+    devs = (ctypes.c_int * len(devices))(*devices)
+    _check(lib().bwts_b200_bwt_forward_blocks(src.ctypes.data, len(src), block_len, out.ctypes.data,
+                                              primary.ctypes.data, devs, len(devices)), "bwts_b200_bwt_forward_blocks")
+    return out.tobytes(), primary.tolist()
+
+
+def bwt_inverse_blocks(data, block_len, primary, devices=(0,)):
+    """bwts_b200_bwt_inverse_blocks: `primary` holds one index per block"""
+    src = _as_u8(data)
+    out = np.empty(len(src), dtype=np.uint8)
+    idx = np.ascontiguousarray(primary, dtype=np.int64)
+    if len(idx) != _nblocks(len(src), block_len):
+        raise ValueError(f"{len(idx)} primary indices for {_nblocks(len(src), block_len)} blocks")
+    devs = (ctypes.c_int * len(devices))(*devices)
+    _check(lib().bwts_b200_bwt_inverse_blocks(src.ctypes.data, len(src), block_len, idx.ctypes.data,
+                                              out.ctypes.data, devs, len(devices)), "bwts_b200_bwt_inverse_blocks")
+    return out.tobytes()
+
+
+def bwt_blocks_ptr(direction, in_ptr, length, block_len, out_ptr, primary, devices=(0,)):
+    """bwts_b200_bwt_{forward,inverse}_blocks on raw host pointers; `primary`: int64 array, one per block
+    (written by the forward, read by the inverse)"""
+    fn = lib().bwts_b200_bwt_inverse_blocks if direction else lib().bwts_b200_bwt_forward_blocks
+    assert primary.dtype == np.int64 and primary.flags.c_contiguous and len(primary) == _nblocks(length, block_len)
+    devs = (ctypes.c_int * len(devices))(*devices)
+    if direction:
+        rc = fn(in_ptr, length, block_len, primary.ctypes.data, out_ptr, devs, len(devices))
+    else:
+        rc = fn(in_ptr, length, block_len, out_ptr, primary.ctypes.data, devs, len(devices))
+    _check(rc, "bwts_b200_bwt_*_blocks")
+
+
 def suffix_array(data, device=0):
     """bwts_b200_divsufsort: suffix array (int32) of `data`."""
     src = _as_u8(data)
@@ -220,12 +292,46 @@ class Context:
         self.inverse_host_ptr(src.ctypes.data, len(src), out.ctypes.data)
         return out.tobytes()
 
+    def bwt_forward_host_ptr(self, in_ptr, length, out_ptr):
+        """classic BWT on host addresses; returns the primary index"""
+        primary = ctypes.c_long(-1)
+        _check(lib().bwts_b200_bwt_forward_host(self._h, in_ptr, length, out_ptr, ctypes.byref(primary)),
+               "bwts_b200_bwt_forward_host")
+        return primary.value
+
+    def bwt_inverse_host_ptr(self, in_ptr, length, primary, out_ptr):
+        _check(lib().bwts_b200_bwt_inverse_host(self._h, in_ptr, length, primary, out_ptr), "bwts_b200_bwt_inverse_host")
+
+    def bwt_forward_host(self, data):
+        """-> (bytes, primary index)"""
+        src = _as_u8(data)
+        out = np.empty(len(src), dtype=np.uint8)
+        primary = self.bwt_forward_host_ptr(src.ctypes.data, len(src), out.ctypes.data)
+        return out.tobytes(), primary
+
+    def bwt_inverse_host(self, data, primary):
+        src = _as_u8(data)
+        out = np.empty(len(src), dtype=np.uint8)
+        self.bwt_inverse_host_ptr(src.ctypes.data, len(src), primary, out.ctypes.data)
+        return out.tobytes()
+
     # device-resident buffers (device addresses, e.g. torch cuda tensors' data_ptr())
     def forward_device(self, d_in, length, d_out, stream=None):
         _check(lib().bwts_b200_forward_device(self._h, d_in, length, d_out, stream), "bwts_b200_forward_device")
 
     def inverse_device(self, d_in, length, d_out, stream=None):
         _check(lib().bwts_b200_inverse_device(self._h, d_in, length, d_out, stream), "bwts_b200_inverse_device")
+
+    def bwt_forward_device(self, d_in, length, d_out, stream=None):
+        """classic BWT on device addresses; returns the primary index"""
+        primary = ctypes.c_long(-1)
+        _check(lib().bwts_b200_bwt_forward_device(self._h, d_in, length, d_out, ctypes.byref(primary), stream),
+               "bwts_b200_bwt_forward_device")
+        return primary.value
+
+    def bwt_inverse_device(self, d_in, length, primary, d_out, stream=None):
+        _check(lib().bwts_b200_bwt_inverse_device(self._h, d_in, length, primary, d_out, stream),
+               "bwts_b200_bwt_inverse_device")
 
     def stats(self):
         s = Stats()

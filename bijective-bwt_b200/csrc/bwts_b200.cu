@@ -317,9 +317,11 @@ enum FwdMode {
     FWD_BWTS = 0,        // forward BWTS into d_out
     FWD_SA = 1,          // suffix array into d_sa (successor i+1, end of text smallest)
     FWD_LYNDON = 2,      // suffix sort, then factor-start flags (prefix minima of the ISA) into d_out
-    FWD_BWTS_FLAGS = 3   // forward BWTS, factor-start flags already in d_out (after FWD_LYNDON)
+    FWD_BWTS_FLAGS = 3,  // forward BWTS, factor-start flags already in d_out (after FWD_LYNDON)
+    FWD_BWT = 4          // classic BWT into d_out: rotations of the one factor [0, n), *primary = rank[0]
 };
-static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 *d_sa, int mode, cudaStream_t st)
+static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 *d_sa, int mode, cudaStream_t st,
+                        long *primary = nullptr)
 {
     const int linear = (mode == FWD_SA || mode == FWD_LYNDON);
     int rc = arena_reserve(ctx, workspace_bytes(n));
@@ -386,6 +388,11 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
 
     if (mode == FWD_BWTS_FLAGS) {
         CK(cudaMemcpyAsync(flags, d_out, n, cudaMemcpyDeviceToDevice, st));
+    } else if (mode == FWD_BWT) {
+        // no Lyndon boundaries: the factor table is {0, n}; nothing below assumes a factor is Lyndon or primitive
+        // (the cyclic successor is taken mod the factor length, ties that survive are equal rotations)
+        CK(cudaMemsetAsync(flags, 0, n, st));
+        LAUNCH(KC_FACTORS, 0, k_one_factor, 1, 1, n, FS, flags, small);
     } else if (!linear) {
         // -- Lyndon boundaries
         u32 chunk = g_tune_chunk > 0 ? (u32)g_tune_chunk : max(512u, cdiv(n, 1u << 21));
@@ -457,7 +464,7 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             }
         }
     }
-    if (!linear) {
+    if (!linear && mode != FWD_BWT) {
         // -- factor table
         LAUNCH(KC_FACTORS, 1.0 * n, k_flag_count, ntl, 256, flags, n, tilecnt);
         LAUNCH(KC_FACTORS, 8.0 * ntl, k_scan_excl_u32_block, 1, 1024, tilecnt, tilecnt, ntl, small + 0);
@@ -872,6 +879,11 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             }
         }
         LAUNCH(KC_EMIT, 10.0 * F, k_emit_heads, cdiv(F, 256), 256, dT, FS, F, rank, d_out);
+        if (mode == FWD_BWT) {  // the row of rotation 0: ties are ranked in text order, so rotation 0 leads its own
+            rc = readback(ctx, st, rank, 4);
+            if (rc) return rc;
+            *primary = (long)ctx->h_small[0];
+        }
     } else if (mode == FWD_SA) {
         LAUNCH(KC_EMIT, 8.0 * n, k_emit_sa, cdiv(n, 256), 256, rank, n, d_sa);
     } else {
@@ -889,8 +901,10 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
 // ---- inverse -----------------------------------------------------------------------------------
 // One attempt with the splitter hash h.  budget_k: step budget (in units of 1024 steps) of the
 // fallback walks over cycles without splitters, 0 = unbounded; *over is set when it ran out.
+// bwt_out != nullptr: classic inverse BWT from row `primary` into bwt_out; d_out then receives the
+// BWTS layout, which the attempt rotates into bwt_out with its own sublist records (k_bwt_locate).
 static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cudaStream_t st, SplHash h, u32 budget_k,
-                           bool *over)
+                           bool *over, u8 *bwt_out = nullptr, u32 primary = 0)
 {
     *over = false;
     const u32 shift = h.shift;
@@ -910,7 +924,7 @@ static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, c
     uint2 *cyc = arena_take<uint2>(ctx, n);
     u32 *tilecnt = arena_take<u32>(ctx, max(nst, nsc) + 1);
     // [0] ns, [2] reached, [4] unreached handled, [5] fallback steps / 1024, [6] cycles, [8] scan total,
-    // [10] deficient blocks, [12] budget exhausted, [64..320] C
+    // [10] deficient blocks, [12] budget exhausted, [16..18] classic BWT (d, L, off) of the primary, [64..320] C
     u32 *small = arena_take<u32>(ctx, 512);
     if (!tilehist || !chunksum || !prev || (!staged && !sid) || !len_at_min || !off || !cyc || !tilecnt || !small)
         return BWTS_B200_EINTERNAL;
@@ -1055,13 +1069,19 @@ static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, c
     if (rc) return rc;
     if (g_tune_nomark) return 0;                            // timing experiment, the output is not checked
     if (ctx->h_small[8] != n) return BWTS_B200_EINTERNAL;  // cycle lengths must add up to n
+    if (bwt_out) {
+        u32 *loc = small + 16;
+        LAUNCH(KC_INV_PLACE, 0, k_bwt_locate, 1, 1, prev, h, primary, sid, blkoff, srec, off, loc);
+        LAUNCH(KC_INV_PLACE, 2.0 * n, k_bwt_rotate, cdiv(cdiv(n, 16), 256), 256, d_out, n, loc, bwt_out);
+    }
     ctx->stats.splitters = ns;
     ctx->stats.unreached = ctx->h_small[4];
     ctx->stats.factors = ctx->h_small[6];
     return 0;
 }
 
-static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cudaStream_t st)
+// primary >= 0: classic inverse BWT (the BWTS layout goes to an n-byte scratch S in the workspace first)
+static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cudaStream_t st, long primary = -1)
 {
     int rc = arena_reserve(ctx, workspace_bytes(n));
     if (rc) return rc;
@@ -1086,7 +1106,13 @@ static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cuda
         const u32 budget_k = (a == 3) ? 0u : (u32)bk64;
         bool over = false;
         ctx->stats.inverse_attempts++;
-        rc = inverse_attempt(ctx, dB, n, d_out, st, SplHash{muls[a], shift}, budget_k, &over);
+        if (primary >= 0) {
+            u8 *S = arena_take<u8>(ctx, n);
+            if (!S) return BWTS_B200_EINTERNAL;
+            rc = inverse_attempt(ctx, dB, n, S, st, SplHash{muls[a], shift}, budget_k, &over, d_out, (u32)primary);
+        } else {
+            rc = inverse_attempt(ctx, dB, n, d_out, st, SplHash{muls[a], shift}, budget_k, &over);
+        }
         if (rc || !over) return rc;
         if (shift < 30) {
             // denser splitters if ~(80 + slot) bytes per sublist fit behind the per-element arrays (~33 n)
@@ -1095,7 +1121,7 @@ static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cuda
             u64 slot2 = (4ull << (32 - s2)) & ~31ull;
             if (slot2 < 32) slot2 = 32;
             if (slot2 > INV_SLOT_MAX) slot2 = INV_SLOT_MAX;
-            const u64 need = 34ull * n + ns2 * (80 + slot2) * 5 / 4 + (ctx->io_in ? 2 * (u64)ctx->io_bytes : 0) + (16u << 20);
+            const u64 need = (primary >= 0 ? 35ull : 34ull) * n + ns2 * (80 + slot2) * 5 / 4 + (ctx->io_in ? 2 * (u64)ctx->io_bytes : 0) + (16u << 20);
             if (need <= ctx->arena_bytes) shift = s2;
         }
     }
@@ -1182,10 +1208,35 @@ static int check_len(const void *in, long len, void *out)
     return 0;
 }
 
-static int run_device(bwts_b200_ctx *ctx, int direction, const void *d_in, long len, void *d_out, void *stream)
+// What a call computes.  The classic BWT ops take a primary index: the forward writes it, the inverse reads it.
+enum Op { OP_FORWARD = 0, OP_INVERSE = 1, OP_BWT_FORWARD = 2, OP_BWT_INVERSE = 3 };
+static inline int op_direction(int op) { return op & 1; }  // stats.direction: 0 forward, 1 inverse
+
+static int check_primary(int op, long len, const long *primary)
+{
+    if (op < OP_BWT_FORWARD) return 0;
+    if (!primary) return BWTS_B200_EINVAL;
+    if (op == OP_BWT_INVERSE && (*primary < 0 || *primary >= len)) return BWTS_B200_EINVAL;
+    return 0;
+}
+
+static int run_core(bwts_b200_ctx *ctx, int op, const u8 *d_in, u32 n, u8 *d_out, long *primary, cudaStream_t st)
+{
+    switch (op) {
+    case OP_FORWARD: return forward_core(ctx, d_in, n, d_out, nullptr, FWD_BWTS, st);
+    case OP_INVERSE: return inverse_core(ctx, d_in, n, d_out, st);
+    case OP_BWT_FORWARD: return forward_core(ctx, d_in, n, d_out, nullptr, FWD_BWT, st, primary);
+    case OP_BWT_INVERSE: return inverse_core(ctx, d_in, n, d_out, st, *primary);
+    }
+    return BWTS_B200_EINVAL;
+}
+
+static int run_device(bwts_b200_ctx *ctx, int op, const void *d_in, long len, void *d_out, void *stream,
+                      long *primary = nullptr)
 {
     if (!ctx) return BWTS_B200_EINVAL;
     int rc = check_len(d_in, len, d_out);
+    if (!rc) rc = check_primary(op, len, primary);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
@@ -1201,9 +1252,8 @@ static int run_device(bwts_b200_ctx *ctx, int direction, const void *d_in, long 
         d_in = ctx->arena;
         ctx->io_in = ctx->arena;  // tells the cores to skip the I/O region of the arena
     }
-    stats_begin(ctx, len, direction, st);
-    rc = direction == 0 ? forward_core(ctx, (const u8 *)d_in, (u32)len, (u8 *)d_out, nullptr, FWD_BWTS, st)
-                        : inverse_core(ctx, (const u8 *)d_in, (u32)len, (u8 *)d_out, st);
+    stats_begin(ctx, len, op_direction(op), st);
+    rc = run_core(ctx, op, (const u8 *)d_in, (u32)len, (u8 *)d_out, primary, st);
     ctx->io_in = nullptr;
     if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
     stats_end(ctx, st);
@@ -1214,11 +1264,21 @@ static int run_device(bwts_b200_ctx *ctx, int direction, const void *d_in, long 
 
 extern "C" int bwts_b200_forward_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, void *stream)
 {
-    return run_device(ctx, 0, d_in, len, d_out, stream);
+    return run_device(ctx, OP_FORWARD, d_in, len, d_out, stream);
 }
 extern "C" int bwts_b200_inverse_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, void *stream)
 {
-    return run_device(ctx, 1, d_in, len, d_out, stream);
+    return run_device(ctx, OP_INVERSE, d_in, len, d_out, stream);
+}
+extern "C" int bwts_b200_bwt_forward_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, long *primary,
+                                            void *stream)
+{
+    return run_device(ctx, OP_BWT_FORWARD, d_in, len, d_out, stream, primary);
+}
+extern "C" int bwts_b200_bwt_inverse_device(bwts_b200_ctx *ctx, const void *d_in, long len, long primary, void *d_out,
+                                            void *stream)
+{
+    return run_device(ctx, OP_BWT_INVERSE, d_in, len, d_out, stream, &primary);
 }
 
 #define MAX_DEV 64
@@ -1242,10 +1302,12 @@ static bwts_b200_ctx *create_default_ctx(int device)
     return ctx;
 }
 
-static int run_host(bwts_b200_ctx *ctx, int direction, const unsigned char *in, long len, unsigned char *out)
+static int run_host(bwts_b200_ctx *ctx, int op, const unsigned char *in, long len, unsigned char *out,
+                    long *primary = nullptr)
 {
     if (!ctx) return BWTS_B200_EINVAL;
     int rc = check_len(in, len, out);
+    if (!rc) rc = check_primary(op, len, primary);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     // workspace first (it may have to be re-allocated), then the two I/O buffers in its first bytes
@@ -1260,9 +1322,8 @@ static int run_host(bwts_b200_ctx *ctx, int direction, const unsigned char *in, 
     rc = stage_h2d(ctx, d_in, in, (size_t)len, st);
     if (rc) return rc;
     ctx->io_in = d_in;  // tells the cores to skip the I/O region of the arena
-    stats_begin(ctx, len, direction, st);
-    rc = direction == 0 ? forward_core(ctx, d_in, (u32)len, d_out, nullptr, FWD_BWTS, st)
-                        : inverse_core(ctx, d_in, (u32)len, d_out, st);
+    stats_begin(ctx, len, op_direction(op), st);
+    rc = run_core(ctx, op, d_in, (u32)len, d_out, primary, st);
     ctx->io_in = nullptr;
     if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
     stats_end(ctx, st);
@@ -1278,18 +1339,30 @@ static int run_host(bwts_b200_ctx *ctx, int direction, const unsigned char *in, 
 
 extern "C" int bwts_b200_forward_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, unsigned char *out)
 {
-    return run_host(ctx, 0, in, len, out);
+    return run_host(ctx, OP_FORWARD, in, len, out);
 }
 extern "C" int bwts_b200_inverse_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, unsigned char *out)
 {
-    return run_host(ctx, 1, in, len, out);
+    return run_host(ctx, OP_INVERSE, in, len, out);
+}
+extern "C" int bwts_b200_bwt_forward_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, unsigned char *out,
+                                          long *primary)
+{
+    return run_host(ctx, OP_BWT_FORWARD, in, len, out, primary);
+}
+extern "C" int bwts_b200_bwt_inverse_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, long primary,
+                                          unsigned char *out)
+{
+    return run_host(ctx, OP_BWT_INVERSE, in, len, out, &primary);
 }
 
 // ---- one-call entry points ---------------------------------------------------------------------------
 
-static int with_default_ctx(int device, int direction, const unsigned char *in, long len, unsigned char *out)
+static int with_default_ctx(int device, int op, const unsigned char *in, long len, unsigned char *out,
+                            long *primary = nullptr)
 {
     int rc = check_len(in, len, out);
+    if (!rc) rc = check_primary(op, len, primary);
     if (rc) return rc;
     const int ndev = bwts_b200_device_count();
     if (ndev == 0) return BWTS_B200_ENODEV;
@@ -1297,16 +1370,24 @@ static int with_default_ctx(int device, int direction, const unsigned char *in, 
     std::lock_guard<std::mutex> lock(g_dev_mutex[device]);
     if (!g_dev_ctx[device]) g_dev_ctx[device] = create_default_ctx(device);
     if (!g_dev_ctx[device]) return BWTS_B200_ENODEV;
-    return run_host(g_dev_ctx[device], direction, in, len, out);
+    return run_host(g_dev_ctx[device], op, in, len, out, primary);
 }
 
 extern "C" int bwts_b200_forward(const unsigned char *in, long len, unsigned char *out, int device)
 {
-    return with_default_ctx(device, 0, in, len, out);
+    return with_default_ctx(device, OP_FORWARD, in, len, out);
 }
 extern "C" int bwts_b200_inverse(const unsigned char *in, long len, unsigned char *out, int device)
 {
-    return with_default_ctx(device, 1, in, len, out);
+    return with_default_ctx(device, OP_INVERSE, in, len, out);
+}
+extern "C" int bwts_b200_bwt_forward(const unsigned char *in, long len, unsigned char *out, long *primary, int device)
+{
+    return with_default_ctx(device, OP_BWT_FORWARD, in, len, out, primary);
+}
+extern "C" int bwts_b200_bwt_inverse(const unsigned char *in, long len, long primary, unsigned char *out, int device)
+{
+    return with_default_ctx(device, OP_BWT_INVERSE, in, len, out, &primary);
 }
 
 // ---- independent blocks: per device a three-stage pipeline ------------------------------------------
@@ -1456,9 +1537,10 @@ static int stage_d2h(bwts_b200_ctx *ctx, u8 *dst, const u8 *d_src, size_t len, c
 
 static long g_tune_pipeline = 0;  // 1 = no overlap between blocks on one device
 
-// all blocks b = first, first + stride, ... < nblocks on device `dev`
-static int run_blocks_on_device(int direction, const u8 *in, long len, long block_len, u8 *out, int dev, long first,
-                                long stride, long nblocks)
+// all blocks b = first, first + stride, ... < nblocks on device `dev`; primary[b]: block b's primary index
+// (classic BWT ops only, else nullptr)
+static int run_blocks_on_device(int op, const u8 *in, long len, long block_len, u8 *out, long *primary, int dev,
+                                long first, long stride, long nblocks)
 {
     std::vector<long> mine;
     for (long b = first; b < nblocks; b += stride) mine.push_back(b);
@@ -1476,7 +1558,8 @@ static int run_blocks_on_device(int direction, const u8 *in, long len, long bloc
     if (g_tune_pipeline == 1 || mine.size() == 1) {
         int rc = 0;
         for (size_t i = 0; i < mine.size() && rc == 0; i++)
-            rc = run_host(ctx, direction, in + blk_off(mine[i]), blk_len(mine[i]), out + blk_off(mine[i]));
+            rc = run_host(ctx, op, in + blk_off(mine[i]), blk_len(mine[i]), out + blk_off(mine[i]),
+                          primary ? primary + mine[i] : nullptr);
         return rc;
     }
 
@@ -1561,7 +1644,8 @@ static int run_blocks_on_device(int direction, const u8 *in, long len, long bloc
                 int r = 0;
                 if (cudaStreamWaitEvent(st, ev_loaded[i & 1], 0) != cudaSuccess) r = BWTS_B200_ECUDA;
                 const double t0 = since();
-                if (r == 0) r = run_device(ctx, direction, d_in[i & 1], blk_len(b), d_out[i & 1], nullptr);
+                if (r == 0)
+                    r = run_device(ctx, op, d_in[i & 1], blk_len(b), d_out[i & 1], nullptr, primary ? primary + b : nullptr);
                 if (dbg) fprintf(stderr, "[pipe dev %d] block %zu: waited until %.2f, transform %.2f ms (device %.2f)\n", dev, i, t0, since() - t0, ctx->stats.total_ms);
                 if (r) fail(r);
             }
@@ -1579,12 +1663,16 @@ static int run_blocks_on_device(int direction, const u8 *in, long len, long bloc
     return rc;
 }
 
-static int run_blocks(int direction, const unsigned char *in, long len, long block_len, unsigned char *out,
+static int run_blocks(int op, const unsigned char *in, long len, long block_len, unsigned char *out, long *primary,
                       const int *devices, int ndev)
 {
     if (!in || !out || len <= 0 || ndev < 1) return BWTS_B200_EINVAL;
     if (block_len <= 0 || block_len > len) block_len = len;
     if (block_len > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
+    if (op >= OP_BWT_FORWARD && !primary) return BWTS_B200_EINVAL;
+    if (op == OP_BWT_INVERSE)  // every block's index against that block's length, before any work
+        for (long b = 0, off = 0; off < len; b++, off += block_len)
+            if (primary[b] < 0 || primary[b] >= (len - off < block_len ? len - off : block_len)) return BWTS_B200_EINVAL;
     const int have = bwts_b200_device_count();
     if (have == 0) return BWTS_B200_ENODEV;
     std::vector<int> dev(ndev);
@@ -1597,7 +1685,7 @@ static int run_blocks(int direction, const unsigned char *in, long len, long blo
     std::vector<std::thread> workers;
     for (int w = 0; w < ndev; w++)
         workers.emplace_back([&, w]() {
-            status[w] = run_blocks_on_device(direction, in, len, block_len, out, dev[w], w, ndev, nblocks);
+            status[w] = run_blocks_on_device(op, in, len, block_len, out, primary, dev[w], w, ndev, nblocks);
         });
     for (std::thread &t : workers) t.join();
     for (int w = 0; w < ndev; w++)
@@ -1608,12 +1696,23 @@ static int run_blocks(int direction, const unsigned char *in, long len, long blo
 extern "C" int bwts_b200_forward_blocks(const unsigned char *in, long len, long block_len, unsigned char *out,
                                         const int *devices, int ndev)
 {
-    return run_blocks(0, in, len, block_len, out, devices, ndev);
+    return run_blocks(OP_FORWARD, in, len, block_len, out, nullptr, devices, ndev);
 }
 extern "C" int bwts_b200_inverse_blocks(const unsigned char *in, long len, long block_len, unsigned char *out,
                                         const int *devices, int ndev)
 {
-    return run_blocks(1, in, len, block_len, out, devices, ndev);
+    return run_blocks(OP_INVERSE, in, len, block_len, out, nullptr, devices, ndev);
+}
+extern "C" int bwts_b200_bwt_forward_blocks(const unsigned char *in, long len, long block_len, unsigned char *out,
+                                            long *primary, const int *devices, int ndev)
+{
+    return run_blocks(OP_BWT_FORWARD, in, len, block_len, out, primary, devices, ndev);
+}
+extern "C" int bwts_b200_bwt_inverse_blocks(const unsigned char *in, long len, long block_len, const long *primary,
+                                            unsigned char *out, const int *devices, int ndev)
+{
+    // read only: the inverse never writes through it
+    return run_blocks(OP_BWT_INVERSE, in, len, block_len, out, (long *)primary, devices, ndev);
 }
 
 // ---- suffix array behind libdivsufsort's seam ------------------------------------------------------

@@ -1549,3 +1549,13 @@ __global__ void k_set_u32(u32 *p, const u32 *idx_src, u32 value)
 {
     p[*idx_src] = value;  // FS[F] = n
 }
+
+// classic BWT: the whole text is one factor [0, n) (F = small[0] = 1); its head is the only flagged
+// position (flags zeroed by the host), so k_emit leaves out[rank[0]] to k_emit_heads
+__global__ void k_one_factor(u32 n, u32 *__restrict__ FS, u8 *__restrict__ flags, u32 *__restrict__ small)
+{
+    FS[0] = 0;
+    FS[1] = n;
+    flags[0] = 1;
+    small[0] = 1;
+}

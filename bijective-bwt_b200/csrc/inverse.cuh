@@ -591,6 +591,62 @@ __global__ void __launch_bounds__(256) k_inv_place_copy(const u8 *__restrict__ s
     }
 }
 
+// ---- classic inverse BWT: out[n-1-j] = B[LF^j(primary)] ------------------------------------------
+// The BWTS layout S (above) holds the cycle c of `primary` as S[n-1-off(c)-d(i)] = B[i], and d grows by
+// one per prev-step (mod L), so the classic output is that window of L bytes rotated to start at
+// d(primary) and repeated (once when the input came from the forward: then L = n):
+//     out[n-1-j] = S[n-1-off - ((d(primary) + j) mod L)]
+// One thread finds (d(primary), L, off): it walks prev from primary to the first splitter p, t steps,
+// where d(p) = A of the sublist p starts; a cycle without splitters brings the walk back to primary
+// (t = L), and the walk's own minimum gives d as in k_inv_self_walk.  loc = (d, L, off).
+__global__ void k_bwt_locate(const u32 *__restrict__ prev, SplHash h, u32 primary, const u32 *__restrict__ sid,
+                             const u32 *__restrict__ blkoff, const uint4 *__restrict__ srec,
+                             const u32 *__restrict__ off, u32 *__restrict__ loc)
+{
+    u32 j = primary, t = 0, mn = primary, mstep = 0;
+    while (!is_splitter(j, h)) {
+        j = prev[j];
+        t++;
+        if (j == primary) break;
+        if (j < mn) { mn = j; mstep = t; }
+    }
+    if (is_splitter(j, h)) {
+        const uint4 r = srec[sid ? sid[j] : sid_of(blkoff, j, h)];  // (A, L, off); t < L
+        loc[0] = r.x >= t ? r.x - t : r.x + r.y - t;
+        loc[1] = r.y;
+        loc[2] = r.z;
+    } else {
+        loc[0] = mstep == 0 ? 0 : t - mstep;
+        loc[1] = t;
+        loc[2] = off[mn];
+    }
+}
+
+// 16 output bytes per thread: the source runs forward through the window [n - off - L, n - off) and wraps
+__global__ void __launch_bounds__(256) k_bwt_rotate(const u8 *__restrict__ S, u32 n, const u32 *__restrict__ loc,
+                                                    u8 *__restrict__ out)
+{
+    const u64 q0 = ((u64)blockIdx.x * blockDim.x + threadIdx.x) * 16;
+    if (q0 >= n) return;
+    const u32 d = __ldg(loc), L = __ldg(loc + 1), base = n - __ldg(loc + 2) - L;
+    // out[q] = S[base + g(q)], g(q) = L-1 - ((d + n-1-q) mod L), and g(q+1) = g(q) + 1 mod L
+    u32 g = L - 1 - (u32)(((u64)d + (n - 1 - (u32)q0)) % L);
+    u8 v[16];
+#pragma unroll
+    for (int e = 0; e < 16; e++) {
+        v[e] = (q0 + e < n) ? S[base + g] : 0;
+        if (++g == L) g = 0;
+    }
+    u8 *dst = out + q0;
+    if (q0 + 16 <= n && ((uintptr_t)dst & 15) == 0) {
+        uint4 w;
+        memcpy(&w, v, 16);
+        *(uint4 *)dst = w;
+    } else {
+        for (int e = 0; e < 16 && q0 + e < n; e++) dst[e] = v[e];
+    }
+}
+
 // the elements beyond offset slot of their sublist: a second walk from cont[s]
 __global__ void __launch_bounds__(128) k_inv_walk_tail(const u32 *__restrict__ prev, u32 n, SplHash shift,
                                                        const u32 *__restrict__ wlen, const u32 *__restrict__ cont,

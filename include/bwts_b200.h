@@ -12,6 +12,8 @@
  *   bwts_b200_inverse   replaces  unbwts.c:31-86          (counts, scan, LF map, cycle walk)
  *   bwts_b200_*_blocks  additive: independent fixed-size blocks dealt over several GPUs
  *                       (the reference transforms the whole file as one block).
+ *   bwts_b200_bwt_*     additive: the classic Burrows-Wheeler transform with a primary index
+ *                       and its inverse, on the same kernels (see the section below).
  *
  * Byte layout is the reference's: `len` raw input bytes in, exactly `len` raw bytes
  * out, no header, no primary index, no terminator (mk_bwts_sa.c:60, unbwts.c:173).
@@ -87,6 +89,44 @@ int bwts_b200_inverse_host(bwts_b200_ctx *ctx, const unsigned char *in, long len
  * reads a few counters back per doubling round).                                      */
 int bwts_b200_forward_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, void *stream);
 int bwts_b200_inverse_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, void *stream);
+
+/* ---- classic Burrows-Wheeler transform with a primary index ------------------------ */
+/* The index-carrying counterpart of BWTS (Gil & Scott), as in bzip2-style block sorting.
+ * Bytes compare as unsigned char; n = len, 1 <= len <= BWTS_B200_MAX_LEN.
+ *
+ * Forward: the rows are the n cyclic rotations of T, sorted; rows that tie (only when T = u^k)
+ * are ordered by start position.  out[r] = T[(s_r - 1) mod n], s_r the start of row r, and
+ * *primary = the row of rotation 0 = the number of rotations strictly smaller than T.
+ * So a Lyndon word T gives the BWTS output and *primary == 0, every rotation of T gives the
+ * same out, and out[*primary] == T[n-1].
+ *
+ * Inverse: out[n-1-j] = in[LF^j(primary)] for j = 0..n-1, LF the stable LF map
+ * (C[c] + occ(c, i), unbwts.c:50-52).  For a pair made by the forward this is T again, and
+ * for a row r other than the primary it is rotation s_r of T.  Any other pair still has a
+ * defined result (the LF cycle through `primary`, written repeatedly): the inverse fails on
+ * bad arguments only, never because of the content.
+ *
+ * Arguments: a NULL `primary`, or a `primary` outside [0, len), is BWTS_B200_EINVAL; the
+ * *_blocks inverse checks every block's index against that block's length before any work.
+ * Block layout and devices are those of the BWTS *_blocks calls, with one primary index per
+ * block.  Statistics: a forward reports factors = 1, longest_factor = n, lyndon_fallback = 0;
+ * an inverse reports its cycles in `factors` and books the final rotation of the cycle layout
+ * into the output (one n-byte copy) to phase 4, "Place bytes".  The workspace is that of the
+ * BWTS call of the same length.                                                         */
+int bwts_b200_bwt_forward(const unsigned char *in, long len, unsigned char *out, long *primary, int device);
+int bwts_b200_bwt_inverse(const unsigned char *in, long len, long primary, unsigned char *out, int device);
+int bwts_b200_bwt_forward_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, unsigned char *out,
+                               long *primary);
+int bwts_b200_bwt_inverse_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, long primary,
+                               unsigned char *out);
+int bwts_b200_bwt_forward_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, long *primary,
+                                 void *stream);
+int bwts_b200_bwt_inverse_device(bwts_b200_ctx *ctx, const void *d_in, long len, long primary, void *d_out,
+                                 void *stream);
+int bwts_b200_bwt_forward_blocks(const unsigned char *in, long len, long block_len, unsigned char *out,
+                                 long *primary /* one per block */, const int *devices, int ndev);
+int bwts_b200_bwt_inverse_blocks(const unsigned char *in, long len, long block_len, const long *primary,
+                                 unsigned char *out, const int *devices, int ndev);
 
 /* ---- introspection --------------------------------------------------------------- */
 
