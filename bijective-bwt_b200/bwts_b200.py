@@ -29,6 +29,9 @@ EXPORTS = [
     "bwts_b200_bwt_forward", "bwts_b200_bwt_inverse", "bwts_b200_bwt_forward_host", "bwts_b200_bwt_inverse_host",
     "bwts_b200_bwt_forward_device", "bwts_b200_bwt_inverse_device", "bwts_b200_bwt_forward_blocks",
     "bwts_b200_bwt_inverse_blocks",
+    "bwts_b200_divbwt", "bwts_b200_inverse_bw_transform", "bwts_b200_divbwt_forward_host",
+    "bwts_b200_divbwt_inverse_host", "bwts_b200_divbwt_forward_device", "bwts_b200_divbwt_inverse_device",
+    "bwts_b200_divbwt_forward_blocks", "bwts_b200_divbwt_inverse_blocks",
 ]
 
 
@@ -102,6 +105,14 @@ def lib():
     L.bwts_b200_bwt_inverse_device.argtypes = [vp, vp, cl, cl, vp, vp]
     L.bwts_b200_bwt_forward_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
     L.bwts_b200_bwt_inverse_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
+    L.bwts_b200_divbwt.argtypes = [vp, vp, vp, ci, ci]
+    L.bwts_b200_inverse_bw_transform.argtypes = [vp, vp, vp, ci, ci, ci]
+    L.bwts_b200_divbwt_forward_host.argtypes = [vp, vp, cl, vp, vp]
+    L.bwts_b200_divbwt_inverse_host.argtypes = [vp, vp, cl, cl, vp]
+    L.bwts_b200_divbwt_forward_device.argtypes = [vp, vp, cl, vp, vp, vp]
+    L.bwts_b200_divbwt_inverse_device.argtypes = [vp, vp, cl, cl, vp, vp]
+    L.bwts_b200_divbwt_forward_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
+    L.bwts_b200_divbwt_inverse_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
     _lib = L
     return L
 
@@ -231,6 +242,54 @@ def bwt_blocks_ptr(direction, in_ptr, length, block_len, out_ptr, primary, devic
     _check(rc, "bwts_b200_bwt_*_blocks")
 
 
+def divbwt_forward(data, device=0):
+    """bwts_b200_divbwt (libdivsufsort's divbwt): end-of-text BWT of `data` -> (bytes, primary), primary in [1, n]
+    (0 for empty data)"""
+    src = _as_u8(data)
+    if len(src) == 0:
+        return b"", 0
+    out = np.empty(len(src), dtype=np.uint8)
+    rc = lib().bwts_b200_divbwt(src.ctypes.data, out.ctypes.data, None, len(src), device)
+    if rc < 0:
+        raise BwtsError(rc, "bwts_b200_divbwt")
+    return out.tobytes(), rc
+
+
+def divbwt_inverse(data, primary, device=0):
+    """bwts_b200_inverse_bw_transform (libdivsufsort's inverse_bw_transform) of (`data`, `primary`) -> bytes"""
+    src = _as_u8(data)
+    if len(src) == 0 and primary == 0:
+        return b""
+    out = np.empty(len(src), dtype=np.uint8)
+    _check(lib().bwts_b200_inverse_bw_transform(src.ctypes.data, out.ctypes.data, None, len(src), primary, device),
+           "bwts_b200_inverse_bw_transform")
+    return out.tobytes()
+
+
+def divbwt_forward_blocks(data, block_len, devices=(0,)):
+    """bwts_b200_divbwt_forward_blocks -> (bytes, [primary of each block])"""
+    src = _as_u8(data)
+    out = np.empty(len(src), dtype=np.uint8)
+    primary = np.full(_nblocks(len(src), block_len), -1, dtype=np.int64)
+    devs = (ctypes.c_int * len(devices))(*devices)
+    _check(lib().bwts_b200_divbwt_forward_blocks(src.ctypes.data, len(src), block_len, out.ctypes.data,
+                                                 primary.ctypes.data, devs, len(devices)), "bwts_b200_divbwt_forward_blocks")
+    return out.tobytes(), primary.tolist()
+
+
+def divbwt_inverse_blocks(data, block_len, primary, devices=(0,)):
+    """bwts_b200_divbwt_inverse_blocks: `primary` holds one index per block"""
+    src = _as_u8(data)
+    out = np.empty(len(src), dtype=np.uint8)
+    idx = np.ascontiguousarray(primary, dtype=np.int64)
+    if len(idx) != _nblocks(len(src), block_len):
+        raise ValueError(f"{len(idx)} primary indices for {_nblocks(len(src), block_len)} blocks")
+    devs = (ctypes.c_int * len(devices))(*devices)
+    _check(lib().bwts_b200_divbwt_inverse_blocks(src.ctypes.data, len(src), block_len, idx.ctypes.data,
+                                                 out.ctypes.data, devs, len(devices)), "bwts_b200_divbwt_inverse_blocks")
+    return out.tobytes()
+
+
 def suffix_array(data, device=0):
     """bwts_b200_divsufsort: suffix array (int32) of `data`."""
     src = _as_u8(data)
@@ -315,6 +374,22 @@ class Context:
         self.bwt_inverse_host_ptr(src.ctypes.data, len(src), primary, out.ctypes.data)
         return out.tobytes()
 
+    def divbwt_forward_host(self, data):
+        """libdivsufsort's divbwt -> (bytes, primary)"""
+        src = _as_u8(data)
+        out = np.empty(len(src), dtype=np.uint8)
+        primary = ctypes.c_long(-1)
+        _check(lib().bwts_b200_divbwt_forward_host(self._h, src.ctypes.data, len(src), out.ctypes.data,
+                                                   ctypes.byref(primary)), "bwts_b200_divbwt_forward_host")
+        return out.tobytes(), primary.value
+
+    def divbwt_inverse_host(self, data, primary):
+        src = _as_u8(data)
+        out = np.empty(len(src), dtype=np.uint8)
+        _check(lib().bwts_b200_divbwt_inverse_host(self._h, src.ctypes.data, len(src), primary, out.ctypes.data),
+               "bwts_b200_divbwt_inverse_host")
+        return out.tobytes()
+
     # device-resident buffers (device addresses, e.g. torch cuda tensors' data_ptr())
     def forward_device(self, d_in, length, d_out, stream=None):
         _check(lib().bwts_b200_forward_device(self._h, d_in, length, d_out, stream), "bwts_b200_forward_device")
@@ -332,6 +407,17 @@ class Context:
     def bwt_inverse_device(self, d_in, length, primary, d_out, stream=None):
         _check(lib().bwts_b200_bwt_inverse_device(self._h, d_in, length, primary, d_out, stream),
                "bwts_b200_bwt_inverse_device")
+
+    def divbwt_forward_device(self, d_in, length, d_out, stream=None):
+        """divbwt on device addresses; returns the primary"""
+        primary = ctypes.c_long(-1)
+        _check(lib().bwts_b200_divbwt_forward_device(self._h, d_in, length, d_out, ctypes.byref(primary), stream),
+               "bwts_b200_divbwt_forward_device")
+        return primary.value
+
+    def divbwt_inverse_device(self, d_in, length, primary, d_out, stream=None):
+        _check(lib().bwts_b200_divbwt_inverse_device(self._h, d_in, length, primary, d_out, stream),
+               "bwts_b200_divbwt_inverse_device")
 
     def stats(self):
         s = Stats()

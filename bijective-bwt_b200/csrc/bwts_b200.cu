@@ -318,12 +318,13 @@ enum FwdMode {
     FWD_SA = 1,          // suffix array into d_sa (successor i+1, end of text smallest)
     FWD_LYNDON = 2,      // suffix sort, then factor-start flags (prefix minima of the ISA) into d_out
     FWD_BWTS_FLAGS = 3,  // forward BWTS, factor-start flags already in d_out (after FWD_LYNDON)
-    FWD_BWT = 4          // classic BWT into d_out: rotations of the one factor [0, n), *primary = rank[0]
+    FWD_BWT = 4,         // classic BWT into d_out: rotations of the one factor [0, n), *primary = rank[0]
+    FWD_DIVBWT = 5       // libdivsufsort's divbwt into d_out: the FWD_SA sort, bytes at shifted rows, *primary = rank[0] + 1
 };
 static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 *d_sa, int mode, cudaStream_t st,
                         long *primary = nullptr)
 {
-    const int linear = (mode == FWD_SA || mode == FWD_LYNDON);
+    const int linear = (mode == FWD_SA || mode == FWD_LYNDON || mode == FWD_DIVBWT);
     int rc = arena_reserve(ctx, workspace_bytes(n));
     if (rc) return rc;
     ctx->arena_used = 0;
@@ -834,7 +835,8 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
     // -- emit
     ctx->phase = PH_EMIT;
     (void)PH_SORT0;
-    if (!linear) {
+    const bool div = mode == FWD_DIVBWT;  // the byte emit below with emit_slot<true> (forward.cuh)
+    if (!linear || div) {
         const bool emit_binned = g_tune_emit >= 2 || (g_tune_emit == 0 && n >= (512u << 20));
         if (emit_binned && kb >= 8 && g_tune_emit != 3) {
             // one packed word per element, binned by rank region, then scattered through L2: the bin pass reads
@@ -851,7 +853,8 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); }
             r__.phase = ctx->phase; ctx->recs.push_back(r__);
             CK(cudaGetLastError());
-            LAUNCH(KC_EMIT, 5.0 * n, k_scatter_packed, cdiv(cdiv(n, 4), 256), 256, packed, n, shift, d_out);
+            if (div) LAUNCH(KC_EMIT, 5.0 * n, k_scatter_packed<true>, cdiv(cdiv(n, 4), 256), 256, packed, n, shift, d_out, rank);
+            else LAUNCH(KC_EMIT, 5.0 * n, k_scatter_packed, cdiv(cdiv(n, 4), 256), 256, packed, n, shift, d_out);
         } else if (emit_binned && kb >= 8) {
             // (round 1, tune 9 = 3) (rank, byte) pairs as two u32 streams binned by rank region
             u32 *val = (u32 *)sb.k[0], *bin_pos = val + (((size_t)n + 3) & ~(size_t)3);
@@ -868,17 +871,29 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); }
             r__.phase = ctx->phase; ctx->recs.push_back(r__);
             CK(cudaGetLastError());
-            LAUNCH(KC_EMIT, 9.0 * n, k_scatter_bytes, cdiv(cdiv(n, 4), 256), 256, bin_pos, bin_val, n, d_out);
+            if (div) LAUNCH(KC_EMIT, 9.0 * n, k_scatter_bytes<true>, cdiv(cdiv(n, 4), 256), 256, bin_pos, bin_val, n, d_out, rank);
+            else LAUNCH(KC_EMIT, 9.0 * n, k_scatter_bytes, cdiv(cdiv(n, 4), 256), 256, bin_pos, bin_val, n, d_out);
         } else {
             // rank windows of 64 Mi slots: the scatter target of one launch stays resident in the 126 MB L2
             const u32 win = (g_tune_emitwin >= 16 && g_tune_emitwin <= 1024) ? (u32)g_tune_emitwin << 20 : 64u << 20;
             for (u64 lo = 0; lo < n; lo += win) {
                 const u32 hi = (u32)min((u64)n, lo + win);
-                LAUNCH(KC_EMIT, (lo == 0 ? 7.0 : 4.0) * n, k_emit, cdiv(cdiv(n, 4), 256), 256, dT, n, rank, flags, d_out,
-                       (u32)lo, hi);
+                if (div)
+                    LAUNCH(KC_EMIT, (lo == 0 ? 7.0 : 4.0) * n, k_emit<true>, cdiv(cdiv(n, 4), 256), 256, dT, n, rank, flags,
+                           d_out, (u32)lo, hi);
+                else
+                    LAUNCH(KC_EMIT, (lo == 0 ? 7.0 : 4.0) * n, k_emit, cdiv(cdiv(n, 4), 256), 256, dT, n, rank, flags, d_out,
+                           (u32)lo, hi);
             }
         }
-        LAUNCH(KC_EMIT, 10.0 * F, k_emit_heads, cdiv(F, 256), 256, dT, FS, F, rank, d_out);
+        if (div) {  // slot 0 after every lane has stored; the row of suffix 0 is where the end of text stood
+            LAUNCH(KC_EMIT, 0, k_divbwt_first, 1, 1, dT, n, d_out);
+            rc = readback(ctx, st, rank, 4);
+            if (rc) return rc;
+            *primary = (long)ctx->h_small[0] + 1;
+        } else {
+            LAUNCH(KC_EMIT, 10.0 * F, k_emit_heads, cdiv(F, 256), 256, dT, FS, F, rank, d_out);
+        }
         if (mode == FWD_BWT) {  // the row of rotation 0: ties are ranked in text order, so rotation 0 leads its own
             rc = readback(ctx, st, rank, 4);
             if (rc) return rc;
@@ -903,8 +918,10 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
 // fallback walks over cycles without splitters, 0 = unbounded; *over is set when it ran out.
 // bwt_out != nullptr: classic inverse BWT from row `primary` into bwt_out; d_out then receives the
 // BWTS layout, which the attempt rotates into bwt_out with its own sublist records (k_bwt_locate).
+// div_primary > 0 (with bwt_out, primary 0): libdivsufsort's inverse_bw_transform, the same path over the
+// map prev_s of k_inv_lf_rank<true>.
 static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cudaStream_t st, SplHash h, u32 budget_k,
-                           bool *over, u8 *bwt_out = nullptr, u32 primary = 0)
+                           bool *over, u8 *bwt_out = nullptr, u32 primary = 0, u32 div_primary = 0)
 {
     *over = false;
     const u32 shift = h.shift;
@@ -924,7 +941,8 @@ static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, c
     uint2 *cyc = arena_take<uint2>(ctx, n);
     u32 *tilecnt = arena_take<u32>(ctx, max(nst, nsc) + 1);
     // [0] ns, [2] reached, [4] unreached handled, [5] fallback steps / 1024, [6] cycles, [8] scan total,
-    // [10] deficient blocks, [12] budget exhausted, [16..18] classic BWT (d, L, off) of the primary, [64..320] C
+    // [10] deficient blocks, [12] budget exhausted, [16..18] classic BWT (d, L, off) of the primary,
+    // [20] divbwt: the byte of the element whose prev_s is 0, [64..320] C
     u32 *small = arena_take<u32>(ctx, 512);
     if (!tilehist || !chunksum || !prev || (!staged && !sid) || !len_at_min || !off || !cyc || !tilecnt || !small)
         return BWTS_B200_EINTERNAL;
@@ -938,7 +956,10 @@ static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, c
     LAUNCH(KC_INV_SCAN, 0, k_inv_chunk_scan, 1, 256, chunksum, nchunks, Ctab);
     LAUNCH(KC_INV_SCAN, 2048.0 * ntiles, k_inv_tile_base, nchunks, 256, tilehist, ntiles, chunksum);
     ctx->phase = 1;
-    LAUNCH(KC_INV_LF, 5.0 * n, k_inv_lf_rank, ntiles, INV_NT, dB, n, tilehist, prev);
+    if (div_primary)
+        LAUNCH(KC_INV_LF, 5.0 * n, k_inv_lf_rank<true>, ntiles, INV_NT, dB, n, tilehist, prev, div_primary, Ctab, small + 20);
+    else
+        LAUNCH(KC_INV_LF, 5.0 * n, k_inv_lf_rank, ntiles, INV_NT, dB, n, tilehist, prev);
 
     // -- splitters
     ctx->phase = 2;
@@ -1071,7 +1092,10 @@ static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, c
     if (ctx->h_small[8] != n) return BWTS_B200_EINTERNAL;  // cycle lengths must add up to n
     if (bwt_out) {
         u32 *loc = small + 16;
-        LAUNCH(KC_INV_PLACE, 0, k_bwt_locate, 1, 1, prev, h, primary, sid, blkoff, srec, off, loc);
+        if (div_primary)
+            LAUNCH(KC_INV_PLACE, 0, k_bwt_locate<true>, 1, 1, prev, h, primary, sid, blkoff, srec, off, loc, d_out, n, small + 20);
+        else
+            LAUNCH(KC_INV_PLACE, 0, k_bwt_locate, 1, 1, prev, h, primary, sid, blkoff, srec, off, loc);
         LAUNCH(KC_INV_PLACE, 2.0 * n, k_bwt_rotate, cdiv(cdiv(n, 16), 256), 256, d_out, n, loc, bwt_out);
     }
     ctx->stats.splitters = ns;
@@ -1080,8 +1104,10 @@ static int inverse_attempt(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, c
     return 0;
 }
 
-// primary >= 0: classic inverse BWT (the BWTS layout goes to an n-byte scratch S in the workspace first)
-static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cudaStream_t st, long primary = -1)
+// primary >= 0: classic inverse BWT (the BWTS layout goes to an n-byte scratch S in the workspace first);
+// div: libdivsufsort's inverse_bw_transform with primary in [1, n], the classic path from row 0
+static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cudaStream_t st, long primary = -1,
+                        bool div = false)
 {
     int rc = arena_reserve(ctx, workspace_bytes(n));
     if (rc) return rc;
@@ -1109,7 +1135,8 @@ static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cuda
         if (primary >= 0) {
             u8 *S = arena_take<u8>(ctx, n);
             if (!S) return BWTS_B200_EINTERNAL;
-            rc = inverse_attempt(ctx, dB, n, S, st, SplHash{muls[a], shift}, budget_k, &over, d_out, (u32)primary);
+            rc = inverse_attempt(ctx, dB, n, S, st, SplHash{muls[a], shift}, budget_k, &over, d_out, div ? 0u : (u32)primary,
+                                 div ? (u32)primary : 0u);
         } else {
             rc = inverse_attempt(ctx, dB, n, d_out, st, SplHash{muls[a], shift}, budget_k, &over);
         }
@@ -1208,8 +1235,9 @@ static int check_len(const void *in, long len, void *out)
     return 0;
 }
 
-// What a call computes.  The classic BWT ops take a primary index: the forward writes it, the inverse reads it.
-enum Op { OP_FORWARD = 0, OP_INVERSE = 1, OP_BWT_FORWARD = 2, OP_BWT_INVERSE = 3 };
+// What a call computes.  The classic BWT and divbwt ops take a primary index: the forward writes it, the
+// inverse reads it (classic: a row in [0, len); divbwt: where the end of text stood, in [1, len]).
+enum Op { OP_FORWARD = 0, OP_INVERSE = 1, OP_BWT_FORWARD = 2, OP_BWT_INVERSE = 3, OP_DIVBWT_FORWARD = 4, OP_DIVBWT_INVERSE = 5 };
 static inline int op_direction(int op) { return op & 1; }  // stats.direction: 0 forward, 1 inverse
 
 static int check_primary(int op, long len, const long *primary)
@@ -1217,6 +1245,7 @@ static int check_primary(int op, long len, const long *primary)
     if (op < OP_BWT_FORWARD) return 0;
     if (!primary) return BWTS_B200_EINVAL;
     if (op == OP_BWT_INVERSE && (*primary < 0 || *primary >= len)) return BWTS_B200_EINVAL;
+    if (op == OP_DIVBWT_INVERSE && (*primary < 1 || *primary > len)) return BWTS_B200_EINVAL;
     return 0;
 }
 
@@ -1227,6 +1256,8 @@ static int run_core(bwts_b200_ctx *ctx, int op, const u8 *d_in, u32 n, u8 *d_out
     case OP_INVERSE: return inverse_core(ctx, d_in, n, d_out, st);
     case OP_BWT_FORWARD: return forward_core(ctx, d_in, n, d_out, nullptr, FWD_BWT, st, primary);
     case OP_BWT_INVERSE: return inverse_core(ctx, d_in, n, d_out, st, *primary);
+    case OP_DIVBWT_FORWARD: return forward_core(ctx, d_in, n, d_out, nullptr, FWD_DIVBWT, st, primary);
+    case OP_DIVBWT_INVERSE: return inverse_core(ctx, d_in, n, d_out, st, *primary, true);
     }
     return BWTS_B200_EINVAL;
 }
@@ -1279,6 +1310,16 @@ extern "C" int bwts_b200_bwt_inverse_device(bwts_b200_ctx *ctx, const void *d_in
                                             void *stream)
 {
     return run_device(ctx, OP_BWT_INVERSE, d_in, len, d_out, stream, &primary);
+}
+extern "C" int bwts_b200_divbwt_forward_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, long *primary,
+                                               void *stream)
+{
+    return run_device(ctx, OP_DIVBWT_FORWARD, d_in, len, d_out, stream, primary);
+}
+extern "C" int bwts_b200_divbwt_inverse_device(bwts_b200_ctx *ctx, const void *d_in, long len, long primary, void *d_out,
+                                               void *stream)
+{
+    return run_device(ctx, OP_DIVBWT_INVERSE, d_in, len, d_out, stream, &primary);
 }
 
 #define MAX_DEV 64
@@ -1355,6 +1396,16 @@ extern "C" int bwts_b200_bwt_inverse_host(bwts_b200_ctx *ctx, const unsigned cha
 {
     return run_host(ctx, OP_BWT_INVERSE, in, len, out, &primary);
 }
+extern "C" int bwts_b200_divbwt_forward_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, unsigned char *out,
+                                             long *primary)
+{
+    return run_host(ctx, OP_DIVBWT_FORWARD, in, len, out, primary);
+}
+extern "C" int bwts_b200_divbwt_inverse_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, long primary,
+                                             unsigned char *out)
+{
+    return run_host(ctx, OP_DIVBWT_INVERSE, in, len, out, &primary);
+}
 
 // ---- one-call entry points ---------------------------------------------------------------------------
 
@@ -1388,6 +1439,25 @@ extern "C" int bwts_b200_bwt_forward(const unsigned char *in, long len, unsigned
 extern "C" int bwts_b200_bwt_inverse(const unsigned char *in, long len, long primary, unsigned char *out, int device)
 {
     return with_default_ctx(device, OP_BWT_INVERSE, in, len, out, &primary);
+}
+// libdivsufsort's signatures.  A (its temporary array) is never touched; U may be T: the input is on the
+// device before the first output byte comes back.
+extern "C" int bwts_b200_divbwt(const unsigned char *T, unsigned char *U, int *A, int n, int device)
+{
+    (void)A;
+    if (!T || !U || n < 0) return BWTS_B200_EINVAL;
+    if (n == 0) return 0;
+    long primary = 0;
+    const int rc = with_default_ctx(device, OP_DIVBWT_FORWARD, T, n, U, &primary);
+    return rc ? rc : (int)primary;
+}
+extern "C" int bwts_b200_inverse_bw_transform(const unsigned char *T, unsigned char *U, int *A, int n, int idx, int device)
+{
+    (void)A;
+    if (!T || !U || n < 0 || idx < 0 || idx > n || (idx == 0 && n > 0)) return BWTS_B200_EINVAL;
+    if (n == 0) return 0;
+    long primary = idx;
+    return with_default_ctx(device, OP_DIVBWT_INVERSE, T, n, U, &primary);
 }
 
 // ---- independent blocks: per device a three-stage pipeline ------------------------------------------
@@ -1538,7 +1608,7 @@ static int stage_d2h(bwts_b200_ctx *ctx, u8 *dst, const u8 *d_src, size_t len, c
 static long g_tune_pipeline = 0;  // 1 = no overlap between blocks on one device
 
 // all blocks b = first, first + stride, ... < nblocks on device `dev`; primary[b]: block b's primary index
-// (classic BWT ops only, else nullptr)
+// (classic BWT and divbwt ops only, else nullptr)
 static int run_blocks_on_device(int op, const u8 *in, long len, long block_len, u8 *out, long *primary, int dev,
                                 long first, long stride, long nblocks)
 {
@@ -1670,9 +1740,11 @@ static int run_blocks(int op, const unsigned char *in, long len, long block_len,
     if (block_len <= 0 || block_len > len) block_len = len;
     if (block_len > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
     if (op >= OP_BWT_FORWARD && !primary) return BWTS_B200_EINVAL;
-    if (op == OP_BWT_INVERSE)  // every block's index against that block's length, before any work
+    if (op == OP_BWT_INVERSE || op == OP_DIVBWT_INVERSE) {  // every block's index against that block's length, before any work
+        const long lo = op == OP_DIVBWT_INVERSE ? 1 : 0;      // [0, len) for the classic row, [1, len] for divbwt
         for (long b = 0, off = 0; off < len; b++, off += block_len)
-            if (primary[b] < 0 || primary[b] >= (len - off < block_len ? len - off : block_len)) return BWTS_B200_EINVAL;
+            if (primary[b] < lo || primary[b] >= (len - off < block_len ? len - off : block_len) + lo) return BWTS_B200_EINVAL;
+    }
     const int have = bwts_b200_device_count();
     if (have == 0) return BWTS_B200_ENODEV;
     std::vector<int> dev(ndev);
@@ -1713,6 +1785,16 @@ extern "C" int bwts_b200_bwt_inverse_blocks(const unsigned char *in, long len, l
 {
     // read only: the inverse never writes through it
     return run_blocks(OP_BWT_INVERSE, in, len, block_len, out, (long *)primary, devices, ndev);
+}
+extern "C" int bwts_b200_divbwt_forward_blocks(const unsigned char *in, long len, long block_len, unsigned char *out,
+                                               long *primary, const int *devices, int ndev)
+{
+    return run_blocks(OP_DIVBWT_FORWARD, in, len, block_len, out, primary, devices, ndev);
+}
+extern "C" int bwts_b200_divbwt_inverse_blocks(const unsigned char *in, long len, long block_len, const long *primary,
+                                               unsigned char *out, const int *devices, int ndev)
+{
+    return run_blocks(OP_DIVBWT_INVERSE, in, len, block_len, out, (long *)primary, devices, ndev);
 }
 
 // ---- suffix array behind libdivsufsort's seam ------------------------------------------------------

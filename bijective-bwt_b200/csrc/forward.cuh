@@ -1415,33 +1415,47 @@ __global__ void __launch_bounds__(LSR_NT, 2) k_local_sort_cta_radix(const u32 *_
 }
 
 // ---- emit -----------------------------------------------------------------------------------------
+// DIV: libdivsufsort's divbwt after the linear suffix sort.  Row r0 = rank[0] (suffix 0, whose byte
+// would be the end of text) goes to slot 0, where k_divbwt_first writes T[n-1] afterwards; the rows
+// in front of it move up by one.  One store per slot, so no two lanes write the same byte.  Without
+// DIV the slot is the rank itself (BWTS and classic BWT).
+template <bool DIV>
+static __device__ __forceinline__ u32 emit_slot(u32 r, u32 r0)
+{
+    return DIV ? (r == r0 ? 0u : r + (r < r0)) : r;
+}
+
 // out[rank[i]] = T[i-1] for every position that does not start a factor and whose rank lies in
 // [lo, hi).  Large outputs are emitted in rank windows small enough to stay in L2, so the
 // one-byte scatter merges into full sectors there instead of read-modify-writing DRAM.
+// DIV: out[emit_slot(rank[i])] for every position, windows over the slot; flags are not read.
+template <bool DIV = false>
 __global__ void __launch_bounds__(256) k_emit(const u8 *__restrict__ T, u32 n, const u32 *__restrict__ rank,
                                               const u8 *__restrict__ flags, u8 *__restrict__ out, u32 lo, u32 hi)
 {
     const u32 i0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (i0 >= n) return;
+    const u32 r0 = DIV ? __ldg(rank) : 0u;
     if (i0 + 4 <= n && i0 >= 4) {
         // every load is issued before the first store: the ranks, the four flags as one word, and
         // T[i0-1 .. i0+2] out of the aligned words around it (a word that holds a valid byte lies
         // inside the allocation)
         const uint4 r = ldg_stream_u4((const uint4 *)(rank + i0));
-        const u32 fl = *(const u32 *)(flags + i0);
+        const u32 fl = DIV ? 0u : *(const u32 *)(flags + i0);
         const uintptr_t a = (uintptr_t)(T + i0 - 1);
         const u32 *w = (const u32 *)(a & ~(uintptr_t)3);
         const u32 o = (u32)(a & 3);
         const u32 w0 = w[0], w1 = o ? w[1] : 0u;
         const u32 bytes = (u32)((((u64)w1 << 32) | w0) >> (8 * o));
-        const u32 rr[4] = {r.x, r.y, r.z, r.w};
+        const u32 rr[4] = {emit_slot<DIV>(r.x, r0), emit_slot<DIV>(r.y, r0), emit_slot<DIV>(r.z, r0),
+                           emit_slot<DIV>(r.w, r0)};
 #pragma unroll
         for (int q = 0; q < 4; q++)
             if (rr[q] >= lo && rr[q] < hi && !((fl >> (8 * q)) & 0xffu)) out[rr[q]] = (u8)(bytes >> (8 * q));
     } else {
         for (u32 i = i0; i < min(n, i0 + 4); i++) {
-            const u32 r = rank[i];
-            if (r >= lo && r < hi && !flags[i]) out[r] = T[i - 1];
+            const u32 r = emit_slot<DIV>(rank[i], r0);
+            if (r >= lo && r < hi && (DIV || !flags[i])) out[r] = (DIV && i == 0) ? (u8)0 : T[i - 1];
         }
     }
 }
@@ -1458,34 +1472,41 @@ __global__ void __launch_bounds__(256) k_emit_vals(const u8 *__restrict__ T, u32
     for (int q = 0; q < 4; q++)
         if (i0 + q < n) val[i0 + q] = (i0 + q > 0) ? (u32)T[i0 + q - 1] : 0u;
 }
+// DIV: the store goes to emit_slot of the rank, rank0 = &rank[0] (unused otherwise)
+template <bool DIV = false>
 __global__ void __launch_bounds__(256) k_scatter_bytes(const u32 *__restrict__ pos, const u32 *__restrict__ val, u32 n,
-                                                       u8 *__restrict__ out)
+                                                       u8 *__restrict__ out, const u32 *__restrict__ rank0 = nullptr)
 {
     const u32 j0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (j0 >= n) return;
+    const u32 r0 = DIV ? __ldg(rank0) : 0u;
     if (j0 + 4 <= n) {
         const uint4 p = ldg_stream_u4((const uint4 *)(pos + j0));
         const uint4 v = ldg_stream_u4((const uint4 *)(val + j0));
-        out[p.x] = (u8)v.x; out[p.y] = (u8)v.y; out[p.z] = (u8)v.z; out[p.w] = (u8)v.w;
+        out[emit_slot<DIV>(p.x, r0)] = (u8)v.x; out[emit_slot<DIV>(p.y, r0)] = (u8)v.y;
+        out[emit_slot<DIV>(p.z, r0)] = (u8)v.z; out[emit_slot<DIV>(p.w, r0)] = (u8)v.w;
     } else {
-        for (u32 j = j0; j < n; j++) out[pos[j]] = (u8)val[j];
+        for (u32 j = j0; j < n; j++) out[emit_slot<DIV>(pos[j], r0)] = (u8)val[j];
     }
 }
 // packed form of the same (k_onesweep_pass MODE 2): word j of the binned stream belongs to rank bin
 // j >> shift (the bins hold exactly 2^shift ranks each: the ranks are a permutation of 0..n-1)
+template <bool DIV = false>
 __global__ void __launch_bounds__(256) k_scatter_packed(const u32 *__restrict__ packed, u32 n, u32 shift,
-                                                        u8 *__restrict__ out)
+                                                        u8 *__restrict__ out, const u32 *__restrict__ rank0 = nullptr)
 {
     const u32 j0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (j0 >= n) return;
     const u32 mask = (1u << shift) - 1u;
+    const u32 r0 = DIV ? __ldg(rank0) : 0u;
     if (j0 + 4 <= n) {
         const uint4 w = ldg_stream_u4((const uint4 *)(packed + j0));
         const u32 ww[4] = {w.x, w.y, w.z, w.w};
 #pragma unroll
-        for (int q = 0; q < 4; q++) out[(((j0 + q) >> shift) << shift) | (ww[q] & mask)] = (u8)(ww[q] >> shift);
+        for (int q = 0; q < 4; q++)
+            out[emit_slot<DIV>((((j0 + q) >> shift) << shift) | (ww[q] & mask), r0)] = (u8)(ww[q] >> shift);
     } else {
-        for (u32 j = j0; j < n; j++) out[((j >> shift) << shift) | (packed[j] & mask)] = (u8)(packed[j] >> shift);
+        for (u32 j = j0; j < n; j++) out[emit_slot<DIV>(((j >> shift) << shift) | (packed[j] & mask), r0)] = (u8)(packed[j] >> shift);
     }
 }
 // factor heads receive the last byte of their own factor
@@ -1558,4 +1579,10 @@ __global__ void k_one_factor(u32 n, u32 *__restrict__ FS, u8 *__restrict__ flags
     FS[1] = n;
     flags[0] = 1;
     small[0] = 1;
+}
+
+// divbwt: slot 0 holds the last byte of the text (the row of the end of text, "$T", ends with it)
+__global__ void k_divbwt_first(const u8 *__restrict__ T, u32 n, u8 *__restrict__ out)
+{
+    out[0] = T[n - 1];
 }

@@ -109,13 +109,30 @@ __global__ void __launch_bounds__(256) k_inv_tile_base(u32 *__restrict__ tilehis
 }
 
 // ---- stable LF map ------------------------------------------------------------------------------
+// DIV (libdivsufsort's inverse_bw_transform, `primary` in [1, n]): B is the sentinel BWT with its end of
+// text removed, and prev receives the map with that row cut out of the cycle,
+//     p = 1 + LF(i),  prev_s(i) = (p == primary) ? 0 : p - (p > primary),
+// a permutation of [0, n) whatever B and primary are; out[n-1-j] = B[prev_s^j(0)] is the classic walk
+// from row 0.  The placement kernels recover the byte of i from prev[i] through C (byte_of_rank), so
+// block 0 also rewrites Ctab to C'[c] = C[c] + (C[c] < primary): then byte_of_rank(C', prev_s(i)) = B[i]
+// for every prev_s(i) > 0.  The one element with prev_s = 0 gets byte 0 there; its byte c*, the c with
+// C[c] < primary <= C[c+1], goes to *cstar and k_bwt_locate<true> puts it in place.
+template <bool DIV = false>
 __global__ void __launch_bounds__(INV_NT) k_inv_lf_rank(const u8 *__restrict__ B, u32 n,
-                                                        const u32 *__restrict__ tilebase, u32 *__restrict__ prev)
+                                                        const u32 *__restrict__ tilebase, u32 *__restrict__ prev,
+                                                        u32 primary = 0, u32 *__restrict__ Ctab = nullptr,
+                                                        u32 *__restrict__ cstar = nullptr)
 {
     __shared__ __align__(16) u8 s_b[INV_TILE];
     __shared__ u32 s_wcnt[INV_NT / 32][256];
     const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const u32 base = blockIdx.x * INV_TILE;
+    if (DIV && blockIdx.x == 0) {  // block-uniform
+        const u32 c = Ctab[tid], c1 = Ctab[tid + 1];
+        __syncthreads();
+        if (c < primary && primary <= c1) *cstar = tid;
+        Ctab[tid] = c + (c < primary);
+    }
     for (u32 i = tid; i < (INV_NT / 32) * 256; i += INV_NT) ((u32 *)s_wcnt)[i] = 0;
 #pragma unroll
     for (int v = 0; v < 2; v++) {
@@ -164,7 +181,14 @@ __global__ void __launch_bounds__(INV_NT) k_inv_lf_rank(const u8 *__restrict__ B
 #pragma unroll
     for (int j = 0; j < ROUNDS; j++) {
         const u32 o = wo + j * 32 + lane;
-        if (base + o < n) prev[base + o] = wc[s_b[o]] + rnk[j];
+        if (base + o < n) {
+            u32 v = wc[s_b[o]] + rnk[j];
+            if (DIV) {
+                const u32 p = v + 1;
+                v = p == primary ? 0u : p - (p > primary);
+            }
+            prev[base + o] = v;
+        }
     }
 }
 
@@ -599,9 +623,14 @@ __global__ void __launch_bounds__(256) k_inv_place_copy(const u8 *__restrict__ s
 // One thread finds (d(primary), L, off): it walks prev from primary to the first splitter p, t steps,
 // where d(p) = A of the sublist p starts; a cycle without splitters brings the walk back to primary
 // (t = L), and the walk's own minimum gives d as in k_inv_self_walk.  loc = (d, L, off).
+// DIV (primary = 0, prev = prev_s of k_inv_lf_rank<true>): the element whose prev_s is 0 is the last of
+// the cycle of 0 (d = L - 1, and off = 0: no cycle has a smaller index), so its byte sits at
+// S[n - off - L]; that byte is written here from *cstar, before k_bwt_rotate reads the window.
+template <bool DIV = false>
 __global__ void k_bwt_locate(const u32 *__restrict__ prev, SplHash h, u32 primary, const u32 *__restrict__ sid,
                              const u32 *__restrict__ blkoff, const uint4 *__restrict__ srec,
-                             const u32 *__restrict__ off, u32 *__restrict__ loc)
+                             const u32 *__restrict__ off, u32 *__restrict__ loc, u8 *__restrict__ S = nullptr,
+                             u32 n = 0, const u32 *__restrict__ cstar = nullptr)
 {
     u32 j = primary, t = 0, mn = primary, mstep = 0;
     while (!is_splitter(j, h)) {
@@ -620,6 +649,7 @@ __global__ void k_bwt_locate(const u32 *__restrict__ prev, SplHash h, u32 primar
         loc[1] = t;
         loc[2] = off[mn];
     }
+    if (DIV) S[n - loc[2] - loc[1]] = (u8)*cstar;
 }
 
 // 16 output bytes per thread: the source runs forward through the window [n - off - L, n - off) and wraps

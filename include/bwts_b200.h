@@ -14,6 +14,9 @@
  *                       (the reference transforms the whole file as one block).
  *   bwts_b200_bwt_*     additive: the classic Burrows-Wheeler transform with a primary index
  *                       and its inverse, on the same kernels (see the section below).
+ *   bwts_b200_divbwt*, bwts_b200_inverse_bw_transform
+ *                       additive: libdivsufsort's end-of-text BWT (divbwt / inverse_bw_transform),
+ *                       on the same kernels (see the last section).
  *
  * Byte layout is the reference's: `len` raw input bytes in, exactly `len` raw bytes
  * out, no header, no primary index, no terminator (mk_bwts_sa.c:60, unbwts.c:173).
@@ -208,6 +211,51 @@ int bwts_b200_tune(int key, long value);
 /* Same contract as divsufsort(T, SA, n) (/root/reference/mk_bwts_sa.c:48): SA[0..n) =
  * start offsets of the suffixes of T in ascending order; returns 0 or a negative code. */
 int bwts_b200_divsufsort(const unsigned char *T, int *SA, int n, int device);
+
+/* ---- libdivsufsort's BWT: divbwt and inverse_bw_transform ---------------------------- */
+/* The end-of-text ("sentinel") BWT of libdivsufsort, the form FM-index and DNA tools read.
+ * Bytes compare as unsigned char; n = len.  SA is the suffix array of T with the end of text
+ * smaller than every byte (the order of the suffixes of T$, bwts_b200_divsufsort).
+ *
+ * Forward (divbwt): B[r] = T[SA[r] - 1] for SA[r] > 0, r0 the row with SA[r0] == 0,
+ *     U = T[n-1] . B[0..r0) . B[r0+1..n),   primary = r0 + 1, in [1, n].
+ * That is the BWT of T$ with the $ removed, and primary is where the $ stood.  Examples:
+ * banana -> (annbaa, 4), abracadabra -> (ardrcaaaabb, 3), mississippi -> (ipssmpissii, 5),
+ * aaaa -> (aaaa, 4), a -> (a, 1).
+ *
+ * Inverse (inverse_bw_transform): prev the stable LF map over U (C[c] + occ(c, i)), p = 1 + prev[u],
+ *     prev_s[u] = (p == primary) ? 0 : p - (p > primary),   out[n-1-j] = U[prev_s^j(0)], j = 0..n-1.
+ * prev_s is a permutation of [0, n) for every U and every primary in [1, n], so every pair has a
+ * defined result (the cycle through 0, written repeatedly); for a pair made by the forward it is
+ * one n-cycle and the result is T.  The inverse fails on bad arguments only.  (libdivsufsort's
+ * own inverse is defined on the pairs its forward makes; there the two agree.)
+ *
+ * The one-call functions keep libdivsufsort's signatures and argument rules: a NULL T or U,
+ * n < 0, idx < 0, idx > n, or idx == 0 with n > 0 is BWTS_B200_EINVAL; n == 0 returns 0;
+ * U may be T; A (libdivsufsort's temporary array) may be NULL and is never touched.
+ * bwts_b200_divbwt returns primary (> 0) or a negative code, bwts_b200_inverse_bw_transform
+ * 0 or a negative code.  They run on the per-device context of the other one-call functions.
+ *
+ * The context and block calls have the shape of the bwts_b200_bwt_* calls: len bytes, never
+ * aliased, a NULL `primary` or an inverse `primary` outside [1, len] is BWTS_B200_EINVAL, and the
+ * *_blocks inverse checks every block's index against [1, that block's length] before any work.
+ * Statistics: a forward reports factors = 1, longest_factor = n, lyndon_fallback = 0; an inverse
+ * reports its cycles in `factors` (1 for a pair made by the forward) and books the rotation into
+ * the output to phase 4, "Place bytes".  The workspace is that of the BWTS call of the same length. */
+int bwts_b200_divbwt(const unsigned char *T, unsigned char *U, int *A, int n, int device);
+int bwts_b200_inverse_bw_transform(const unsigned char *T, unsigned char *U, int *A, int n, int idx, int device);
+int bwts_b200_divbwt_forward_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, unsigned char *out,
+                                  long *primary);
+int bwts_b200_divbwt_inverse_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, long primary,
+                                  unsigned char *out);
+int bwts_b200_divbwt_forward_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, long *primary,
+                                    void *stream);
+int bwts_b200_divbwt_inverse_device(bwts_b200_ctx *ctx, const void *d_in, long len, long primary, void *d_out,
+                                    void *stream);
+int bwts_b200_divbwt_forward_blocks(const unsigned char *in, long len, long block_len, unsigned char *out,
+                                    long *primary /* one per block */, const int *devices, int ndev);
+int bwts_b200_divbwt_inverse_blocks(const unsigned char *in, long len, long block_len, const long *primary,
+                                    unsigned char *out, const int *devices, int ndev);
 
 #ifdef __cplusplus
 }
