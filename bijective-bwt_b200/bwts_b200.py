@@ -32,6 +32,7 @@ EXPORTS = [
     "bwts_b200_divbwt", "bwts_b200_inverse_bw_transform", "bwts_b200_divbwt_forward_host",
     "bwts_b200_divbwt_inverse_host", "bwts_b200_divbwt_forward_device", "bwts_b200_divbwt_inverse_device",
     "bwts_b200_divbwt_forward_blocks", "bwts_b200_divbwt_inverse_blocks",
+    "bwts_b200_sa_host", "bwts_b200_sa_device", "bwts_b200_sa_lcp_host", "bwts_b200_sa_lcp_device", "bwts_b200_sa_lcp",
 ]
 
 
@@ -113,6 +114,11 @@ def lib():
     L.bwts_b200_divbwt_inverse_device.argtypes = [vp, vp, cl, cl, vp, vp]
     L.bwts_b200_divbwt_forward_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
     L.bwts_b200_divbwt_inverse_blocks.argtypes = [vp, cl, cl, vp, vp, ctypes.POINTER(ci), ci]
+    L.bwts_b200_sa_host.argtypes = [vp, vp, cl, vp]
+    L.bwts_b200_sa_device.argtypes = [vp, vp, cl, vp, vp]
+    L.bwts_b200_sa_lcp_host.argtypes = [vp, vp, cl, vp, vp]
+    L.bwts_b200_sa_lcp_device.argtypes = [vp, vp, cl, vp, vp, vp]
+    L.bwts_b200_sa_lcp.argtypes = [vp, vp, vp, ci, ci]
     _lib = L
     return L
 
@@ -300,6 +306,19 @@ def suffix_array(data, device=0):
     return sa
 
 
+def suffix_array_lcp(data, device=0):
+    """bwts_b200_sa_lcp: (suffix array, LCP array) of `data`, both int32; LCP[r] = lcp of the suffixes SA[r-1] and
+    SA[r], LCP[0] = 0"""
+    src = _as_u8(data)
+    sa = np.empty(len(src), dtype=np.int32)
+    lcp = np.empty(len(src), dtype=np.int32)
+    if len(src) == 0:
+        return sa, lcp
+    _check(lib().bwts_b200_sa_lcp(src.ctypes.data, sa.ctypes.data, lcp.ctypes.data, len(src), device),
+           "bwts_b200_sa_lcp")
+    return sa, lcp
+
+
 class Context:
     """bwts_b200_ctx: reusable device workspace (one per device per host thread)."""
 
@@ -390,6 +409,22 @@ class Context:
                "bwts_b200_divbwt_inverse_host")
         return out.tobytes()
 
+    def sa_host(self, data):
+        """suffix array (int32)"""
+        src = _as_u8(data)
+        sa = np.empty(len(src), dtype=np.int32)
+        _check(lib().bwts_b200_sa_host(self._h, src.ctypes.data, len(src), sa.ctypes.data), "bwts_b200_sa_host")
+        return sa
+
+    def sa_lcp_host(self, data):
+        """-> (suffix array, LCP array), int32"""
+        src = _as_u8(data)
+        sa = np.empty(len(src), dtype=np.int32)
+        lcp = np.empty(len(src), dtype=np.int32)
+        _check(lib().bwts_b200_sa_lcp_host(self._h, src.ctypes.data, len(src), sa.ctypes.data, lcp.ctypes.data),
+               "bwts_b200_sa_lcp_host")
+        return sa, lcp
+
     # device-resident buffers (device addresses, e.g. torch cuda tensors' data_ptr())
     def forward_device(self, d_in, length, d_out, stream=None):
         _check(lib().bwts_b200_forward_device(self._h, d_in, length, d_out, stream), "bwts_b200_forward_device")
@@ -418,6 +453,14 @@ class Context:
     def divbwt_inverse_device(self, d_in, length, primary, d_out, stream=None):
         _check(lib().bwts_b200_divbwt_inverse_device(self._h, d_in, length, primary, d_out, stream),
                "bwts_b200_divbwt_inverse_device")
+
+    def sa_device(self, d_in, length, d_sa, stream=None):
+        """suffix array into d_sa (length int32, 4-byte aligned)"""
+        _check(lib().bwts_b200_sa_device(self._h, d_in, length, d_sa, stream), "bwts_b200_sa_device")
+
+    def sa_lcp_device(self, d_in, length, d_sa, d_lcp, stream=None):
+        """suffix array into d_sa and LCP array into d_lcp (length int32 each, 4-byte aligned)"""
+        _check(lib().bwts_b200_sa_lcp_device(self._h, d_in, length, d_sa, d_lcp, stream), "bwts_b200_sa_lcp_device")
 
     def stats(self):
         s = Stats()

@@ -21,6 +21,7 @@
 #include "common.cuh"
 #include "forward.cuh"
 #include "inverse.cuh"
+#include "lcp.cuh"
 #include "lyndon.cuh"
 #include "radix.cuh"
 #include "scan.cuh"
@@ -58,6 +59,7 @@ static long g_tune_invq = 0;       // inverse staged walk: sublists per warp (0 
 static long g_tune_invmark = 0;    // inverse staged walk marks: 0 = by size (counts per 128 above 256 MiB), 1 = one bit per element, 2 = counts
 static long g_tune_invbudget = 0;  // inverse fallback walks: step budget per attempt (0 = 32 n)
 static long g_tune_nomark = 0;     // TIMING EXPERIMENT ONLY: inverse first walk without visited marks (wrong output when a cycle has no splitter)
+static long g_tune_lcp = 0;        // LCP pairs: 0 = by length through the three tiers, 1 = all from the warp tier on, 2 = all through the multi-CTA tier
 
 static void apply_device_limits()
 {
@@ -312,17 +314,77 @@ static int radix_sort(bwts_b200_ctx *ctx, cudaStream_t st, SortBufs &sb, u32 m, 
     return 0;
 }
 
+// ---- LCP array (lcp.cuh) ------------------------------------------------------------------------
+// After the FWD_SA emit: d_lcp[r] = lcp of the suffixes d_sa[r-1] and d_sa[r].  Scratch, all dead after
+// the sort: P n words (the text-order PLCP array), tiles n / LCP_TILE words, res and the two pair lists
+// n entries each, cnt 10 words: [0..2] open-pair counts, [4..9] three u64 counters of compared bytes
+// (rows, warp tier, the current round), read back with the counts and added to the launches' byte
+// figures.  Booked to kernel class emit and the forward's phase 3 by the caller.
+static int lcp_stage(bwts_b200_ctx *ctx, cudaStream_t st, const u8 *dT, u32 n, const i32 *d_sa, i32 *d_lcp, u32 *P,
+                     u32 *tiles, u32 *res, u64 *listA, u64 *listB, u32 *cnt)
+{
+    const u32 mode = (g_tune_lcp == 1 || g_tune_lcp == 2) ? (u32)g_tune_lcp : 0u;
+    unsigned long long *cmp = (unsigned long long *)(cnt + 4);
+    const auto compared = [&](int k) { return (double)((u64)ctx->h_small[4 + 2 * k] | ((u64)ctx->h_small[5 + 2 * k] << 32)); };
+    CK(cudaMemsetAsync(P, 0, (size_t)n * 4, st));
+    CK(cudaMemsetAsync(cnt, 0, 10 * sizeof(u32), st));
+    // SA 4, B 1 (gather), P 4 (scatter, irreducible rows only: an upper bound), plus the bytes compared
+    LAUNCH(KC_EMIT, 9.0 * n, k_lcp_rows, cdiv(n, 256), 256, dT, n, d_sa, P, listA, cnt, mode, cmp);
+    const size_t rec_rows = ctx->recs.size() - 1;
+    int rc = readback(ctx, st, cnt, 40);
+    if (rc) return rc;
+    ctx->recs[rec_rows].bytes += compared(0);
+    const u32 m2 = ctx->h_small[0];
+    if (m2) {
+        LAUNCH(KC_EMIT, 8.0 * m2, k_lcp_warp, cdiv(m2, 8), 256, dT, n, listA, m2, mode == 0 ? LCP_T1 : 0u,
+               mode == 2 ? 0u : LCP_T2, P, listB, cnt + 1, cmp + 1);
+        const size_t rec_warp = ctx->recs.size() - 1;
+        rc = readback(ctx, st, cnt, 40);
+        if (rc) return rc;
+        ctx->recs[rec_warp].bytes += compared(1);
+        u32 m = ctx->h_small[1];
+        u64 off = mode == 2 ? 0 : LCP_T2;
+        u64 *cur = listB, *nxt = listA;
+        while (m) {
+            // each round covers [off, off + W) of every open pair, W at least 4 x what is behind it, so an
+            // a^n pair of 2^31 bytes takes seven rounds; segments past a pair's mismatch or end return at once
+            const u64 W = max((u64)LCP_SEG * 16, 4 * off);
+            const u32 S = (u32)(W / LCP_SEG);
+            const u64 items = (u64)m * S;
+            const u32 gx = (u32)min(items, (u64)1 << 30), gy = (u32)((items + gx - 1) / gx);
+            CK(cudaMemsetAsync(res, 0xff, (size_t)m * 4, st));
+            CK(cudaMemsetAsync(cnt + 2, 0, 4, st));
+            CK(cudaMemsetAsync(cmp + 2, 0, 8, st));
+            LAUNCH(KC_EMIT, 8.0 * m, k_lcp_span, dim3(gx, gy), 256, dT, n, cur, m, S, (u32)off, res, cmp + 2);
+            const size_t rec_span = ctx->recs.size() - 1;
+            LAUNCH(KC_EMIT, 16.0 * m, k_lcp_span_close, cdiv(m, 256), 256, n, cur, m, off + W, res, P, nxt, cnt + 2);
+            rc = readback(ctx, st, cnt, 40);
+            if (rc) return rc;
+            ctx->recs[rec_span].bytes += compared(2);
+            m = ctx->h_small[2];
+            off += W;
+            u64 *t = cur; cur = nxt; nxt = t;
+        }
+    }
+    const u32 nt = cdiv(n, LCP_TILE);
+    LAUNCH(KC_EMIT, 4.0 * n, k_lcp_tile_max, nt, 256, P, n, tiles);
+    LAUNCH(KC_EMIT, 8.0 * nt, k_lcp_tile_scan, 1, 1024, tiles, nt);
+    LAUNCH(KC_EMIT, 8.0 * n, k_lcp_plcp, nt, 256, P, n, tiles);
+    LAUNCH(KC_EMIT, 12.0 * n, k_lcp_emit, cdiv(n, 256), 256, d_sa, n, P, d_lcp);
+    return 0;
+}
+
 // ---- forward ---------------------------------------------------------------------------------
 enum FwdMode {
     FWD_BWTS = 0,        // forward BWTS into d_out
-    FWD_SA = 1,          // suffix array into d_sa (successor i+1, end of text smallest)
+    FWD_SA = 1,          // suffix array into d_sa (successor i+1, end of text smallest), then the LCP array into d_lcp if given
     FWD_LYNDON = 2,      // suffix sort, then factor-start flags (prefix minima of the ISA) into d_out
     FWD_BWTS_FLAGS = 3,  // forward BWTS, factor-start flags already in d_out (after FWD_LYNDON)
     FWD_BWT = 4,         // classic BWT into d_out: rotations of the one factor [0, n), *primary = rank[0]
     FWD_DIVBWT = 5       // libdivsufsort's divbwt into d_out: the FWD_SA sort, bytes at shifted rows, *primary = rank[0] + 1
 };
 static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 *d_sa, int mode, cudaStream_t st,
-                        long *primary = nullptr)
+                        long *primary = nullptr, i32 *d_lcp = nullptr)
 {
     const int linear = (mode == FWD_SA || mode == FWD_LYNDON || mode == FWD_DIVBWT);
     int rc = arena_reserve(ctx, workspace_bytes(n));
@@ -901,6 +963,10 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
         }
     } else if (mode == FWD_SA) {
         LAUNCH(KC_EMIT, 8.0 * n, k_emit_sa, cdiv(n, 256), 256, rank, n, d_sa);
+        if (d_lcp) {
+            rc = lcp_stage(ctx, st, dT, n, d_sa, d_lcp, sb.v[0], grp, gst, sb.k[0], sb.k[1], small + 128);
+            if (rc) return rc;
+        }
     } else {
         // FWD_LYNDON: rank[] is now the inverse suffix array; factor starts = its strict prefix minima
         const u32 pmt = cdiv(n, PM_TILE);
@@ -1797,40 +1863,137 @@ extern "C" int bwts_b200_divbwt_inverse_blocks(const unsigned char *in, long len
     return run_blocks(OP_DIVBWT_INVERSE, in, len, block_len, out, (long *)primary, devices, ndev);
 }
 
-// ---- suffix array behind libdivsufsort's seam ------------------------------------------------------
-extern "C" int bwts_b200_divsufsort(const unsigned char *T, int *SA, int n, int device)
+// ---- suffix array and LCP array ----------------------------------------------------------------------
+// [a, a + na) and [b, b + nb) share a byte
+static bool spans_overlap(const void *a, size_t na, const void *b, size_t nb)
 {
-    if (!T || !SA || n < 0) return BWTS_B200_EINVAL;
-    if (n == 0) return 0;
-    if ((long)n > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
+    const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+    return x < y + nb && y < x + na;
+}
+// the bwts_b200_bwt_* rules, plus: no two of in, sa and lcp (if wanted) share a byte
+static int check_sa_args(const void *in, long len, const void *sa, const void *lcp, bool want_lcp)
+{
+    if (!in || !sa || (want_lcp && !lcp) || len <= 0) return BWTS_B200_EINVAL;
+    if (len > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
+    const size_t n = (size_t)len;
+    if (spans_overlap(in, n, sa, 4 * n)) return BWTS_B200_EINVAL;
+    if (want_lcp && (spans_overlap(in, n, lcp, 4 * n) || spans_overlap(sa, 4 * n, lcp, 4 * n))) return BWTS_B200_EINVAL;
+    return 0;
+}
+
+static int run_sa_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_sa, void *d_lcp, void *stream,
+                         bool want_lcp)
+{
+    if (!ctx) return BWTS_B200_EINVAL;
+    int rc = check_sa_args(d_in, len, d_sa, d_lcp, want_lcp);
+    if (rc) return rc;
+    if (((uintptr_t)d_sa & 3) || ((uintptr_t)d_lcp & 3)) return BWTS_B200_EINVAL;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    apply_device_limits();
+    ctx->io_in = nullptr;
+    if ((uintptr_t)d_in & 15) {  // as run_device: an unaligned slice is copied to the bottom of the workspace
+        rc = arena_reserve(ctx, workspace_bytes((size_t)len) + 2 * (size_t)len + 1024);
+        if (rc) return rc;
+        ctx->io_bytes = ((size_t)len + 255) & ~(size_t)255;
+        CK(cudaMemcpyAsync(ctx->arena, d_in, (size_t)len, cudaMemcpyDeviceToDevice, st));
+        d_in = ctx->arena;
+        ctx->io_in = ctx->arena;
+    }
+    stats_begin(ctx, len, 0, st);
+    rc = forward_core(ctx, (const u8 *)d_in, (u32)len, nullptr, (i32 *)d_sa, FWD_SA, st, nullptr,
+                      want_lcp ? (i32 *)d_lcp : nullptr);
+    ctx->io_in = nullptr;
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    stats_end(ctx, st);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
+    return 0;
+}
+
+// host buffers: the text, the suffix array and the LCP array (if wanted) in the I/O region in front of the
+// workspace, 1 + 4 + 4 bytes per input byte; arguments already checked
+static int run_sa_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa, int *lcp)
+{
+    CK(cudaSetDevice(ctx->device));
+    const size_t io = ((size_t)len + 255) & ~(size_t)255;
+    const size_t sa_bytes = ((size_t)len * 4 + 255) & ~(size_t)255;
+    const size_t out_bytes = lcp ? 2 * sa_bytes : sa_bytes;
+    int rc = arena_reserve(ctx, workspace_bytes((size_t)len) + io + out_bytes + 1024);
+    if (rc) return rc;
+    // forward_core skips 2 * io_bytes of the arena: the I/O region
+    ctx->io_bytes = ((io + out_bytes + 1) / 2 + 255) & ~(size_t)255;
+    ctx->io_in = nullptr;
+    u8 *d_in = ctx->arena;
+    i32 *d_sa = (i32 *)(ctx->arena + io), *d_lcp = lcp ? (i32 *)(ctx->arena + io + sa_bytes) : nullptr;
+    cudaStream_t st = ctx->own_stream;
+    apply_device_limits();
+    CK(cudaEventRecord(ctx->ev_io0, st));
+    rc = stage_h2d(ctx, d_in, in, (size_t)len, st);
+    if (rc) return rc;
+    ctx->io_in = d_in;
+    stats_begin(ctx, len, 0, st);
+    rc = forward_core(ctx, d_in, (u32)len, nullptr, d_sa, FWD_SA, st, nullptr, d_lcp);
+    ctx->io_in = nullptr;
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    stats_end(ctx, st);
+    rc = stage_d2h(ctx, (u8 *)sa, (const u8 *)d_sa, (size_t)len * 4, st);
+    if (!rc && lcp) rc = stage_d2h(ctx, (u8 *)lcp, (const u8 *)d_lcp, (size_t)len * 4, st);
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->ev_io1, st));
+    CK(cudaStreamSynchronize(st));
+    float t = 0;
+    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
+    if (cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
+    return 0;
+}
+
+extern "C" int bwts_b200_sa_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa)
+{
+    if (!ctx) return BWTS_B200_EINVAL;
+    const int rc = check_sa_args(in, len, sa, nullptr, false);
+    return rc ? rc : run_sa_host(ctx, in, len, sa, nullptr);
+}
+extern "C" int bwts_b200_sa_lcp_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa, int *lcp)
+{
+    if (!ctx) return BWTS_B200_EINVAL;
+    const int rc = check_sa_args(in, len, sa, lcp, true);
+    return rc ? rc : run_sa_host(ctx, in, len, sa, lcp);
+}
+extern "C" int bwts_b200_sa_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_sa, void *stream)
+{
+    return run_sa_device(ctx, d_in, len, d_sa, nullptr, stream, false);
+}
+extern "C" int bwts_b200_sa_lcp_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_sa, void *d_lcp,
+                                       void *stream)
+{
+    return run_sa_device(ctx, d_in, len, d_sa, d_lcp, stream, true);
+}
+
+// the one-call forms, on the per-device context of the other one-call functions; n == 0 returns 0
+static int sa_default_ctx(const unsigned char *T, int *SA, int *LCP, int n, int device)
+{
     const int ndev = bwts_b200_device_count();
     if (ndev == 0) return BWTS_B200_ENODEV;
     if (device < 0 || device >= ndev || device >= MAX_DEV) return BWTS_B200_EINVAL;
     std::lock_guard<std::mutex> lock(g_dev_mutex[device]);
     if (!g_dev_ctx[device]) g_dev_ctx[device] = create_default_ctx(device);
-    bwts_b200_ctx *ctx = g_dev_ctx[device];
-    if (!ctx) return BWTS_B200_ENODEV;
-    CK(cudaSetDevice(device));
-    const size_t io = ((size_t)n + 255) & ~(size_t)255;
-    const size_t sa_bytes = ((size_t)n * 4 + 255) & ~(size_t)255;
-    int rc = arena_reserve(ctx, workspace_bytes((size_t)n) + io + sa_bytes + 1024);
-    if (rc) return rc;
-    // I/O region: text, then the suffix array
-    ctx->io_bytes = (io + sa_bytes + 1) / 2;
-    ctx->io_bytes = (ctx->io_bytes + 255) & ~(size_t)255;
-    u8 *d_in = ctx->arena;
-    i32 *d_sa = (i32 *)(ctx->arena + io);
-    cudaStream_t st = ctx->own_stream;
-    CK(cudaMemcpyAsync(d_in, T, (size_t)n, cudaMemcpyHostToDevice, st));
-    ctx->io_in = d_in;
-    stats_begin(ctx, n, 0, st);
-    rc = forward_core(ctx, d_in, (u32)n, nullptr, d_sa, FWD_SA, st);
-    ctx->io_in = nullptr;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    CK(cudaMemcpyAsync(SA, d_sa, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return 0;
+    if (!g_dev_ctx[device]) return BWTS_B200_ENODEV;
+    return run_sa_host(g_dev_ctx[device], T, n, SA, LCP);
+}
+// libdivsufsort's seam
+extern "C" int bwts_b200_divsufsort(const unsigned char *T, int *SA, int n, int device)
+{
+    if (!T || !SA || n < 0) return BWTS_B200_EINVAL;
+    if (n == 0) return 0;
+    return sa_default_ctx(T, SA, nullptr, n, device);
+}
+extern "C" int bwts_b200_sa_lcp(const unsigned char *T, int *SA, int *LCP, int n, int device)
+{
+    if (!T || !SA || !LCP || n < 0) return BWTS_B200_EINVAL;
+    if (n == 0) return 0;
+    const int rc = check_sa_args(T, n, SA, LCP, true);
+    return rc ? rc : sa_default_ctx(T, SA, LCP, n, device);
 }
 
 // ---- introspection --------------------------------------------------------------------------------------
@@ -1910,5 +2073,6 @@ extern "C" int bwts_b200_tune(int key, long value)
     if (key == 23) { g_tune_emitwin = value; return 0; }
     if (key == 16) { if (value < 0) return BWTS_B200_EINVAL; g_tune_invbudget = value; return 0; }
     if (key == 13) { if (value < 0) return BWTS_B200_EINVAL; g_tune_invq = value; return 0; }
+    if (key == 24) { if (value < 0 || value > 2) return BWTS_B200_EINVAL; g_tune_lcp = value; return 0; }
     return BWTS_B200_EINVAL;
 }

@@ -16,7 +16,10 @@
  *                       and its inverse, on the same kernels (see the section below).
  *   bwts_b200_divbwt*, bwts_b200_inverse_bw_transform
  *                       additive: libdivsufsort's end-of-text BWT (divbwt / inverse_bw_transform),
- *                       on the same kernels (see the last section).
+ *                       on the same kernels (see the section below).
+ *   bwts_b200_sa_*, bwts_b200_sa_lcp
+ *                       additive: the suffix array and the LCP array on the context, device and
+ *                       one-call entry points (see the last section).
  *
  * Byte layout is the reference's: `len` raw input bytes in, exactly `len` raw bytes
  * out, no header, no primary index, no terminator (mk_bwts_sa.c:60, unbwts.c:173).
@@ -204,7 +207,8 @@ const char *bwts_b200_version(void);
  * groups of up to 32 (1; measured slower than one thread per member), 21 = digit histograms of the initial sort by a
  * sweep over the keys (1) instead of the window histogram taken while the keys are built, 22 = initial keys of whole
  * symbols only (1; default: spare key bits hold the top bits of the next symbol), 23 = MiB of output per emit window
- * (16..1024; default 64: the scatter target of one sweep stays in L2).  value 0 = default. */
+ * (16..1024; default 64: the scatter target of one sweep stays in L2), 24 = LCP array: every irreducible pair
+ * through the warp tier (1) or the multi-CTA tier (2) instead of by its length.  value 0 = default. */
 int bwts_b200_tune(int key, long value);
 
 /* ---- "next" row (SURVEY.md 8f.2): suffix array behind libdivsufsort's own seam ----- */
@@ -256,6 +260,44 @@ int bwts_b200_divbwt_forward_blocks(const unsigned char *in, long len, long bloc
                                     long *primary /* one per block */, const int *devices, int ndev);
 int bwts_b200_divbwt_inverse_blocks(const unsigned char *in, long len, long block_len, const long *primary,
                                     unsigned char *out, const int *devices, int ndev);
+
+/* ---- suffix array and LCP array ------------------------------------------------------ */
+/* n = len, 1 <= len <= BWTS_B200_MAX_LEN.  Bytes compare as unsigned char and the end of text is
+ * smaller than every byte (the order of bwts_b200_divsufsort).  Both arrays are int32:
+ *     SA[0..n)   the start offsets of the suffixes of in, ascending;
+ *     LCP[0] = 0, and for r >= 1 LCP[r] = the length of the longest common prefix of the suffixes
+ *                starting at SA[r-1] and SA[r] (Kasai's convention).
+ * Examples:  banana       SA [5,3,1,0,4,2]              LCP [0,1,3,0,0,2]
+ *            mississippi  SA [10,7,4,1,0,9,8,6,3,5,2]   LCP [0,1,1,4,0,0,1,0,2,1,3]
+ *            abracadabra  SA [10,7,0,3,5,8,1,4,6,9,2]   LCP [0,1,4,1,1,0,3,0,0,0,2]
+ *            aaaa         SA [3,2,1,0]                  LCP [0,1,2,3]
+ *            a            SA [0]                        LCP [0]
+ * and in general a^n gives SA[r] = n-1-r, LCP[r] = r.
+ *
+ * The LCP array is computed on the GPU after the suffix sort from the irreducible LCP values
+ * (Kärkkäinen, Manzini and Puglisi, CPM 2009; DESIGN.md section 4.8): only the pairs at the BWT's run
+ * boundaries are compared, in tiers of one thread, one warp and many CTAs per pair, and the rest
+ * follows from one max-scan.
+ *
+ * Arguments follow the bwts_b200_bwt_* calls: a NULL pointer or len <= 0 is BWTS_B200_EINVAL,
+ * len > BWTS_B200_MAX_LEN is BWTS_B200_ETOOBIG, and no two of in, sa and lcp may share a byte
+ * (BWTS_B200_EINVAL).  The device calls take device addresses: sa and lcp must be 4-byte
+ * aligned (else BWTS_B200_EINVAL), the input may lie at any offset.  bwts_b200_sa_lcp takes the rules of
+ * bwts_b200_divsufsort: n == 0 returns 0, n < 0 is BWTS_B200_EINVAL; it runs on the per-device
+ * context of the other one-call functions.  Without a device every call returns BWTS_B200_ENODEV.
+ *
+ * Device memory: the workspace of the BWTS call of the same length (71 bytes per input byte + 64 MiB);
+ * the LCP stage takes its scratch from the sort's buffers, which are dead by then.  The host and one-call
+ * forms add an I/O region of 5 bytes per input byte (text, SA), 9 with the LCP array: ~80 bytes per
+ * byte in all, 172 GB at len = 2^31 - 1.  The device forms add nothing for an input at a 16-byte aligned
+ * address (2 bytes per byte otherwise, as the other device calls).
+ * Statistics: direction 0, factors = 1, longest_factor = n; the LCP kernels (k_lcp_*) are booked to
+ * kernel class "emit" and phase 3, beside k_emit_sa. */
+int bwts_b200_sa_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa);
+int bwts_b200_sa_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_sa, void *stream);
+int bwts_b200_sa_lcp_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa, int *lcp);
+int bwts_b200_sa_lcp_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_sa, void *d_lcp, void *stream);
+int bwts_b200_sa_lcp(const unsigned char *T, int *SA, int *LCP, int n, int device);   /* divsufsort-shaped */
 
 #ifdef __cplusplus
 }
