@@ -33,6 +33,8 @@ EXPORTS = [
     "bwts_b200_divbwt_inverse_host", "bwts_b200_divbwt_forward_device", "bwts_b200_divbwt_inverse_device",
     "bwts_b200_divbwt_forward_blocks", "bwts_b200_divbwt_inverse_blocks",
     "bwts_b200_sa_host", "bwts_b200_sa_device", "bwts_b200_sa_lcp_host", "bwts_b200_sa_lcp_device", "bwts_b200_sa_lcp",
+    "bwts_b200_fm_build_host", "bwts_b200_fm_build_device", "bwts_b200_fm_free", "bwts_b200_fm_bytes",
+    "bwts_b200_fm_count_host", "bwts_b200_fm_count_device", "bwts_b200_fm_locate_host", "bwts_b200_fm_locate_device",
 ]
 
 
@@ -119,6 +121,16 @@ def lib():
     L.bwts_b200_sa_lcp_host.argtypes = [vp, vp, cl, vp, vp]
     L.bwts_b200_sa_lcp_device.argtypes = [vp, vp, cl, vp, vp, vp]
     L.bwts_b200_sa_lcp.argtypes = [vp, vp, vp, ci, ci]
+    L.bwts_b200_fm_build_host.argtypes = [vp, vp, cl, ci, vp]
+    L.bwts_b200_fm_build_device.argtypes = [vp, vp, cl, ci, vp, vp]
+    L.bwts_b200_fm_free.argtypes = [vp]
+    L.bwts_b200_fm_free.restype = None
+    L.bwts_b200_fm_bytes.argtypes = [vp]
+    L.bwts_b200_fm_bytes.restype = cl
+    L.bwts_b200_fm_count_host.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp]
+    L.bwts_b200_fm_count_device.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp, vp]
+    L.bwts_b200_fm_locate_host.argtypes = [vp, vp, vp, cl, vp, cl, vp]
+    L.bwts_b200_fm_locate_device.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp]
     _lib = L
     return L
 
@@ -319,6 +331,51 @@ def suffix_array_lcp(data, device=0):
     return sa, lcp
 
 
+class FMIndex:
+    """bwts_b200_fm: a device-resident FM-index (Context.fm_build_host / fm_build_device).  It owns its device
+    memory until close(), outlives the context that built it, and any context on its device may query it."""
+
+    def __init__(self, handle, length, sample):
+        self._h = handle
+        self.length = length
+        self.sample = sample
+
+    @property
+    def handle(self):
+        """the bwts_b200_fm pointer, for the C calls"""
+        return self._h
+
+    @property
+    def nbytes(self):
+        """device bytes the index holds (bwts_b200_fm_bytes)"""
+        return lib().bwts_b200_fm_bytes(self._h)
+
+    def close(self):
+        if self._h:
+            lib().bwts_b200_fm_free(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def fm_patterns(patterns):
+    """list of bytes -> (concatenated uint8 array, int64 offsets of npat + 1 entries)"""
+    pats = [bytes(p) for p in patterns]
+    off = np.zeros(len(pats) + 1, dtype=np.int64)
+    np.cumsum([len(p) for p in pats], out=off[1:])
+    return np.frombuffer(b"".join(pats), dtype=np.uint8), off
+
+
 class Context:
     """bwts_b200_ctx: reusable device workspace (one per device per host thread)."""
 
@@ -461,6 +518,62 @@ class Context:
     def sa_lcp_device(self, d_in, length, d_sa, d_lcp, stream=None):
         """suffix array into d_sa and LCP array into d_lcp (length int32 each, 4-byte aligned)"""
         _check(lib().bwts_b200_sa_lcp_device(self._h, d_in, length, d_sa, d_lcp, stream), "bwts_b200_sa_lcp_device")
+
+    # FM-index (include/bwts_b200.h, last section)
+    def fm_build_host(self, data, sample=32):
+        """-> FMIndex over `data` (host bytes), SA sampled at text positions that are multiples of `sample`"""
+        src = _as_u8(data)
+        h = ctypes.c_void_p()
+        _check(lib().bwts_b200_fm_build_host(self._h, src.ctypes.data, len(src), sample, ctypes.byref(h)),
+               "bwts_b200_fm_build_host")
+        return FMIndex(h.value, len(src), sample)
+
+    def fm_build_device(self, d_in, length, sample=32, stream=None):
+        """-> FMIndex over `length` device bytes at d_in"""
+        h = ctypes.c_void_p()
+        _check(lib().bwts_b200_fm_build_device(self._h, d_in, length, sample, ctypes.byref(h), stream),
+               "bwts_b200_fm_build_device")
+        return FMIndex(h.value, length, sample)
+
+    def fm_count_host(self, fm, patterns):
+        """list of bytes -> (lo, hi), int32 arrays: pattern k occurs hi[k] - lo[k] times, at SA[lo[k]:hi[k]]"""
+        pat, off = fm_patterns(patterns)
+        rng = np.empty(2 * (len(off) - 1), dtype=np.int32)
+        total = ctypes.c_long()
+        _check(lib().bwts_b200_fm_count_host(self._h, fm.handle, pat.ctypes.data, len(pat), off.ctypes.data,
+                                             len(off) - 1, rng.ctypes.data, ctypes.byref(total)),
+               "bwts_b200_fm_count_host")
+        return rng[0::2].copy(), rng[1::2].copy()
+
+    def fm_locate_host(self, fm, lo, hi):
+        """-> (positions int32, offsets int64 of len(lo) + 1): range k's SA[lo[k]:hi[k]] is
+        positions[offsets[k]:offsets[k+1]]"""
+        lo = np.asarray(lo, dtype=np.int32)
+        hi = np.asarray(hi, dtype=np.int32)
+        rng = np.empty(2 * len(lo), dtype=np.int32)
+        rng[0::2], rng[1::2] = lo, hi
+        off = np.zeros(len(lo) + 1, dtype=np.int64)
+        np.cumsum(hi.astype(np.int64) - lo, out=off[1:])
+        cap = max(int(off[-1]), 0)
+        pos = np.empty(max(cap, 1), dtype=np.int32)
+        total = ctypes.c_long()
+        _check(lib().bwts_b200_fm_locate_host(self._h, fm.handle, rng.ctypes.data, len(lo), pos.ctypes.data, cap,
+                                              ctypes.byref(total)), "bwts_b200_fm_locate_host")
+        return pos[:total.value], off
+
+    def fm_count_device(self, fm, d_pat, pat_len, d_off, npat, d_range, stream=None):
+        """device arrays: patterns, int64 offsets (npat + 1), int32 ranges (2 npat) -> total of hi - lo"""
+        total = ctypes.c_long()
+        _check(lib().bwts_b200_fm_count_device(self._h, fm.handle, d_pat, pat_len, d_off, npat, d_range,
+                                               ctypes.byref(total), stream), "bwts_b200_fm_count_device")
+        return total.value
+
+    def fm_locate_device(self, fm, d_range, nrange, d_pos, cap, stream=None):
+        """device arrays: int32 ranges (2 nrange), int32 positions (cap) -> number of positions written"""
+        total = ctypes.c_long()
+        _check(lib().bwts_b200_fm_locate_device(self._h, fm.handle, d_range, nrange, d_pos, cap, ctypes.byref(total),
+                                                stream), "bwts_b200_fm_locate_device")
+        return total.value
 
     def stats(self):
         s = Stats()

@@ -19,6 +19,7 @@
 
 #include "../../include/bwts_b200.h"
 #include "common.cuh"
+#include "fm.cuh"
 #include "forward.cuh"
 #include "inverse.cuh"
 #include "lcp.cuh"
@@ -381,12 +382,13 @@ enum FwdMode {
     FWD_LYNDON = 2,      // suffix sort, then factor-start flags (prefix minima of the ISA) into d_out
     FWD_BWTS_FLAGS = 3,  // forward BWTS, factor-start flags already in d_out (after FWD_LYNDON)
     FWD_BWT = 4,         // classic BWT into d_out: rotations of the one factor [0, n), *primary = rank[0]
-    FWD_DIVBWT = 5       // libdivsufsort's divbwt into d_out: the FWD_SA sort, bytes at shifted rows, *primary = rank[0] + 1
+    FWD_DIVBWT = 5,      // libdivsufsort's divbwt into d_out: the FWD_SA sort, bytes at shifted rows, *primary = rank[0] + 1
+    FWD_FM = 6           // FM-index build: the FWD_DIVBWT emit into d_out, then the suffix array into d_sa (fm_build)
 };
 static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 *d_sa, int mode, cudaStream_t st,
                         long *primary = nullptr, i32 *d_lcp = nullptr)
 {
-    const int linear = (mode == FWD_SA || mode == FWD_LYNDON || mode == FWD_DIVBWT);
+    const int linear = (mode == FWD_SA || mode == FWD_LYNDON || mode == FWD_DIVBWT || mode == FWD_FM);
     int rc = arena_reserve(ctx, workspace_bytes(n));
     if (rc) return rc;
     ctx->arena_used = 0;
@@ -897,7 +899,7 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
     // -- emit
     ctx->phase = PH_EMIT;
     (void)PH_SORT0;
-    const bool div = mode == FWD_DIVBWT;  // the byte emit below with emit_slot<true> (forward.cuh)
+    const bool div = mode == FWD_DIVBWT || mode == FWD_FM;  // the byte emit below with emit_slot<true> (forward.cuh)
     if (!linear || div) {
         const bool emit_binned = g_tune_emit >= 2 || (g_tune_emit == 0 && n >= (512u << 20));
         if (emit_binned && kb >= 8 && g_tune_emit != 3) {
@@ -961,6 +963,7 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             if (rc) return rc;
             *primary = (long)ctx->h_small[0];
         }
+        if (mode == FWD_FM) LAUNCH(KC_EMIT, 8.0 * n, k_emit_sa, cdiv(n, 256), 256, rank, n, d_sa);
     } else if (mode == FWD_SA) {
         LAUNCH(KC_EMIT, 8.0 * n, k_emit_sa, cdiv(n, 256), 256, rank, n, d_sa);
         if (d_lcp) {
@@ -1994,6 +1997,337 @@ extern "C" int bwts_b200_sa_lcp(const unsigned char *T, int *SA, int *LCP, int n
     if (n == 0) return 0;
     const int rc = check_sa_args(T, n, SA, LCP, true);
     return rc ? rc : sa_default_ctx(T, SA, LCP, n, device);
+}
+
+// ---- FM-index (fm.cuh) --------------------------------------------------------------------------------------
+// One cudaMalloc per index, laid out in this order, every array rounded up to 256 bytes:
+//     U n, S 4 sg (n/65536 + 1), B 2 sg (n/256 + 1), marks 4 ceil(n/32), dir 4 (n/256 + 1), samples 4 ceil(n/sample),
+//     C 4 x 257, map 256
+struct bwts_b200_fm {
+    int device;
+    u32 n, primary, sample, sg;
+    u8 *mem;
+    size_t bytes;
+    FmView v;
+};
+
+static size_t r256(size_t b) { return (b + 255) & ~(size_t)255; }
+static size_t fm_layout(u32 n, u32 sg, u32 sample, size_t off[9])
+{
+    const size_t sz[8] = {(size_t)n, 4ull * sg * ((n >> 16) + 1), 2ull * sg * ((n >> 8) + 1), 4ull * ((n + 31ull) / 32),
+                          4ull * ((n >> 8) + 1), 4ull * ((n + (u64)sample - 1) / sample), 4 * 257, 256};
+    off[0] = 0;
+    for (int k = 0; k < 8; k++) off[k + 1] = off[k] + r256(sz[k]);
+    return off[8];
+}
+static bool fm_sample_ok(int sample) { return sample >= 1 && sample <= 1024 && (sample & (sample - 1)) == 0; }
+
+// The build: the byte histogram (C, the symbol map, sg, and so the index's size), the FWD_FM sort -- divbwt bytes
+// into the index's U, the suffix array into the I/O region -- then the checkpoints, marks, directory and samples.
+// d_text lies at the bottom of the arena, in an I/O region of io bytes reserved by the caller.
+static int fm_build_core(bwts_b200_ctx *ctx, const u8 *d_text, u32 n, u32 sample, size_t io, bwts_b200_fm **out,
+                         cudaStream_t st)
+{
+    const u32 nb = (n >> 8) + 1, ns = (n >> 16) + 1;
+    const u32 nt = cdiv(nb, SC_TILE);
+    u8 *p = ctx->arena + r256(n);
+    i32 *d_sa = (i32 *)p;            p += r256(4ull * n);
+    u32 *dircnt = (u32 *)p;          p += r256(4ull * nb);
+    u32 *tiles = (u32 *)p;           p += r256(4ull * (nt + 1));
+    u32 *hist = (u32 *)p;            p += 1024;
+    u8 *syms = p;                    p += 256;
+    if ((size_t)(p - ctx->arena) > io) return BWTS_B200_EINTERNAL;
+    ctx->io_bytes = (io + 1) / 2;    // forward_core skips 2 io_bytes (+ up to 511) of the arena
+    ctx->io_in = (u8 *)d_text;
+
+    stats_begin(ctx, n, 0, st);
+    ctx->phase = 3;
+    CK(cudaMemsetAsync(hist, 0, 1024, st));
+    LAUNCH(KC_EMIT, 1.0 * n, k_fm_hist, min(cdiv(n, 256), (u32)ctx->sm_count * 8), 256, d_text, n, hist);
+    int rc = readback(ctx, st, hist, 1024);
+    if (rc) return rc;
+    ctx->phase = 0;
+    std::vector<u32> C(257);
+    std::vector<u8> map(256, 0), sy;
+    u32 acc = 1;  // the end of text
+    for (int c = 0; c < 256; c++) {
+        C[c] = acc;
+        acc += ctx->h_small[c];
+        if (ctx->h_small[c]) { map[c] = (u8)sy.size(); sy.push_back((u8)c); }
+    }
+    C[256] = acc;
+    const u32 sg = (u32)sy.size();
+    size_t off[9];
+    const size_t bytes = fm_layout(n, sg, sample, off);
+    bwts_b200_fm *fm = new bwts_b200_fm();
+    fm->device = ctx->device; fm->n = n; fm->sample = sample; fm->sg = sg; fm->bytes = bytes;
+    const cudaError_t ea = cudaMalloc((void **)&fm->mem, bytes);
+    if (ea != cudaSuccess) {
+        delete fm;
+        ctx->last_cuda = (int)ea;
+        cudaGetLastError();
+        return ea == cudaErrorMemoryAllocation ? BWTS_B200_ENOMEM : BWTS_B200_ECUDA;
+    }
+    u8 *U = fm->mem + off[0];
+    u32 *S = (u32 *)(fm->mem + off[1]);
+    u16 *B = (u16 *)(fm->mem + off[2]);
+    u32 *marks = (u32 *)(fm->mem + off[3]), *dir = (u32 *)(fm->mem + off[4]), *samples = (u32 *)(fm->mem + off[5]);
+    u32 *dC = (u32 *)(fm->mem + off[6]);
+    u8 *dmap = fm->mem + off[7];
+    const auto fail = [&](int code) { cudaStreamSynchronize(st); cudaGetLastError(); cudaFree(fm->mem); delete fm; return code; };
+#define FCK(call) do { const cudaError_t e__ = (call); if (e__ != cudaSuccess) { ctx->last_cuda = (int)e__; return fail(BWTS_B200_ECUDA); } } while (0)
+    FCK(cudaMemcpyAsync(dC, C.data(), 4 * 257, cudaMemcpyHostToDevice, st));
+    FCK(cudaMemcpyAsync(dmap, map.data(), 256, cudaMemcpyHostToDevice, st));
+    FCK(cudaMemcpyAsync(syms, sy.data(), sg, cudaMemcpyHostToDevice, st));
+    FCK(cudaStreamSynchronize(st));  // the host vectors go out of scope below
+    long primary = 0;
+    rc = forward_core(ctx, d_text, n, U, d_sa, FWD_FM, st, &primary);
+    if (rc) return fail(rc);
+    fm->primary = (u32)primary;
+    // the k_fm_* build kernels, booked like the LCP stage: class emit, phase 3
+    ctx->phase = 3;
+    rc = [&]() -> int {
+        LAUNCH(KC_EMIT, 1.0 * n + 2.0 * sg * nb, k_fm_block_counts, cdiv(nb, 8), 256, U, n, syms, sg, B);
+        LAUNCH(KC_EMIT, 4.0 * sg * nb + 4.0 * sg * ns, k_fm_block_scan, ns, 256, n, sg, B, S);
+        LAUNCH(KC_EMIT, 8.0 * sg * ns, k_fm_super_scan, sg, 32, n, sg, S);
+        LAUNCH(KC_EMIT, 4.0 * n + n / 8.0 + 4.0 * nb, k_fm_marks, nb, 256, d_sa, n, sample, marks, dircnt);
+        LAUNCH(KC_EMIT, 4.0 * nb, k_tile_sum_u32, nt, 256, dircnt, nb, tiles, nullptr);
+        LAUNCH(KC_EMIT, 8.0 * nt, k_scan_excl_u32_block, 1, 1024, tiles, tiles, nt, nullptr);
+        LAUNCH(KC_EMIT, 8.0 * nb, k_tile_scan_apply_u32, nt, 256, dircnt, dir, nb, tiles);
+        LAUNCH(KC_EMIT, 4.0 * n + n / 8.0 + 4.0 * n / sample, k_fm_samples, cdiv(n, 256), 256, d_sa, n, sample, marks, dir,
+               samples);
+        return 0;
+    }();
+    ctx->io_in = nullptr;
+    if (rc) return fail(rc);
+    stats_end(ctx, st);
+    FCK(cudaGetLastError());
+#undef FCK
+    fm->v.U = U; fm->v.S = S; fm->v.B = B; fm->v.marks = marks; fm->v.dir = dir; fm->v.samples = samples;
+    fm->v.C = dC; fm->v.map = dmap;
+    fm->v.n = n; fm->v.primary = fm->primary; fm->v.sample = sample; fm->v.sg = sg;
+    *out = fm;
+    return 0;
+}
+
+// I/O region of a build: the text, the suffix array, the directory's block counts and its tile sums, the histogram
+// and the symbol list
+static size_t fm_build_io(size_t n)
+{
+    const size_t nb = (n >> 8) + 1;
+    return r256(n) + r256(4 * n) + r256(4 * nb) + r256(4 * (cdiv(nb, SC_TILE) + 1)) + 1024 + 256;
+}
+static int fm_build_args(bwts_b200_ctx *ctx, const void *in, long len, int sample, bwts_b200_fm **fm)
+{
+    if (fm) *fm = nullptr;
+    if (!ctx || !in || !fm || len <= 0 || !fm_sample_ok(sample)) return BWTS_B200_EINVAL;
+    if (len > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    return 0;
+}
+static int fm_build(bwts_b200_ctx *ctx, const void *src, long len, int sample, bwts_b200_fm **fm, cudaStream_t st,
+                    bool host)
+{
+    CK(cudaSetDevice(ctx->device));
+    const size_t io = fm_build_io((size_t)len);
+    int rc = arena_reserve(ctx, workspace_bytes((size_t)len) + io + 1024);
+    if (rc) return rc;
+    apply_device_limits();
+    ctx->io_in = nullptr;
+    if (host) {
+        CK(cudaEventRecord(ctx->ev_io0, st));
+        rc = stage_h2d(ctx, ctx->arena, (const u8 *)src, (size_t)len, st);
+        if (rc) return rc;
+    } else {  // the text is copied next to the suffix array whatever its alignment: one n-byte copy
+        CK(cudaMemcpyAsync(ctx->arena, src, (size_t)len, cudaMemcpyDeviceToDevice, st));
+    }
+    rc = fm_build_core(ctx, ctx->arena, (u32)len, (u32)sample, io, fm, st);
+    ctx->io_in = nullptr;
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    if (host) {
+        float t = 0;
+        if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
+    }
+    return 0;
+}
+
+extern "C" int bwts_b200_fm_build_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int sample,
+                                       bwts_b200_fm **fm)
+{
+    const int rc = fm_build_args(ctx, in, len, sample, fm);
+    return rc ? rc : fm_build(ctx, in, len, sample, fm, ctx->own_stream, true);
+}
+extern "C" int bwts_b200_fm_build_device(bwts_b200_ctx *ctx, const void *d_in, long len, int sample, bwts_b200_fm **fm,
+                                         void *stream)
+{
+    const int rc = fm_build_args(ctx, d_in, len, sample, fm);
+    return rc ? rc : fm_build(ctx, d_in, len, sample, fm, stream ? (cudaStream_t)stream : ctx->own_stream, false);
+}
+extern "C" void bwts_b200_fm_free(bwts_b200_fm *fm)
+{
+    if (!fm) return;
+    cudaSetDevice(fm->device);
+    cudaFree(fm->mem);
+    delete fm;
+}
+extern "C" long bwts_b200_fm_bytes(const bwts_b200_fm *fm)
+{
+    return fm ? (long)fm->bytes : 0;
+}
+
+// Queries run on the context's arena: 64 bytes of counters at its start, then (host forms) the staged arrays.
+// direction 1, phase 2 ("Walk sublists"): the searches and walks in class inv_walk, the checks and the offsets
+// scan in class inv_scan.
+static int fm_query_ctx(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, size_t arena_bytes, cudaStream_t st)
+{
+    if (ctx->device != fm->device) return BWTS_B200_EINVAL;
+    CK(cudaSetDevice(ctx->device));
+    int rc = arena_reserve(ctx, max(arena_bytes, (size_t)4096));
+    if (rc) return rc;
+    stats_begin(ctx, fm->n, 1, st);
+    ctx->phase = 2;
+    return 0;
+}
+static int fm_query_end(bwts_b200_ctx *ctx, cudaStream_t st)
+{
+    stats_end(ctx, st);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
+    return 0;
+}
+static u64 h_small_u64(const bwts_b200_ctx *ctx, int w) { return (u64)ctx->h_small[w] | ((u64)ctx->h_small[w + 1] << 32); }
+
+// arguments and stream set up by the caller; check_off: the device form's offsets check
+static int fm_count_core(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const u8 *d_pat, long pat_len, const long long *d_off,
+                         long npat, i32 *d_range, long *total, bool check_off, cudaStream_t st)
+{
+    u32 *flags = (u32 *)ctx->arena;  // [0] bad offsets, [2..3] sum of hi - lo, [4..5] bytes read
+    unsigned long long *cnt = (unsigned long long *)(flags + 2);
+    CK(cudaMemsetAsync(flags, 0, 64, st));
+    if (check_off)
+        LAUNCH(KC_INV_SCAN, 8.0 * (npat + 1), k_fm_check_off, min(cdiv((u64)npat + 1, 256), (u32)ctx->sm_count * 8), 256,
+               d_off, (u64)npat, (long long)pat_len, flags);
+    LAUNCH(KC_INV_WALK, 16.0 * npat, k_fm_count, min(cdiv((u64)npat, 8), (u32)ctx->sm_count * 64), 256, fm->v, d_pat,
+           d_off, (u64)npat, d_range, flags, cnt);
+    const size_t rec = ctx->recs.size() - 1;
+    int rc = readback(ctx, st, flags, 24);
+    if (rc) return rc;
+    if (ctx->h_small[0]) return BWTS_B200_EINVAL;
+    ctx->recs[rec].bytes += (double)h_small_u64(ctx, 4);
+    if (total) *total = (long)h_small_u64(ctx, 2);
+    return 0;
+}
+
+// the rules of off on the host: off[0] == 0, non-decreasing, off[npat] == pat_len
+static bool fm_off_ok(const long *off, long npat, long pat_len)
+{
+    if (off[0] != 0 || off[npat] != pat_len) return false;
+    for (long k = 0; k < npat; k++)
+        if (off[k] > off[k + 1]) return false;
+    return true;
+}
+
+extern "C" int bwts_b200_fm_count_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const unsigned char *pat, long pat_len,
+                                       const long *off, long npat, int *range, long *total)
+{
+    if (!ctx || !fm || npat < 0 || pat_len < 0) return BWTS_B200_EINVAL;
+    if (npat == 0) { if (total) *total = 0; return 0; }
+    if (!off || !range || (pat_len > 0 && !pat)) return BWTS_B200_EINVAL;
+    if (!fm_off_ok(off, npat, pat_len)) return BWTS_B200_EINVAL;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    const size_t a_pat = 256, a_off = a_pat + r256((size_t)pat_len), a_range = a_off + r256(8 * ((size_t)npat + 1));
+    cudaStream_t st = ctx->own_stream;
+    int rc = fm_query_ctx(ctx, fm, a_range + r256(8 * (size_t)npat), st);
+    if (rc) return rc;
+    u8 *d_pat = ctx->arena + a_pat;
+    long long *d_off = (long long *)(ctx->arena + a_off);
+    i32 *d_range = (i32 *)(ctx->arena + a_range);
+    if (pat_len) { rc = stage_h2d(ctx, d_pat, pat, (size_t)pat_len, st); if (rc) return rc; }
+    rc = stage_h2d(ctx, (u8 *)d_off, (const u8 *)off, 8 * ((size_t)npat + 1), st);
+    if (!rc) rc = fm_count_core(ctx, fm, d_pat, pat_len, d_off, npat, d_range, total, false, st);
+    if (!rc) rc = stage_d2h(ctx, (u8 *)range, (const u8 *)d_range, 8 * (size_t)npat, st);
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    CK(cudaStreamSynchronize(st));
+    return fm_query_end(ctx, st);
+}
+extern "C" int bwts_b200_fm_count_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_pat, long pat_len,
+                                         const void *d_off, long npat, void *d_range, long *total, void *stream)
+{
+    if (!ctx || !fm || npat < 0 || pat_len < 0) return BWTS_B200_EINVAL;
+    if (npat == 0) { if (total) *total = 0; return 0; }
+    if (!d_off || !d_range || (pat_len > 0 && !d_pat)) return BWTS_B200_EINVAL;
+    if (((uintptr_t)d_off & 7) || ((uintptr_t)d_range & 3)) return BWTS_B200_EINVAL;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    int rc = fm_query_ctx(ctx, fm, 4096, st);
+    if (!rc) rc = fm_count_core(ctx, fm, (const u8 *)d_pat, pat_len, (const long long *)d_off, npat, (i32 *)d_range, total,
+                                true, st);
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    return fm_query_end(ctx, st);
+}
+
+// offsets of the ranges at arena + 256 (nrange + 1 u64); a bad range or a total above cap is EINVAL, nothing written
+static int fm_locate_core(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const i32 *d_range, long nrange, i32 *d_pos, long cap,
+                          long *total, cudaStream_t st)
+{
+    u32 *flags = (u32 *)ctx->arena;  // [0] bad range, [1] over cap, [2..3] total, [4..5] bytes read
+    unsigned long long *offs = (unsigned long long *)(ctx->arena + 256);
+    CK(cudaMemsetAsync(flags, 0, 64, st));
+    LAUNCH(KC_INV_SCAN, 16.0 * nrange, k_fm_range_scan, 1, 1024, d_range, (u64)nrange, fm->n, (u64)cap, offs, flags);
+    int rc = readback(ctx, st, flags, 16);
+    if (rc) return rc;
+    if (ctx->h_small[0] || ctx->h_small[1]) return BWTS_B200_EINVAL;
+    const u64 tot = h_small_u64(ctx, 2);
+    if (tot) {
+        LAUNCH(KC_INV_WALK, 4.0 * tot, k_fm_locate, (u32)min((tot + 15) / 16, (u64)ctx->sm_count * 64), 256, fm->v, d_range,
+               (u64)nrange, offs, tot, d_pos, (unsigned long long *)(flags + 4));
+        const size_t rec = ctx->recs.size() - 1;
+        rc = readback(ctx, st, flags, 24);
+        if (rc) return rc;
+        ctx->recs[rec].bytes += (double)h_small_u64(ctx, 4);
+    }
+    if (total) *total = (long)tot;
+    return 0;
+}
+
+extern "C" int bwts_b200_fm_locate_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const int *range, long nrange,
+                                        int *pos, long cap, long *total)
+{
+    if (!ctx || !fm || nrange < 0 || cap < 0) return BWTS_B200_EINVAL;
+    if (nrange == 0) { if (total) *total = 0; return 0; }
+    if (!range || !pos) return BWTS_B200_EINVAL;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    u64 tot = 0;
+    for (long k = 0; k < nrange; k++) {
+        const int lo = range[2 * k], hi = range[2 * k + 1];
+        if (lo < 0 || lo > hi || (u32)hi > fm->n) return BWTS_B200_EINVAL;
+        tot += (u64)(hi - lo);
+    }
+    if (tot > (u64)cap) return BWTS_B200_EINVAL;
+    const size_t a_range = 256 + r256(8 * ((size_t)nrange + 1)), a_pos = a_range + r256(8 * (size_t)nrange);
+    cudaStream_t st = ctx->own_stream;
+    int rc = fm_query_ctx(ctx, fm, a_pos + r256(4 * tot), st);
+    if (rc) return rc;
+    i32 *d_range = (i32 *)(ctx->arena + a_range), *d_pos = (i32 *)(ctx->arena + a_pos);
+    rc = stage_h2d(ctx, (u8 *)d_range, (const u8 *)range, 8 * (size_t)nrange, st);
+    if (!rc) rc = fm_locate_core(ctx, fm, d_range, nrange, d_pos, cap, total, st);
+    if (!rc && tot) rc = stage_d2h(ctx, (u8 *)pos, (const u8 *)d_pos, 4 * tot, st);
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    CK(cudaStreamSynchronize(st));
+    return fm_query_end(ctx, st);
+}
+extern "C" int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_range, long nrange,
+                                          void *d_pos, long cap, long *total, void *stream)
+{
+    if (!ctx || !fm || nrange < 0 || cap < 0) return BWTS_B200_EINVAL;
+    if (nrange == 0) { if (total) *total = 0; return 0; }
+    if (!d_range || !d_pos || ((uintptr_t)d_range & 3) || ((uintptr_t)d_pos & 3)) return BWTS_B200_EINVAL;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    int rc = fm_query_ctx(ctx, fm, 256 + r256(8 * ((size_t)nrange + 1)), st);
+    if (!rc) rc = fm_locate_core(ctx, fm, (const i32 *)d_range, nrange, (i32 *)d_pos, cap, total, st);
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    return fm_query_end(ctx, st);
 }
 
 // ---- introspection --------------------------------------------------------------------------------------

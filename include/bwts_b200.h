@@ -19,7 +19,9 @@
  *                       on the same kernels (see the section below).
  *   bwts_b200_sa_*, bwts_b200_sa_lcp
  *                       additive: the suffix array and the LCP array on the context, device and
- *                       one-call entry points (see the last section).
+ *                       one-call entry points (see the section below).
+ *   bwts_b200_fm_*      additive: an FM-index over the divbwt output, counting and locating many
+ *                       patterns on the GPU (see the last section).
  *
  * Byte layout is the reference's: `len` raw input bytes in, exactly `len` raw bytes
  * out, no header, no primary index, no terminator (mk_bwts_sa.c:60, unbwts.c:173).
@@ -298,6 +300,69 @@ int bwts_b200_sa_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_
 int bwts_b200_sa_lcp_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa, int *lcp);
 int bwts_b200_sa_lcp_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_sa, void *d_lcp, void *stream);
 int bwts_b200_sa_lcp(const unsigned char *T, int *SA, int *LCP, int n, int device);   /* divsufsort-shaped */
+
+/* ---- FM-index: count and locate over libdivsufsort's BWT ----------------------------------- */
+/* Bytes compare as unsigned char and the end of text is smaller than every byte (the order of
+ * bwts_b200_divsufsort and bwts_b200_sa_*); SA is the suffix array of the text T, n = len,
+ * 1 <= len <= BWTS_B200_MAX_LEN.  An index is built once from T and answers batches of patterns.
+ *
+ * Count: for a pattern P of m >= 0 bytes,
+ *     lo = #{ i : T[i..n) < P },   hi = #{ i : T[i..n)[0..m) <= P },   0 <= lo <= hi <= n,
+ * with a suffix that is a proper prefix of P smaller than P.  P occurs hi - lo times, at SA[lo..hi); when it
+ * does not occur, lo == hi is its insertion point among the sorted suffixes; the empty pattern gives [0, n).
+ * (bisect_left / bisect_right over the sorted suffixes.)
+ * Locate: for ranges [lo_k, hi_k) with 0 <= lo_k <= hi_k <= n, pos = SA[lo_0..hi_0) . SA[lo_1..hi_1) . ...,
+ * in range order and in SA row order inside each range -- no sorting by position.
+ *     banana       ana -> (1, 3) [3, 1]     a -> (0, 3) [5, 3, 1]    na -> (4, 6) [4, 2]
+ *                  anan -> (2, 3) [1]       banana -> (3, 4) [0]     bananas -> (4, 4) []
+ *                  nab -> (5, 5) []         z -> (6, 6) []           \x00 -> (0, 0) []
+ *                  (empty) -> (0, 6) [5, 3, 1, 0, 4, 2]
+ *     mississippi  ssi -> (9, 11) [5, 2]    issi -> (2, 4) [4, 1]    ppp -> (7, 7) []
+ *     aaaa         aa -> (1, 4) [2, 1, 0]   aaaaa -> (4, 4) []
+ *
+ * Index (DESIGN.md section 4.9): the divbwt output U and its primary as the L column of T$, occurrence
+ * checkpoints for the sg distinct bytes of T (u32 per 65536 rows, u16 per 256 rows), and the SA values at
+ * the rows whose text position is a multiple of `sample`, found by a bit vector with a directory.  Counting
+ * is backward search, one warp per pattern; locating walks LF from each row to a sampled one, at most
+ * sample - 1 steps.  `sample` is a power of two in [1, 1024], else BWTS_B200_EINVAL.
+ * bwts_b200_fm_bytes, with every term rounded up to a multiple of 256:
+ *     n + 4 sg (n/65536 + 1) + 2 sg (n/256 + 1) + 4 ceil(n/32) + 4 (n/256 + 1) + 4 ceil(n/sample) + 1028 + 256
+ * (/ is integer division): ~1.17 n + 4n/sample for DNA, ~3.16 n + 4n/sample with all 256 byte values.
+ * The build needs the workspace of the SA call of the same length plus an I/O region of ~5 bytes per byte
+ * (text and suffix array); it books like bwts_b200_sa_*: direction 0, factors = 1, the k_fm_* build kernels to
+ * class "emit" and phase 3.  A query resets the statistics: direction 1, backward search and LF walks
+ * (k_fm_count, k_fm_locate) in class "inv_walk", the argument checks and the offsets scan in class
+ * "inv_scan", all in phase 2.
+ *
+ * Patterns: pattern k = pat[off[k] .. off[k+1]); off int64[npat + 1] with off[0] == 0, non-decreasing,
+ * off[npat] == pat_len.  range int32[2 npat] = (lo_k, hi_k).  *total (may be NULL) = the sum of hi_k - lo_k.
+ * Locate: pos int32[cap]; a sum of hi_k - lo_k above cap is BWTS_B200_EINVAL and nothing is written.
+ *
+ * Arguments: a NULL ctx or fm, npat < 0, nrange < 0, pat_len < 0, cap < 0, a NULL array the call needs is
+ * BWTS_B200_EINVAL; npat == 0 (nrange == 0) returns 0 with *total = 0.  The host forms check the offsets and the
+ * ranges on the host; the device forms check the same rules in a validation kernel before any other work and
+ * report a violation as BWTS_B200_EINVAL.  No kernel reads outside the buffers it was given, whatever they
+ * hold.  Device offsets must be 8-byte aligned, ranges and positions 4-byte aligned; patterns may start at
+ * any address.  Without a device every call returns BWTS_B200_ENODEV after the checks that need no index
+ * (the ranges against n and the index's device are checked after it).
+ * Device and lifetime: the index owns one device allocation on the device of the context that built it and
+ * outlives that context; any context on that device may query it (another device is BWTS_B200_EINVAL).
+ * Queries only read the index, so host threads with their own contexts may query one index at once. */
+typedef struct bwts_b200_fm bwts_b200_fm;   /* device-resident index, owned by the caller until fm_free */
+
+int  bwts_b200_fm_build_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int sample, bwts_b200_fm **fm);
+int  bwts_b200_fm_build_device(bwts_b200_ctx *ctx, const void *d_in, long len, int sample, bwts_b200_fm **fm,
+                               void *stream);
+void bwts_b200_fm_free(bwts_b200_fm *fm);                 /* NULL is a no-op */
+long bwts_b200_fm_bytes(const bwts_b200_fm *fm);          /* device bytes the index holds; 0 for NULL */
+int bwts_b200_fm_count_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const unsigned char *pat, long pat_len,
+                            const long *off, long npat, int *range, long *total);
+int bwts_b200_fm_count_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_pat, long pat_len,
+                              const void *d_off, long npat, void *d_range, long *total, void *stream);
+int bwts_b200_fm_locate_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const int *range, long nrange,
+                             int *pos, long cap, long *total);
+int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_range, long nrange,
+                               void *d_pos, long cap, long *total, void *stream);
 
 #ifdef __cplusplus
 }
