@@ -35,6 +35,7 @@ EXPORTS = [
     "bwts_b200_sa_host", "bwts_b200_sa_device", "bwts_b200_sa_lcp_host", "bwts_b200_sa_lcp_device", "bwts_b200_sa_lcp",
     "bwts_b200_fm_build_host", "bwts_b200_fm_build_device", "bwts_b200_fm_free", "bwts_b200_fm_bytes",
     "bwts_b200_fm_count_host", "bwts_b200_fm_count_device", "bwts_b200_fm_locate_host", "bwts_b200_fm_locate_device",
+    "bwts_b200_lpf_host", "bwts_b200_lpf_device", "bwts_b200_lz77_host", "bwts_b200_lz77_device",
 ]
 
 
@@ -131,6 +132,10 @@ def lib():
     L.bwts_b200_fm_count_device.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp, vp]
     L.bwts_b200_fm_locate_host.argtypes = [vp, vp, vp, cl, vp, cl, vp]
     L.bwts_b200_fm_locate_device.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp]
+    L.bwts_b200_lpf_host.argtypes = [vp, vp, cl, vp, vp]
+    L.bwts_b200_lpf_device.argtypes = [vp, vp, cl, vp, vp, vp]
+    L.bwts_b200_lz77_host.argtypes = [vp, vp, cl, vp, cl, ctypes.POINTER(cl)]
+    L.bwts_b200_lz77_device.argtypes = [vp, vp, cl, vp, cl, ctypes.POINTER(cl), vp]
     _lib = L
     return L
 
@@ -519,7 +524,37 @@ class Context:
         """suffix array into d_sa and LCP array into d_lcp (length int32 each, 4-byte aligned)"""
         _check(lib().bwts_b200_sa_lcp_device(self._h, d_in, length, d_sa, d_lcp, stream), "bwts_b200_sa_lcp_device")
 
-    # FM-index (include/bwts_b200.h, last section)
+    # longest-previous-factor array and LZ77 parse (include/bwts_b200.h, last section)
+    def lpf_host(self, data):
+        """-> (LPF, PREV), int32, in text order"""
+        src = _as_u8(data)
+        lpf = np.empty(len(src), dtype=np.int32)
+        prev = np.empty(len(src), dtype=np.int32)
+        _check(lib().bwts_b200_lpf_host(self._h, src.ctypes.data, len(src), lpf.ctypes.data, prev.ctypes.data),
+               "bwts_b200_lpf_host")
+        return lpf, prev
+
+    def lz77_host(self, data):
+        """-> int32 [z, 2]: the greedy parse's factors (source, length), or (byte, 0) for a literal"""
+        src = _as_u8(data)
+        out = np.empty((len(src), 2), dtype=np.int32)
+        z = ctypes.c_long(-1)
+        _check(lib().bwts_b200_lz77_host(self._h, src.ctypes.data, len(src), out.ctypes.data, len(src),
+                                         ctypes.byref(z)), "bwts_b200_lz77_host")
+        return out[:z.value].copy()
+
+    def lpf_device(self, d_in, length, d_lpf, d_prev, stream=None):
+        """LPF into d_lpf and PREV into d_prev (length int32 each, 4-byte aligned)"""
+        _check(lib().bwts_b200_lpf_device(self._h, d_in, length, d_lpf, d_prev, stream), "bwts_b200_lpf_device")
+
+    def lz77_device(self, d_in, length, d_factors, cap, stream=None):
+        """factor pairs into d_factors (room for cap pairs of int32, 4-byte aligned) -> z"""
+        z = ctypes.c_long(-1)
+        _check(lib().bwts_b200_lz77_device(self._h, d_in, length, d_factors, cap, ctypes.byref(z), stream),
+               "bwts_b200_lz77_device")
+        return z.value
+
+    # FM-index (include/bwts_b200.h, section before)
     def fm_build_host(self, data, sample=32):
         """-> FMIndex over `data` (host bytes), SA sampled at text positions that are multiples of `sample`"""
         src = _as_u8(data)

@@ -23,6 +23,7 @@
 #include "forward.cuh"
 #include "inverse.cuh"
 #include "lcp.cuh"
+#include "lz.cuh"
 #include "lyndon.cuh"
 #include "radix.cuh"
 #include "scan.cuh"
@@ -61,6 +62,7 @@ static long g_tune_invmark = 0;    // inverse staged walk marks: 0 = by size (co
 static long g_tune_invbudget = 0;  // inverse fallback walks: step budget per attempt (0 = 32 n)
 static long g_tune_nomark = 0;     // TIMING EXPERIMENT ONLY: inverse first walk without visited marks (wrong output when a cycle has no splitter)
 static long g_tune_lcp = 0;        // LCP pairs: 0 = by length through the three tiers, 1 = all from the warp tier on, 2 = all through the multi-CTA tier
+static long g_tune_lz = 0;         // LPF / LZ77: log2 of the tile and chunk width (5..12; 0 = 12)
 
 static void apply_device_limits()
 {
@@ -375,6 +377,99 @@ static int lcp_stage(bwts_b200_ctx *ctx, cudaStream_t st, const u8 *dT, u32 n, c
     return 0;
 }
 
+// ---- LPF array and greedy LZ77 parse (lz.cuh) ----------------------------------------------------
+// lpf != nullptr: LPF and PREV into lpf / prev (text order).  Otherwise the parse: LPF / PREV into scratch,
+// z = the number of factors, and the pairs into factors when z <= cap (else BWTS_B200_EINVAL).
+struct LzOut {
+    i32 *lpf = nullptr, *prev = nullptr;
+    i32 *factors = nullptr;
+    long cap = 0;
+    long z = -1;
+};
+// scratch, all dead after the LCP stage: lpf / prev n words each (the parse only), w[0..5] n words each, e n
+// words, d[0..1] 2n words each, cnt 2 words
+struct LzScratch {
+    i32 *lpf, *prev;
+    u32 *w[6], *e;
+    u64 *d[2];
+    u32 *cnt;
+};
+// log2 of the tile / chunk width: bwts_b200_tune key 25, and no wider than the next power of two of n
+static u32 lz_tile_bits(u32 n)
+{
+    u32 tb = (g_tune_lz >= LZ_TB_MIN && g_tune_lz <= LZ_TB_MAX) ? (u32)g_tune_lz : (u32)LZ_TB_MAX;
+    while (tb > LZ_TB_MIN && (1u << (tb - 1)) >= n) tb--;
+    return tb;
+}
+// After the LCP stage, SA and LCP in rank order.  Booked to kernel class emit and the forward's phase 3.
+//   LPF: gtree n / 2 bytes at most (w[5]), top 16 P <= n + 32 bytes (e), the listed rows (w[4], d[0]).
+//   parse: X_1 .. X_L in w[0..5] (L <= 6: ceil(n / 32^6) <= 32), the entries of every level in e, chunk
+//   counts in d[0], offsets and tile sums in d[1].
+static int lz_stage(bwts_b200_ctx *ctx, cudaStream_t st, const u8 *dT, u32 n, const i32 *SA, const i32 *LCP, LzOut *lz,
+                    const LzScratch &s)
+{
+    const u32 tb = lz_tile_bits(n), W = 1u << tb, nt = cdiv(n, W);
+    u32 P = 1;
+    while (P < nt) P <<= 1;
+    uint2 *gtree = (uint2 *)s.w[5], *top = (uint2 *)s.e, *listP = (uint2 *)s.d[0];
+    u32 *listR = s.w[4];
+    i32 *lpf = lz->lpf ? lz->lpf : s.lpf, *prev = lz->lpf ? lz->prev : s.prev;
+    CK(cudaMemsetAsync(top, 0xff, (size_t)16 * P, st));
+    CK(cudaMemsetAsync(s.cnt, 0, 8, st));
+    // SA 4, LCP 4 (rank order), LPF 4 and PREV 4 (text order), the tree nodes over 32 rows 0.5
+    LAUNCH_SMEM(KC_EMIT, 16.5 * n, k_lpf_tile, nt, 1024, (size_t)16 * W, SA, LCP, n, tb, gtree, top, P, lpf, prev, listR,
+                listP, s.cnt);
+    for (u32 half = P / 2; half >= 1; half >>= 1) {
+        if (half <= 1024) {
+            LAUNCH(KC_EMIT, 48.0 * half, k_lpf_top, 1, 1024, top, half, 1u);
+            break;
+        }
+        LAUNCH(KC_EMIT, 24.0 * half, k_lpf_top, cdiv(half, 1024), 1024, top, half, 0u);
+    }
+    int rc = readback(ctx, st, s.cnt, 4);
+    if (rc) return rc;
+    const u32 m = ctx->h_small[0];
+    // per listed row: the list 12, SA 4, LPF / PREV 16, the tree walks and one group of 32 rows (~ 2 x 256)
+    if (m) LAUNCH(KC_EMIT, 540.0 * m, k_lpf_cross, cdiv(m, 256), 256, SA, LCP, n, tb, gtree, top, P, lpf, prev, listR, listP, m);
+    if (lz->lpf) return 0;
+
+    int L = 1;
+    while ((u64)cdiv(n, (u64)1 << (L * tb)) > W) L++;
+    if (L > 6) return BWTS_B200_EINTERNAL;
+    u32 *ent[7];
+    ent[1] = s.e;
+    for (int l = 1; l < L; l++) ent[l + 1] = ent[l] + cdiv(n, (u64)1 << (l * tb));
+    CK(cudaMemsetAsync(s.e, 0xff, (size_t)(ent[L] + cdiv(n, (u64)1 << (L * tb)) - s.e) * 4, st));
+    LAUNCH_SMEM(KC_EMIT, 8.0 * n, k_lz_exit1, nt, 256, (size_t)4 * W, lpf, n, tb, s.w[0]);
+    for (int l = 2; l <= L; l++)
+        for (u32 r = 0; r < tb; r++)
+            LAUNCH(KC_EMIT, 12.0 * n, k_lz_jump, cdiv(n, 256), 256, r == 0 ? s.w[l - 2] : s.w[l - 1], s.w[l - 1], n,
+                   (u32)(l * tb));
+    LAUNCH(KC_EMIT, 0, k_lz_top, 1, 1, s.w[L - 1], n, (u32)(L * tb), ent[L]);
+    for (int l = L; l >= 2; l--) {
+        const u32 nb = cdiv(n, (u64)1 << (l * tb));
+        LAUNCH(KC_EMIT, 8.0 * nb, k_lz_down, cdiv(nb, 256), 256, s.w[l - 2], n, (u32)(l * tb), (u32)((l - 1) * tb), ent[l],
+               nb, ent[l - 1]);
+    }
+    u32 *cnt = (u32 *)s.d[0], *off = (u32 *)s.d[1];
+    u32 *tiles = off + (((size_t)nt + 63) & ~(size_t)63);
+    const u32 ntl = cdiv(nt, SC_TILE);
+    LAUNCH_SMEM(KC_EMIT, 4.0 * n, k_lz_chunk<false>, nt, 256, (size_t)8 * W, dT, lpf, prev, n, tb, ent[1], cnt,
+                (const u32 *)nullptr, (i32 *)nullptr);
+    LAUNCH(KC_EMIT, 4.0 * nt, k_tile_sum_u32, ntl, 256, cnt, nt, tiles, nullptr);
+    LAUNCH(KC_EMIT, 8.0 * ntl, k_scan_excl_u32_block, 1, 1024, tiles, tiles, ntl, s.cnt + 1);
+    LAUNCH(KC_EMIT, 8.0 * nt, k_tile_scan_apply_u32, ntl, 256, cnt, off, nt, tiles);
+    rc = readback(ctx, st, s.cnt + 1, 4);
+    if (rc) return rc;
+    const u32 z = ctx->h_small[0];
+    lz->z = z;
+    if ((long)z > lz->cap) return BWTS_B200_EINVAL;
+    // LPF 4 per position, and per factor PREV or the byte, and the pair 8
+    LAUNCH_SMEM(KC_EMIT, 4.0 * n + 12.0 * z, k_lz_chunk<true>, nt, 256, (size_t)8 * W, dT, lpf, prev, n, tb, ent[1],
+                (u32 *)nullptr, off, lz->factors);
+    return 0;
+}
+
 // ---- forward ---------------------------------------------------------------------------------
 enum FwdMode {
     FWD_BWTS = 0,        // forward BWTS into d_out
@@ -383,12 +478,13 @@ enum FwdMode {
     FWD_BWTS_FLAGS = 3,  // forward BWTS, factor-start flags already in d_out (after FWD_LYNDON)
     FWD_BWT = 4,         // classic BWT into d_out: rotations of the one factor [0, n), *primary = rank[0]
     FWD_DIVBWT = 5,      // libdivsufsort's divbwt into d_out: the FWD_SA sort, bytes at shifted rows, *primary = rank[0] + 1
-    FWD_FM = 6           // FM-index build: the FWD_DIVBWT emit into d_out, then the suffix array into d_sa (fm_build)
+    FWD_FM = 6,          // FM-index build: the FWD_DIVBWT emit into d_out, then the suffix array into d_sa (fm_build)
+    FWD_LZ = 7           // the FWD_SA sort and LCP stage into scratch, then LPF / PREV or the LZ77 parse into *lz
 };
 static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 *d_sa, int mode, cudaStream_t st,
-                        long *primary = nullptr, i32 *d_lcp = nullptr)
+                        long *primary = nullptr, i32 *d_lcp = nullptr, LzOut *lz = nullptr)
 {
-    const int linear = (mode == FWD_SA || mode == FWD_LYNDON || mode == FWD_DIVBWT || mode == FWD_FM);
+    const int linear = (mode == FWD_SA || mode == FWD_LYNDON || mode == FWD_DIVBWT || mode == FWD_FM || mode == FWD_LZ);
     int rc = arena_reserve(ctx, workspace_bytes(n));
     if (rc) return rc;
     ctx->arena_used = 0;
@@ -964,10 +1060,18 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             *primary = (long)ctx->h_small[0];
         }
         if (mode == FWD_FM) LAUNCH(KC_EMIT, 8.0 * n, k_emit_sa, cdiv(n, 256), 256, rank, n, d_sa);
-    } else if (mode == FWD_SA) {
-        LAUNCH(KC_EMIT, 8.0 * n, k_emit_sa, cdiv(n, 256), 256, rank, n, d_sa);
-        if (d_lcp) {
-            rc = lcp_stage(ctx, st, dT, n, d_sa, d_lcp, sb.v[0], grp, gst, sb.k[0], sb.k[1], small + 128);
+    } else if (mode == FWD_SA || mode == FWD_LZ) {
+        // FWD_LZ: the suffix array and LCP array go to the S set's kS / vS, which the LCP stage does not use
+        i32 *sa_out = mode == FWD_LZ ? (i32 *)kS : d_sa, *lcp_out = mode == FWD_LZ ? (i32 *)vS : d_lcp;
+        LAUNCH(KC_EMIT, 8.0 * n, k_emit_sa, cdiv(n, 256), 256, rank, n, sa_out);
+        if (lcp_out) {
+            rc = lcp_stage(ctx, st, dT, n, sa_out, lcp_out, sb.v[0], grp, gst, sb.k[0], sb.k[1], small + 128);
+            if (rc) return rc;
+        }
+        if (mode == FWD_LZ) {
+            const LzScratch s = {(i32 *)rank, (i32 *)gid, {sb.v[1], FS, grpS, gstS, sb.v[0], grp}, gst, {sb.k[0], sb.k[1]},
+                                 small + 160};
+            rc = lz_stage(ctx, st, dT, n, sa_out, lcp_out, lz, s);
             if (rc) return rc;
         }
     } else {
@@ -1255,6 +1359,7 @@ extern "C" bwts_b200_ctx *bwts_b200_create(int device)
     cudaFuncSetAttribute(k_local_sort_cta_radix<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LsrSmem::bytes);
     cudaFuncSetAttribute(k_local_sort_cta<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(LS_CAP * sizeof(u64)));
     cudaFuncSetAttribute(k_local_sort_cta<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(LS_CAP * sizeof(u64)));
+    cudaFuncSetAttribute(k_lpf_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, 16 << LZ_TB_MAX);
 #undef OS_ATTR
     bwts_b200_ctx *ctx = new bwts_b200_ctx();
     ctx->device = device;
@@ -1999,6 +2104,129 @@ extern "C" int bwts_b200_sa_lcp(const unsigned char *T, int *SA, int *LCP, int n
     return rc ? rc : sa_default_ctx(T, SA, LCP, n, device);
 }
 
+// ---- longest-previous-factor array and LZ77 parse ---------------------------------------------------------------
+// the bwts_b200_sa_* rules: no two of in, lpf and prev share a byte
+static int check_lpf_args(const bwts_b200_ctx *ctx, const void *in, long len, const void *lpf, const void *prev)
+{
+    if (!ctx || !in || !lpf || !prev || len <= 0) return BWTS_B200_EINVAL;
+    if (len > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
+    const size_t n = (size_t)len;
+    if (spans_overlap(in, n, lpf, 4 * n) || spans_overlap(in, n, prev, 4 * n) || spans_overlap(lpf, 4 * n, prev, 4 * n))
+        return BWTS_B200_EINVAL;
+    return 0;
+}
+// in and factors[0 .. 2 cap) share no byte; z is required, cap >= 0
+static int check_lz_args(const bwts_b200_ctx *ctx, const void *in, long len, const void *factors, long cap, const long *z)
+{
+    if (!ctx || !in || !factors || !z || len <= 0 || cap < 0) return BWTS_B200_EINVAL;
+    if (len > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
+    if (spans_overlap(in, (size_t)len, factors, 8 * (size_t)min(cap, 1L << 56))) return BWTS_B200_EINVAL;
+    return 0;
+}
+
+static int run_lz_device(bwts_b200_ctx *ctx, const void *d_in, long len, LzOut *lz, void *stream)
+{
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    apply_device_limits();
+    ctx->io_in = nullptr;
+    int rc;
+    if ((uintptr_t)d_in & 15) {  // as run_device: an unaligned slice is copied to the bottom of the workspace
+        rc = arena_reserve(ctx, workspace_bytes((size_t)len) + 2 * (size_t)len + 1024);
+        if (rc) return rc;
+        ctx->io_bytes = ((size_t)len + 255) & ~(size_t)255;
+        CK(cudaMemcpyAsync(ctx->arena, d_in, (size_t)len, cudaMemcpyDeviceToDevice, st));
+        d_in = ctx->arena;
+        ctx->io_in = ctx->arena;
+    }
+    stats_begin(ctx, len, 0, st);
+    rc = forward_core(ctx, (const u8 *)d_in, (u32)len, nullptr, nullptr, FWD_LZ, st, nullptr, nullptr, lz);
+    ctx->io_in = nullptr;
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    stats_end(ctx, st);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
+    return 0;
+}
+
+// host buffers: the text and LPF + PREV, or up to n factor pairs, in the I/O region in front of the workspace,
+// 1 + 8 bytes per input byte; arguments already checked
+static int run_lz_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *lpf, int *prev, int *factors,
+                       long cap, long *z)
+{
+    CK(cudaSetDevice(ctx->device));
+    const size_t io = ((size_t)len + 255) & ~(size_t)255;
+    const size_t w_bytes = ((size_t)len * 4 + 255) & ~(size_t)255;
+    int rc = arena_reserve(ctx, workspace_bytes((size_t)len) + io + 2 * w_bytes + 1024);
+    if (rc) return rc;
+    ctx->io_bytes = ((io + 2 * w_bytes + 1) / 2 + 255) & ~(size_t)255;  // forward_core skips 2 * io_bytes
+    ctx->io_in = nullptr;
+    u8 *d_in = ctx->arena;
+    i32 *d_a = (i32 *)(ctx->arena + io), *d_b = (i32 *)(ctx->arena + io + w_bytes);
+    LzOut o;
+    if (lpf) { o.lpf = d_a; o.prev = d_b; }
+    else { o.factors = d_a; o.cap = cap; }
+    cudaStream_t st = ctx->own_stream;
+    apply_device_limits();
+    CK(cudaEventRecord(ctx->ev_io0, st));
+    rc = stage_h2d(ctx, d_in, in, (size_t)len, st);
+    if (rc) return rc;
+    ctx->io_in = d_in;
+    stats_begin(ctx, len, 0, st);
+    rc = forward_core(ctx, d_in, (u32)len, nullptr, nullptr, FWD_LZ, st, nullptr, nullptr, &o);
+    ctx->io_in = nullptr;
+    if (z && o.z >= 0) *z = o.z;
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    stats_end(ctx, st);
+    if (lpf) {
+        rc = stage_d2h(ctx, (u8 *)lpf, (const u8 *)d_a, (size_t)len * 4, st);
+        if (!rc) rc = stage_d2h(ctx, (u8 *)prev, (const u8 *)d_b, (size_t)len * 4, st);
+    } else if (o.z > 0) {
+        rc = stage_d2h(ctx, (u8 *)factors, (const u8 *)d_a, (size_t)o.z * 8, st);
+    }
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->ev_io1, st));
+    CK(cudaStreamSynchronize(st));
+    float t = 0;
+    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
+    if (cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
+    return 0;
+}
+
+extern "C" int bwts_b200_lpf_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *lpf, int *prev)
+{
+    const int rc = check_lpf_args(ctx, in, len, lpf, prev);
+    return rc ? rc : run_lz_host(ctx, in, len, lpf, prev, nullptr, 0, nullptr);
+}
+extern "C" int bwts_b200_lpf_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_lpf, void *d_prev, void *stream)
+{
+    const int rc = check_lpf_args(ctx, d_in, len, d_lpf, d_prev);
+    if (rc) return rc;
+    if (((uintptr_t)d_lpf & 3) || ((uintptr_t)d_prev & 3)) return BWTS_B200_EINVAL;
+    LzOut o;
+    o.lpf = (i32 *)d_lpf;
+    o.prev = (i32 *)d_prev;
+    return run_lz_device(ctx, d_in, len, &o, stream);
+}
+extern "C" int bwts_b200_lz77_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *factors, long cap, long *z)
+{
+    const int rc = check_lz_args(ctx, in, len, factors, cap, z);
+    return rc ? rc : run_lz_host(ctx, in, len, nullptr, nullptr, factors, cap, z);
+}
+extern "C" int bwts_b200_lz77_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_factors, long cap, long *z,
+                                     void *stream)
+{
+    int rc = check_lz_args(ctx, d_in, len, d_factors, cap, z);
+    if (rc) return rc;
+    if ((uintptr_t)d_factors & 3) return BWTS_B200_EINVAL;
+    LzOut o;
+    o.factors = (i32 *)d_factors;
+    o.cap = cap;
+    rc = run_lz_device(ctx, d_in, len, &o, stream);
+    if (o.z >= 0) *z = o.z;
+    return rc;
+}
+
 // ---- FM-index (fm.cuh) --------------------------------------------------------------------------------------
 // One cudaMalloc per index, laid out in this order, every array rounded up to 256 bytes:
 //     U n, S 4 sg (n/65536 + 1), B 2 sg (n/256 + 1), marks 4 ceil(n/32), dir 4 (n/256 + 1), samples 4 ceil(n/sample),
@@ -2408,5 +2636,10 @@ extern "C" int bwts_b200_tune(int key, long value)
     if (key == 16) { if (value < 0) return BWTS_B200_EINVAL; g_tune_invbudget = value; return 0; }
     if (key == 13) { if (value < 0) return BWTS_B200_EINVAL; g_tune_invq = value; return 0; }
     if (key == 24) { if (value < 0 || value > 2) return BWTS_B200_EINVAL; g_tune_lcp = value; return 0; }
+    if (key == 25) {
+        if (value != 0 && (value < LZ_TB_MIN || value > LZ_TB_MAX)) return BWTS_B200_EINVAL;
+        g_tune_lz = value;
+        return 0;
+    }
     return BWTS_B200_EINVAL;
 }

@@ -21,7 +21,10 @@
  *                       additive: the suffix array and the LCP array on the context, device and
  *                       one-call entry points (see the section below).
  *   bwts_b200_fm_*      additive: an FM-index over the divbwt output, counting and locating many
- *                       patterns on the GPU (see the last section).
+ *                       patterns on the GPU (see the section below).
+ *   bwts_b200_lpf_*, bwts_b200_lz77_*
+ *                       additive: the longest-previous-factor array and the greedy LZ77 parse,
+ *                       from the suffix array and LCP array on the GPU (see the last section).
  *
  * Byte layout is the reference's: `len` raw input bytes in, exactly `len` raw bytes
  * out, no header, no primary index, no terminator (mk_bwts_sa.c:60, unbwts.c:173).
@@ -210,7 +213,9 @@ const char *bwts_b200_version(void);
  * sweep over the keys (1) instead of the window histogram taken while the keys are built, 22 = initial keys of whole
  * symbols only (1; default: spare key bits hold the top bits of the next symbol), 23 = MiB of output per emit window
  * (16..1024; default 64: the scatter target of one sweep stays in L2), 24 = LCP array: every irreducible pair
- * through the warp tier (1) or the multi-CTA tier (2) instead of by its length.  value 0 = default. */
+ * through the warp tier (1) or the multi-CTA tier (2) instead of by its length, 25 = LPF array and LZ77 parse: log2 of
+ * the tile and chunk width (5..12; default 12), so that small inputs take the cross-tile and multi-level paths.
+ * value 0 = default. */
 int bwts_b200_tune(int key, long value);
 
 /* ---- "next" row (SURVEY.md 8f.2): suffix array behind libdivsufsort's own seam ----- */
@@ -363,6 +368,52 @@ int bwts_b200_fm_locate_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const i
                              int *pos, long cap, long *total);
 int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_range, long nrange,
                                void *d_pos, long cap, long *total, void *stream);
+
+/* ---- longest-previous-factor array and greedy LZ77 parse ------------------------------------ */
+/* Bytes compare as unsigned char and the end of text is smaller than every byte (the order of
+ * bwts_b200_sa_*); n = len, 1 <= len <= BWTS_B200_MAX_LEN; lcp(i, j) is the length of the longest
+ * common prefix of T[i..n) and T[j..n).
+ *     LPF[i]  = max over j < i of lcp(i, j): 0 for i = 0 and for a byte that has not occurred before.
+ *     PREV[i] = -1 when LPF[i] == 0.  Otherwise, among the j < i with lcp(i, j) == LPF[i]: if some of
+ *               their suffixes are smaller than T[i..n), the one whose suffix is the largest of those;
+ *               else the one whose suffix is the smallest.  (The previous smaller value in suffix array
+ *               order, else the next smaller value, the previous one on a tie.)
+ *     LZ77    the greedy parse, a source may overlap its factor: p_0 = 0; factor k at p_k is
+ *               (PREV[p_k], LPF[p_k]) when LPF[p_k] >= 1, else the literal (T[p_k], 0);
+ *               p_(k+1) = p_k + max(1, LPF[p_k]); z factors, int32 pairs (src_or_byte, len).
+ * Examples:  banana       LPF [0,0,0,3,2,1]  PREV [-1,-1,-1,1,2,3]  LZ77 (98,0) (97,0) (110,0) (1,3)
+ *            abracadabra  LPF [0,0,0,1,0,1,0,4,3,2,1]  PREV [-1,-1,-1,0,-1,3,-1,0,1,2,7]
+ *                         LZ77 (97,0) (98,0) (114,0) (0,1) (99,0) (3,1) (100,0) (0,4)
+ *            mississippi  LPF [0,0,0,1,4,3,2,1,0,1,1]  PREV [-1,-1,-1,2,1,2,3,4,-1,8,7]
+ *                         LZ77 (109,0) (105,0) (115,0) (2,1) (1,4) (112,0) (8,1) (7,1)
+ *            aaaa         LPF [0,3,2,1]  PREV [-1,0,1,2]  LZ77 (97,0) (0,3)
+ *            a            LPF [0]  PREV [-1]  LZ77 (97,0)
+ * and in general a^n gives LPF[i] = n - i, PREV[i] = i - 1 for i >= 1, LZ77 (97,0) (0,n-1).
+ *
+ * GPU path (DESIGN.md section 4.10): the suffix sort and LCP stage of bwts_b200_sa_lcp_*, then the
+ * previous / next smaller values in suffix array order with the LCP minimum over each span (a min tree per
+ * tile of 4096 rows in shared memory, a tree over the tiles for the rest), then the greedy parse by levels of
+ * pointer jumping over chunks of 4096 positions.  Both are O(n log n) for every input.
+ *
+ * Arguments follow bwts_b200_sa_*: a NULL ctx, in or output pointer, or len <= 0 is BWTS_B200_EINVAL,
+ * len > BWTS_B200_MAX_LEN is BWTS_B200_ETOOBIG; no two of in, lpf and prev may share a byte, nor in and
+ * factors[0 .. 2 cap) (BWTS_B200_EINVAL).  Device outputs must be 4-byte aligned, the input may lie at any
+ * offset.  LZ77: z must not be NULL and cap >= 0 (else BWTS_B200_EINVAL); *z is set to the number of factors
+ * whenever the parse ran; z > cap is BWTS_B200_EINVAL and nothing is written to factors.  z <= n, so
+ * cap = len always suffices.  Without a device every call returns BWTS_B200_ENODEV.
+ *
+ * Device memory: the device forms need the workspace of the SA call of the same length (71 bytes per input
+ * byte + 64 MiB) and nothing more for an input at a 16-byte aligned address (2 bytes per byte otherwise);
+ * every stage takes its scratch from the sort's buffers.  The host forms add an I/O region of 9 bytes per
+ * input byte (text, LPF and PREV, or up to n factor pairs): ~80 bytes per byte in all, 172 GB at
+ * len = 2^31 - 1, as bwts_b200_sa_lcp_host.
+ * Statistics: direction 0, factors = 1, longest_factor = n; the LPF and parse kernels (k_lpf_*, k_lz_*) are
+ * booked to kernel class "emit" and phase 3, beside k_lcp_*. */
+int bwts_b200_lpf_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *lpf, int *prev);
+int bwts_b200_lpf_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_lpf, void *d_prev, void *stream);
+int bwts_b200_lz77_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *factors, long cap, long *z);
+int bwts_b200_lz77_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_factors, long cap, long *z,
+                          void *stream);
 
 #ifdef __cplusplus
 }
