@@ -36,6 +36,7 @@ EXPORTS = [
     "bwts_b200_fm_build_host", "bwts_b200_fm_build_device", "bwts_b200_fm_free", "bwts_b200_fm_bytes",
     "bwts_b200_fm_count_host", "bwts_b200_fm_count_device", "bwts_b200_fm_locate_host", "bwts_b200_fm_locate_device",
     "bwts_b200_lpf_host", "bwts_b200_lpf_device", "bwts_b200_lz77_host", "bwts_b200_lz77_device",
+    "bwts_b200_lz77_decode_host", "bwts_b200_lz77_decode_device",
 ]
 
 
@@ -136,6 +137,8 @@ def lib():
     L.bwts_b200_lpf_device.argtypes = [vp, vp, cl, vp, vp, vp]
     L.bwts_b200_lz77_host.argtypes = [vp, vp, cl, vp, cl, ctypes.POINTER(cl)]
     L.bwts_b200_lz77_device.argtypes = [vp, vp, cl, vp, cl, ctypes.POINTER(cl), vp]
+    L.bwts_b200_lz77_decode_host.argtypes = [vp, vp, cl, vp, cl]
+    L.bwts_b200_lz77_decode_device.argtypes = [vp, vp, cl, vp, cl, vp]
     _lib = L
     return L
 
@@ -553,6 +556,19 @@ class Context:
         _check(lib().bwts_b200_lz77_device(self._h, d_in, length, d_factors, cap, ctypes.byref(z), stream),
                "bwts_b200_lz77_device")
         return z.value
+
+    def lz77_decode_host(self, factors, length):
+        """int32 [z, 2] factor pairs (source, length) or (byte, 0) -> the `length` bytes they decode to"""
+        f = np.ascontiguousarray(factors, dtype=np.int32).reshape(-1, 2)
+        out = np.empty(max(length, 1), dtype=np.uint8)
+        _check(lib().bwts_b200_lz77_decode_host(self._h, f.ctypes.data, len(f), out.ctypes.data, length),
+               "bwts_b200_lz77_decode_host")
+        return out[:length].tobytes()
+
+    def lz77_decode_device(self, d_factors, z, length, d_out, stream=None):
+        """z int32 pairs at d_factors (4-byte aligned) -> `length` bytes into d_out (any address)"""
+        _check(lib().bwts_b200_lz77_decode_device(self._h, d_factors, z, d_out, length, stream),
+               "bwts_b200_lz77_decode_device")
 
     # FM-index (include/bwts_b200.h, section before)
     def fm_build_host(self, data, sample=32):

@@ -24,6 +24,7 @@
 #include "inverse.cuh"
 #include "lcp.cuh"
 #include "lz.cuh"
+#include "lzd.cuh"
 #include "lyndon.cuh"
 #include "radix.cuh"
 #include "scan.cuh"
@@ -62,7 +63,7 @@ static long g_tune_invmark = 0;    // inverse staged walk marks: 0 = by size (co
 static long g_tune_invbudget = 0;  // inverse fallback walks: step budget per attempt (0 = 32 n)
 static long g_tune_nomark = 0;     // TIMING EXPERIMENT ONLY: inverse first walk without visited marks (wrong output when a cycle has no splitter)
 static long g_tune_lcp = 0;        // LCP pairs: 0 = by length through the three tiers, 1 = all from the warp tier on, 2 = all through the multi-CTA tier
-static long g_tune_lz = 0;         // LPF / LZ77: log2 of the tile and chunk width (5..12; 0 = 12)
+static long g_tune_lz = 0;         // LPF / LZ77 / LZ77 decoding: log2 of the tile and chunk width (5..12; 0 = 12)
 
 static void apply_device_limits()
 {
@@ -2556,6 +2557,120 @@ extern "C" int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm
     if (!rc) rc = fm_locate_core(ctx, fm, (const i32 *)d_range, nrange, (i32 *)d_pos, cap, total, st);
     if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
     return fm_query_end(ctx, st);
+}
+
+// ---- LZ77 decoding (lzd.cuh) -----------------------------------------------------------------------------------
+// Scratch at the arena's offset `at`: the words v, the starts p (z <= n), the two live lists, 4 n bytes each; the
+// tile sums, 8 per 4096 factors; 256 bytes of counters.
+static size_t lzd_scratch_bytes(size_t n)
+{
+    return 4 * r256(4 * n) + r256(8 * ((size_t)cdiv(n, LZD_TILE) + 1)) + 256;
+}
+// the bwts_b200_lz77_* rules: factors[0 .. 2z) and out[0 .. len) share no byte
+static int check_lzd_args(const bwts_b200_ctx *ctx, const void *factors, long z, const void *out, long len)
+{
+    if (!ctx || !factors || !out || z <= 0 || len <= 0) return BWTS_B200_EINVAL;
+    if (len > BWTS_B200_MAX_LEN) return BWTS_B200_ETOOBIG;
+    if (z > len || spans_overlap(factors, 8 * (size_t)z, out, (size_t)len)) return BWTS_B200_EINVAL;
+    return 0;
+}
+
+// d_f: z pairs on the device, 4-byte aligned; d_out: n bytes.  The content rules are checked before anything is
+// written to d_out.  Direction 1: the checks and the scan in class inv_scan / phase 0, the chunks in inv_walk / 2,
+// the global rounds in inv_jump / 3, the bytes in inv_place / 4.
+static int lzd_core(bwts_b200_ctx *ctx, const i32 *d_f, u32 z, u8 *d_out, u32 n, size_t at, cudaStream_t st)
+{
+    const u32 nt = cdiv(z, LZD_TILE);
+    u8 *a = ctx->arena + at;
+    u32 *v = (u32 *)a;                a += r256(4ull * n);
+    u32 *p = (u32 *)a;                a += r256(4ull * n);
+    u32 *live[2] = {(u32 *)a, nullptr}; a += r256(4ull * n);
+    live[1] = (u32 *)a;               a += r256(4ull * n);
+    u64 *tsum = (u64 *)a;             a += r256(8ull * (nt + 1));
+    u32 *cnt = (u32 *)a;  // [0] bad, [2..3] the sum of max(1, len_k), [4] / [5] the live counts
+    stats_begin(ctx, n, 1, st);
+    ctx->stats.factors = z;
+    CK(cudaMemsetAsync(cnt, 0, 32, st));
+    // pairs 8 per factor (twice), p 4, tile sums
+    LAUNCH(KC_INV_SCAN, 8.0 * z + 8.0 * nt, k_lzd_tile_sum, nt, 256, d_f, (u64)z, tsum, cnt);
+    LAUNCH(KC_INV_SCAN, 16.0 * nt, k_lzd_tile_scan, 1, 1024, tsum, nt, (u64 *)(cnt + 2));
+    LAUNCH(KC_INV_SCAN, 12.0 * z + 8.0 * nt, k_lzd_apply, nt, 256, d_f, (u64)z, tsum, p, cnt);
+    int rc = readback(ctx, st, cnt, 16);
+    if (rc) return rc;
+    if (ctx->h_small[0] || h_small_u64(ctx, 2) != n) return BWTS_B200_EINVAL;
+
+    const u32 tb = lz_tile_bits(n), nc = cdiv(n, 1u << tb);
+    ctx->phase = 2;
+    // per position the word 4 and the live entry 4 (at most), per factor its start 4 and its pair 8
+    LAUNCH_SMEM(KC_INV_WALK, 8.0 * n + 12.0 * z, k_lzd_chunk, nc, 256, (size_t)8 << tb, d_f, p, z, n, tb, v, live[0],
+                cnt + 4);
+    rc = readback(ctx, st, cnt + 4, 4);
+    if (rc) return rc;
+    u32 m = ctx->h_small[0];
+    const int bound = bit_length((u64)nc - 1) + 1;  // ceil(log2 nc) + 1
+    ctx->phase = 3;
+    int cur = 0;
+    while (m) {
+        if (ctx->stats.rounds == bound) return BWTS_B200_EINTERNAL;
+        CK(cudaMemsetAsync(cnt + 5 - cur, 0, 4, st));
+        // the list 4, the two words read 8, the word written 4, the next list 4 (at most)
+        LAUNCH(KC_INV_JUMP, 20.0 * m, k_lzd_jump, cdiv(m, 256), 256, v, live[cur], m, live[cur ^ 1], cnt + 5 - cur);
+        ctx->stats.rounds++;
+        ctx->stats.live_sum += m;
+        rc = readback(ctx, st, cnt + 5 - cur, 4);
+        if (rc) return rc;
+        m = ctx->h_small[0];
+        cur ^= 1;
+    }
+    ctx->phase = 4;
+    LAUNCH(KC_INV_PLACE, 5.0 * n, k_lzd_bytes, cdiv(n, 1024), 256, v, n, d_out);
+    return 0;
+}
+
+extern "C" int bwts_b200_lz77_decode_host(bwts_b200_ctx *ctx, const int *factors, long z, unsigned char *out, long len)
+{
+    int rc = check_lzd_args(ctx, factors, z, out, len);
+    if (rc) return rc;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    CK(cudaSetDevice(ctx->device));
+    // I/O region: the pairs, then the text
+    const size_t fb = r256(8 * (size_t)z), io = fb + r256((size_t)len);
+    rc = arena_reserve(ctx, io + lzd_scratch_bytes((size_t)len));
+    if (rc) return rc;
+    i32 *d_f = (i32 *)ctx->arena;
+    u8 *d_out = ctx->arena + fb;
+    cudaStream_t st = ctx->own_stream;
+    CK(cudaEventRecord(ctx->ev_io0, st));
+    rc = stage_h2d(ctx, (u8 *)d_f, (const u8 *)factors, 8 * (size_t)z, st);
+    if (!rc) rc = lzd_core(ctx, d_f, (u32)z, d_out, (u32)len, io, st);
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    stats_end(ctx, st);
+    rc = stage_d2h(ctx, out, d_out, (size_t)len, st);
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->ev_io1, st));
+    CK(cudaStreamSynchronize(st));
+    float t = 0;
+    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
+    if (cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
+    return 0;
+}
+extern "C" int bwts_b200_lz77_decode_device(bwts_b200_ctx *ctx, const void *d_factors, long z, void *d_out, long len,
+                                            void *stream)
+{
+    int rc = check_lzd_args(ctx, d_factors, z, d_out, len);
+    if (rc) return rc;
+    if ((uintptr_t)d_factors & 3) return BWTS_B200_EINVAL;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    CK(cudaSetDevice(ctx->device));
+    rc = arena_reserve(ctx, lzd_scratch_bytes((size_t)len));
+    if (rc) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    rc = lzd_core(ctx, (const i32 *)d_factors, (u32)z, (u8 *)d_out, (u32)len, 0, st);
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    stats_end(ctx, st);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
+    return 0;
 }
 
 // ---- introspection --------------------------------------------------------------------------------------

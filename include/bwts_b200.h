@@ -150,11 +150,11 @@ typedef struct {
     long   longest_factor;      /* forward only                                         */
     int    alphabet_bits;       /* forward: bits per packed symbol                      */
     int    initial_depth;       /* forward: symbols in the initial key (k0)             */
-    int    rounds;              /* forward: doubling rounds after the initial sort      */
+    int    rounds;              /* forward: doubling rounds after the initial sort; LZ77 decoding: global jumping rounds */
     int    radix_passes;        /* forward: onesweep passes launched                    */
     int    local_rounds;        /* forward: rounds served by the warp-local sort        */
     int    cta_rounds;          /* forward: rounds whose large-group set was sorted CTA-locally */
-    long   live_sum;            /* forward: sum over rounds of live elements            */
+    long   live_sum;            /* forward: sum over rounds of live elements; LZ77 decoding: of live positions */
     long   splitters;           /* inverse: sublists                                    */
     long   unreached;           /* inverse: elements ranked by the self-walk fallback   */
     long   launches;            /* kernels launched by the last transform               */
@@ -214,7 +214,8 @@ const char *bwts_b200_version(void);
  * symbols only (1; default: spare key bits hold the top bits of the next symbol), 23 = MiB of output per emit window
  * (16..1024; default 64: the scatter target of one sweep stays in L2), 24 = LCP array: every irreducible pair
  * through the warp tier (1) or the multi-CTA tier (2) instead of by its length, 25 = LPF array and LZ77 parse: log2 of
- * the tile and chunk width (5..12; default 12), so that small inputs take the cross-tile and multi-level paths.
+ * the tile and chunk width (5..12; default 12), so that small inputs take the cross-tile and multi-level paths; it also
+ * sets LZ77 decoding's chunk width, so that small inputs take the global jumping rounds.
  * value 0 = default. */
 int bwts_b200_tune(int key, long value);
 
@@ -414,6 +415,40 @@ int bwts_b200_lpf_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d
 int bwts_b200_lz77_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *factors, long cap, long *z);
 int bwts_b200_lz77_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_factors, long cap, long *z,
                           void *stream);
+
+/* ---- LZ77 decoding: a factor list back into its text ---------------------------------------- */
+/* factors holds z int32 pairs in the parse's format above.  Factor k starts at p_k: p_0 = 0,
+ * p_(k+1) = p_k + max(1, len_k).  (byte, 0) is a literal, out[p_k] = byte; (src, len) with len >= 1 is a copy,
+ * out[p_k + j] = out[src + j] for j = 0 .. len - 1, applied byte by byte, so src + j may lie inside the factor
+ * itself.  Any valid factorization decodes, greedy or not: literals where a match exists, short copies, lists
+ * of other LZ77 tools that use this convention.
+ * Examples:  (98,0) (97,0) (110,0) (1,3)                                 -> banana
+ *            (97,0) (98,0) (114,0) (0,1) (99,0) (3,1) (100,0) (0,4)      -> abracadabra
+ *            (109,0) (105,0) (115,0) (2,1) (1,4) (112,0) (8,1) (7,1)     -> mississippi
+ *            (97,0) (0,3)                                                -> aaaa
+ * and in general (97,0) (0,n-1) -> a^n.
+ *
+ * Arguments: a NULL ctx, factors or out, z <= 0, len <= 0, z > len, factors[0 .. 2z) sharing a byte with
+ * out[0 .. len), or device factors that are not 4-byte aligned are BWTS_B200_EINVAL; len > BWTS_B200_MAX_LEN is
+ * BWTS_B200_ETOOBIG.  out may lie at any address.  Without a device both calls return BWTS_B200_ENODEV after these
+ * checks.  Content: a literal byte outside [0, 255], a negative length, a copy source outside [0, p_k), or
+ * sum of max(1, len_k) != len is BWTS_B200_EINVAL.  Both forms check these on the GPU before anything is written:
+ * nothing is written to out (the host form copies nothing back).
+ *
+ * GPU path (DESIGN.md section 4.11): a 64-bit scan of the lengths gives p_k; one CTA per chunk of 4096 positions
+ * finds each position's factor and resolves the copies inside the chunk by pointer jumping in shared memory; the
+ * positions left point into earlier chunks and are resolved by at most ceil(log2 ceil(len / 4096)) + 1 rounds of
+ * pointer jumping in global memory.  O(len log len) for every input, whatever the factor lengths.
+ *
+ * Device memory, from the context's workspace (which never shrinks): 16 len + 8 ceil(len / 4096) + 1539 bytes at
+ * most, less than any forward transform of the same length needs, so a context that has run one of length >= len
+ * decodes without allocating.  The host form adds an I/O region of 8 z + len bytes (each rounded up to 256).
+ * Statistics: direction 1, len = n, factors = z; rounds = the global jumping rounds launched and live_sum the sum
+ * of their live positions.  The checks and the scan are booked to class "inv_scan" and phase 0, the chunks to
+ * "inv_walk" and phase 2, the global rounds to "inv_jump" and phase 3, the byte writes to "inv_place" and phase 4. */
+int bwts_b200_lz77_decode_host(bwts_b200_ctx *ctx, const int *factors, long z, unsigned char *out, long len);
+int bwts_b200_lz77_decode_device(bwts_b200_ctx *ctx, const void *d_factors, long z, void *d_out, long len,
+                                 void *stream);
 
 #ifdef __cplusplus
 }
