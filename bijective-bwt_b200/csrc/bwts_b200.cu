@@ -82,7 +82,7 @@ static bool use_binned_scatter(unsigned n, unsigned kb)
     return g_tune_scatterbin == 2 || g_tune_scatterbin == 4 || n >= (1u << 22);
 }
 
-struct LaunchRec { int cls; double bytes; cudaEvent_t e0, e1; const char *name = ""; int phase = 0; };
+struct LaunchRec { int cls; double bytes; cudaEvent_t e0, e1; const char *name; int phase; };
 
 struct bwts_b200_ctx {
     int device = 0;
@@ -90,8 +90,7 @@ struct bwts_b200_ctx {
     cudaStream_t own_stream = nullptr;
     u8 *arena = nullptr;
     size_t arena_bytes = 0, arena_used = 0;
-    u8 *io_in = nullptr;     // host-buffer API: start of the I/O region at the bottom of the arena (while a call runs)
-    size_t io_bytes = 0;
+    size_t io_end = 0;       // bytes at the bottom of the arena that hold the running call's I/O region (0: none)
     u32 *h_small = nullptr;  // pinned + mapped, 4 KiB, for counter read-backs
     u32 *h_small_dev = nullptr;  // its device-side address
     int last_cuda = 0;
@@ -142,28 +141,23 @@ static cudaError_t launch_check(const char *name, cudaStream_t st)
     return e;
 }
 
-// LAUNCH(class, algorithmic bytes, kernel, grid, block, args...)
-#define LAUNCH(KCLS_, NBYTES_, kern, grid, block, ...)                               \
+// LAUNCH_REC(class, algorithmic bytes, name, launch): books the launch statement under the current phase, between
+// two events when profiling
+#define LAUNCH_REC(KCLS_, NBYTES_, NAME_, ...)                                       \
     do {                                                                             \
-        LaunchRec r__;                                                               \
-        r__.cls = (KCLS_); r__.bytes = (double)(NBYTES_); r__.e0 = r__.e1 = nullptr; r__.name = #kern; \
+        LaunchRec r__{(KCLS_), (double)(NBYTES_), nullptr, nullptr, (NAME_), ctx->phase}; \
         if (ctx->profile) { r__.e0 = ctx_event(ctx); if (r__.e0) cudaEventRecord(r__.e0, st); } \
-        kern<<<(grid), (block), 0, st>>>(__VA_ARGS__);                               \
-        if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); } \
-        r__.phase = ctx->phase; ctx->recs.push_back(r__);                                                    \
-        CK(launch_check(#kern, st));                                                 \
+        __VA_ARGS__;                                                                 \
+        if (r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); } \
+        ctx->recs.push_back(r__);                                                    \
+        CK(launch_check((NAME_), st));                                               \
     } while (0)
 
-#define LAUNCH_SMEM(KCLS_, NBYTES_, kern, grid, block, smem_, ...)                   \
-    do {                                                                             \
-        LaunchRec r__;                                                               \
-        r__.cls = (KCLS_); r__.bytes = (double)(NBYTES_); r__.e0 = r__.e1 = nullptr; r__.name = #kern; \
-        if (ctx->profile) { r__.e0 = ctx_event(ctx); if (r__.e0) cudaEventRecord(r__.e0, st); } \
-        kern<<<(grid), (block), (smem_), st>>>(__VA_ARGS__);                         \
-        if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); } \
-        r__.phase = ctx->phase; ctx->recs.push_back(r__);                                                    \
-        CK(launch_check(#kern, st));                                                 \
-    } while (0)
+// LAUNCH(class, algorithmic bytes, kernel, grid, block, args...)
+#define LAUNCH(KCLS_, NBYTES_, kern, grid, block, ...) \
+    LAUNCH_REC(KCLS_, NBYTES_, #kern, kern<<<(grid), (block), 0, st>>>(__VA_ARGS__))
+#define LAUNCH_SMEM(KCLS_, NBYTES_, kern, grid, block, smem_, ...) \
+    LAUNCH_REC(KCLS_, NBYTES_, #kern, kern<<<(grid), (block), (smem_), st>>>(__VA_ARGS__))
 
 static void stats_begin(bwts_b200_ctx *ctx, long len, int direction, cudaStream_t st)
 {
@@ -234,6 +228,7 @@ static size_t workspace_bytes(size_t n)
 }
 
 static inline u32 cdiv(u64 a, u64 b) { return (u32)((a + b - 1) / b); }
+static size_t r256(size_t b) { return (b + 255) & ~(size_t)255; }
 // look-back status of a re-rank over m slots: one word per tile + one per block of 32 tiles (forward.cuh)
 static inline size_t rr_status_bytes(u32 m)
 {
@@ -292,18 +287,10 @@ static int radix_sort(bwts_b200_ctx *ctx, cudaStream_t st, SortBufs &sb, u32 m, 
         do { ctx->epoch = (g_epoch.fetch_add(1) + 1) & 0x3fffffffu; } while (ctx->epoch == 0);
         const u32 *vin = ident ? (const u32 *)nullptr : sb.v[a];
         const double bytes = (ident ? 20.0 : 24.0) * m;
-#define OS_LAUNCH(NT_, IPT_, MINB_, LB_)                                                                  \
-    do {                                                                                                  \
-        LaunchRec r__;                                                                                    \
-        r__.cls = KC_ONESWEEP; r__.bytes = bytes; r__.e0 = r__.e1 = nullptr; r__.name = "k_onesweep_pass<u64>";  \
-        if (ctx->profile) { r__.e0 = ctx_event(ctx); if (r__.e0) cudaEventRecord(r__.e0, st); }           \
-        k_onesweep_pass<u64, NT_, IPT_, MINB_, LB_><<<cdiv(m, (NT_) * (IPT_)), NT_, OsSmem<u64, NT_, IPT_>::bytes, st>>>( \
-            sb.k[a], vin, sb.k[b], sb.v[b], m, (u32)(p * RADIX_BITS), sb.hist + p * RADIX_BINS, sb.status,  \
-            ctx->epoch);                                                                                  \
-        if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); } \
-        r__.phase = ctx->phase; ctx->recs.push_back(r__);                                                                         \
-        CK(cudaGetLastError());                                                                           \
-    } while (0)
+#define OS_LAUNCH(NT_, IPT_, MINB_, LB_)                                                                           \
+    LAUNCH_REC(KC_ONESWEEP, bytes, "k_onesweep_pass<u64>",                                                          \
+               k_onesweep_pass<u64, NT_, IPT_, MINB_, LB_><<<cdiv(m, (NT_) * (IPT_)), NT_, OsSmem<u64, NT_, IPT_>::bytes, st>>>( \
+                   sb.k[a], vin, sb.k[b], sb.v[b], m, (u32)(p * RADIX_BITS), sb.hist + p * RADIX_BINS, sb.status, ctx->epoch))
         switch (g_tune_onesweep) {
         case 1: OS_LAUNCH(512, 8, 3, 8); break;
         case 2: OS_LAUNCH(256, 16, 3, 8); break;
@@ -488,8 +475,7 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
     const int linear = (mode == FWD_SA || mode == FWD_LYNDON || mode == FWD_DIVBWT || mode == FWD_FM || mode == FWD_LZ);
     int rc = arena_reserve(ctx, workspace_bytes(n));
     if (rc) return rc;
-    ctx->arena_used = 0;
-    if (ctx->io_in && ctx->io_in == dT) ctx->arena_used = ((size_t)2 * ctx->io_bytes + 511) & ~(size_t)255;
+    ctx->arena_used = ctx->io_end;
 
     const u32 ntl = cdiv(n, FL_TILE);
     const u32 nblk = cdiv(n, 1u << COARSE_BITS);
@@ -734,14 +720,9 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             LAUNCH(KC_RERANK, 0, k_radix_hist_scan, 1, 256, sb.hist);
         }
         do { ctx->epoch = (g_epoch.fetch_add(1) + 1) & 0x3fffffffu; } while (ctx->epoch == 0);
-        LaunchRec r__;
-        r__.cls = KC_RERANK; r__.bytes = 16.0 * m; r__.e0 = r__.e1 = nullptr; r__.name = "k_onesweep_pass<u32> bin";
-        if (ctx->profile) { r__.e0 = ctx_event(ctx); if (r__.e0) cudaEventRecord(r__.e0, st); }
-        k_onesweep_pass<u32, 384, 12, 3, 4><<<cdiv(m, 384 * 12), 384, OsSmem<u32, 384, 12>::bytes, st>>>(
-            pos, nr, bin_pos, bin_val, m, shift, sb.hist, sb.status, ctx->epoch);
-        if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); }
-        r__.phase = ctx->phase; ctx->recs.push_back(r__);
-        CK(cudaGetLastError());
+        LAUNCH_REC(KC_RERANK, 16.0 * m, "k_onesweep_pass<u32> bin",
+                   k_onesweep_pass<u32, 384, 12, 3, 4><<<cdiv(m, 384 * 12), 384, OsSmem<u32, 384, 12>::bytes, st>>>(
+                       pos, nr, bin_pos, bin_val, m, shift, sb.hist, sb.status, ctx->epoch));
         LAUNCH(KC_RERANK, 12.0 * m, k_scatter_pairs, cdiv(cdiv(m, 8), 256), 256, bin_pos, bin_val, m, rank);
         ctx->stats.binned_rounds++;
         return 0;
@@ -942,28 +923,16 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
                 rc = readback(ctx, st, small + 5, 4);
                 if (rc) return rc;
                 if (ctx->h_small[0] == 0) {
-                    LaunchRec r__;
-                    r__.cls = KC_LOCAL_SORT; r__.bytes = 32.0 * mL; r__.e0 = r__.e1 = nullptr; r__.name = "k_local_sort_cta";
-                    if (ctx->profile) { r__.e0 = ctx_event(ctx); if (r__.e0) cudaEventRecord(r__.e0, st); }
-                    if (g_tune_ctasort == 1) {  // the bitonic network of round 1
-                        if (!linear)
-                            k_local_sort_cta<false><<<cdiv(mL, LS_T), LS_NT, LS_CAP * sizeof(u64), st>>>(
-                                sb.v[sb.cur], gst, mL, rank, FS, cidx, (u32)k, kb, n, sb.k[sb.cur ^ 1], sb.v[sb.cur ^ 1]);
-                        else
-                            k_local_sort_cta<true><<<cdiv(mL, LS_T), LS_NT, LS_CAP * sizeof(u64), st>>>(
-                                sb.v[sb.cur], gst, mL, rank, FS, cidx, (u32)k, kb, n, sb.k[sb.cur ^ 1], sb.v[sb.cur ^ 1]);
-                    } else {
-                        r__.name = "k_local_sort_cta_radix";
-                        if (!linear)
-                            k_local_sort_cta_radix<false><<<cdiv(mL, LS_T), LSR_NT, LsrSmem::bytes, st>>>(
-                                sb.v[sb.cur], gst, mL, rank, FS, cidx, (u32)k, kb, n, sb.k[sb.cur ^ 1], sb.v[sb.cur ^ 1]);
-                        else
-                            k_local_sort_cta_radix<true><<<cdiv(mL, LS_T), LSR_NT, LsrSmem::bytes, st>>>(
-                                sb.v[sb.cur], gst, mL, rank, FS, cidx, (u32)k, kb, n, sb.k[sb.cur ^ 1], sb.v[sb.cur ^ 1]);
-                    }
-                    if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); }
-                    r__.phase = ctx->phase; ctx->recs.push_back(r__);
-                    CK(cudaGetLastError());
+                    if (g_tune_ctasort == 1)  // the bitonic network of round 1
+                        LAUNCH_REC(KC_LOCAL_SORT, 32.0 * mL, "k_local_sort_cta",
+                                   (!linear ? k_local_sort_cta<false> : k_local_sort_cta<true>)
+                                       <<<cdiv(mL, LS_T), LS_NT, LS_CAP * sizeof(u64), st>>>(
+                                       sb.v[sb.cur], gst, mL, rank, FS, cidx, (u32)k, kb, n, sb.k[sb.cur ^ 1], sb.v[sb.cur ^ 1]));
+                    else
+                        LAUNCH_REC(KC_LOCAL_SORT, 32.0 * mL, "k_local_sort_cta_radix",
+                                   (!linear ? k_local_sort_cta_radix<false> : k_local_sort_cta_radix<true>)
+                                       <<<cdiv(mL, LS_T), LSR_NT, LsrSmem::bytes, st>>>(
+                                       sb.v[sb.cur], gst, mL, rank, FS, cidx, (u32)k, kb, n, sb.k[sb.cur ^ 1], sb.v[sb.cur ^ 1]));
                     sb.cur ^= 1;
                     ctx->stats.cta_rounds++;
                     cta_sorted = true;
@@ -1006,14 +975,9 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             const u32 shift = kb - 8;
             LAUNCH(KC_EMIT, 0, k_bin_bases, 1, 256, n, shift, sb.hist);
             do { ctx->epoch = (g_epoch.fetch_add(1) + 1) & 0x3fffffffu; } while (ctx->epoch == 0);
-            LaunchRec r__;
-            r__.cls = KC_EMIT; r__.bytes = 9.0 * n; r__.e0 = r__.e1 = nullptr; r__.name = "k_onesweep_pass<u32> pack";
-            if (ctx->profile) { r__.e0 = ctx_event(ctx); if (r__.e0) cudaEventRecord(r__.e0, st); }
-            k_onesweep_pass<u32, 384, 12, 3, 4, 2><<<cdiv(n, 384 * 12), 384, OsSmem<u32, 384, 12>::bytes, st>>>(
-                rank, (const u32 *)dT, (u32 *)nullptr, packed, n, shift, sb.hist, sb.status, ctx->epoch);
-            if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); }
-            r__.phase = ctx->phase; ctx->recs.push_back(r__);
-            CK(cudaGetLastError());
+            LAUNCH_REC(KC_EMIT, 9.0 * n, "k_onesweep_pass<u32> pack",
+                       k_onesweep_pass<u32, 384, 12, 3, 4, 2><<<cdiv(n, 384 * 12), 384, OsSmem<u32, 384, 12>::bytes, st>>>(
+                           rank, (const u32 *)dT, (u32 *)nullptr, packed, n, shift, sb.hist, sb.status, ctx->epoch));
             if (div) LAUNCH(KC_EMIT, 5.0 * n, k_scatter_packed<true>, cdiv(cdiv(n, 4), 256), 256, packed, n, shift, d_out, rank);
             else LAUNCH(KC_EMIT, 5.0 * n, k_scatter_packed, cdiv(cdiv(n, 4), 256), 256, packed, n, shift, d_out);
         } else if (emit_binned && kb >= 8) {
@@ -1024,14 +988,9 @@ static int forward_core(bwts_b200_ctx *ctx, const u8 *dT, u32 n, u8 *d_out, i32 
             LAUNCH(KC_EMIT, 5.0 * n, k_emit_vals, cdiv(cdiv(n, 4), 256), 256, dT, n, val);
             LAUNCH(KC_EMIT, 0, k_bin_bases, 1, 256, n, shift, sb.hist);
             do { ctx->epoch = (g_epoch.fetch_add(1) + 1) & 0x3fffffffu; } while (ctx->epoch == 0);
-            LaunchRec r__;
-            r__.cls = KC_EMIT; r__.bytes = 16.0 * n; r__.e0 = r__.e1 = nullptr; r__.name = "k_onesweep_pass<u32> bin";
-            if (ctx->profile) { r__.e0 = ctx_event(ctx); if (r__.e0) cudaEventRecord(r__.e0, st); }
-            k_onesweep_pass<u32, 384, 12, 3, 4><<<cdiv(n, 384 * 12), 384, OsSmem<u32, 384, 12>::bytes, st>>>(
-                rank, val, bin_pos, bin_val, n, shift, sb.hist, sb.status, ctx->epoch);
-            if (ctx->profile && r__.e0) { r__.e1 = ctx_event(ctx); if (r__.e1) cudaEventRecord(r__.e1, st); }
-            r__.phase = ctx->phase; ctx->recs.push_back(r__);
-            CK(cudaGetLastError());
+            LAUNCH_REC(KC_EMIT, 16.0 * n, "k_onesweep_pass<u32> bin",
+                       k_onesweep_pass<u32, 384, 12, 3, 4><<<cdiv(n, 384 * 12), 384, OsSmem<u32, 384, 12>::bytes, st>>>(
+                           rank, val, bin_pos, bin_val, n, shift, sb.hist, sb.status, ctx->epoch));
             if (div) LAUNCH(KC_EMIT, 9.0 * n, k_scatter_bytes<true>, cdiv(cdiv(n, 4), 256), 256, bin_pos, bin_val, n, d_out, rank);
             else LAUNCH(KC_EMIT, 9.0 * n, k_scatter_bytes, cdiv(cdiv(n, 4), 256), 256, bin_pos, bin_val, n, d_out);
         } else {
@@ -1297,8 +1256,7 @@ static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cuda
     u32 shift = g_tune_spl_shift ? (u32)g_tune_spl_shift : (n >= (1u << 28) ? 25u : 26u);
     ctx->stats.inverse_attempts = 0;
     for (int a = 0; a < 4; a++) {
-        ctx->arena_used = 0;
-        if (ctx->io_in && ctx->io_in == dB) ctx->arena_used = ((size_t)2 * ctx->io_bytes + 511) & ~(size_t)255;
+        ctx->arena_used = ctx->io_end;
         const u64 steps = g_tune_invbudget > 0 ? (u64)g_tune_invbudget : 32ull * n;
         u64 bk64 = steps >> 10;
         if (bk64 < 1) bk64 = 1;
@@ -1322,7 +1280,7 @@ static int inverse_core(bwts_b200_ctx *ctx, const u8 *dB, u32 n, u8 *d_out, cuda
             u64 slot2 = (4ull << (32 - s2)) & ~31ull;
             if (slot2 < 32) slot2 = 32;
             if (slot2 > INV_SLOT_MAX) slot2 = INV_SLOT_MAX;
-            const u64 need = (primary >= 0 ? 35ull : 34ull) * n + ns2 * (80 + slot2) * 5 / 4 + (ctx->io_in ? 2 * (u64)ctx->io_bytes : 0) + (16u << 20);
+            const u64 need = (primary >= 0 ? 35ull : 34ull) * n + ns2 * (80 + slot2) * 5 / 4 + ctx->io_end + (16u << 20);
             if (need <= ctx->arena_bytes) shift = s2;
         }
     }
@@ -1403,6 +1361,84 @@ extern "C" int bwts_b200_reserve(bwts_b200_ctx *ctx, long max_len)
     return arena_reserve(ctx, workspace_bytes((size_t)max_len) + 2 * (size_t)max_len + 1024);
 }
 
+// ---- the call frame --------------------------------------------------------------------------------
+// host <-> device copies of the host-buffer entry points: pinned buffers go as one async copy,
+// pageable ones (the tools' mmap'ed input, map_file.c, and malloc'ed output) through the context's
+// ring of pinned chunks -- the memcpy into chunk c+1 runs while chunk c is on the bus, where a
+// pageable cudaMemcpy stages serially inside the driver.  Defined behind PinnedRing.
+static int stage_h2d(bwts_b200_ctx *ctx, u8 *d_dst, const u8 *src, size_t len, cudaStream_t st);
+static int stage_d2h(bwts_b200_ctx *ctx, u8 *dst, const u8 *d_src, size_t len, cudaStream_t st);
+
+// copies into the arena at byte `at` before the core runs, and out of it after
+struct CopyIn { size_t at; const void *src; size_t bytes; };
+struct CopyOut { size_t at; void *dst; size_t bytes; };
+// What an entry point states about one call: the stats header, the arena bytes it reserves (workspace and I/O
+// region), the I/O region's end (the cores allocate their workspace from there up) and its copies.  A host form
+// copies in[] host -> device and out[] device -> host, timed into stats.h2d_ms / d2h_ms; a device form copies in[]
+// device -> device (an input its kernels cannot read where it lies) and has no out[].
+struct Frame {
+    long len;
+    int direction;
+    size_t arena, io_end;
+    bool host;
+    CopyIn in[2];
+    CopyOut out[2];  // the core may set the sizes of what is known only once it has run
+};
+
+// The bracket around every entry point's core: device, stream (stream: a device form's, else nullptr for the
+// context's own), workspace, limits, copies in, stats, core, stats, copies out.  On an error of the core the stream
+// is drained, the error cleared and the code returned without stats_end.
+template <typename Core>
+static int run_frame(bwts_b200_ctx *ctx, void *stream, Frame &f, Core &&core)
+{
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
+    int rc = arena_reserve(ctx, f.arena);
+    if (rc) return rc;
+    apply_device_limits();
+    if (f.host) CK(cudaEventRecord(ctx->ev_io0, st));
+    for (const CopyIn &c : f.in) {
+        if (!c.bytes) continue;
+        if (!f.host) CK(cudaMemcpyAsync(ctx->arena + c.at, c.src, c.bytes, cudaMemcpyDeviceToDevice, st));
+        else if ((rc = stage_h2d(ctx, ctx->arena + c.at, (const u8 *)c.src, c.bytes, st))) return rc;
+    }
+    ctx->io_end = f.io_end;
+    stats_begin(ctx, f.len, f.direction, st);
+    rc = core(st);
+    ctx->io_end = 0;
+    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
+    stats_end(ctx, st);
+    if (!f.host) {
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
+        return 0;
+    }
+    size_t copied = 0;
+    for (const CopyOut &c : f.out) {
+        if (!c.bytes) continue;
+        if ((rc = stage_d2h(ctx, (u8 *)c.dst, ctx->arena + c.at, c.bytes, st))) return rc;
+        copied += c.bytes;
+    }
+    CK(cudaEventRecord(ctx->ev_io1, st));
+    CK(cudaStreamSynchronize(st));
+    float t = 0;
+    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
+    if (copied && cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
+    return 0;
+}
+
+// A device form over a text.  The text kernels read 16-byte vectors: a text that is not 16-byte aligned (a slice
+// of a larger buffer) is first copied to the bottom of the arena, and the core reads it there.
+template <typename Core>
+static int run_text_device(bwts_b200_ctx *ctx, const void *d_in, long len, int direction, void *stream, Core &&core)
+{
+    const bool copy = (uintptr_t)d_in & 15;
+    Frame f = {len, direction, workspace_bytes((size_t)len) + (copy ? 2 * (size_t)len + 1024 : 0), copy ? r256(len) : 0,
+               false};
+    if (copy) f.in[0] = {0, d_in, (size_t)len};
+    return run_frame(ctx, stream, f, [&](cudaStream_t st) { return core(copy ? ctx->arena : (const u8 *)d_in, st); });
+}
+
 static int check_len(const void *in, long len, void *out)
 {
     if (!in || !out || len <= 0) return BWTS_B200_EINVAL;
@@ -1444,28 +1480,9 @@ static int run_device(bwts_b200_ctx *ctx, int op, const void *d_in, long len, vo
     int rc = check_len(d_in, len, d_out);
     if (!rc) rc = check_primary(op, len, primary);
     if (rc) return rc;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    apply_device_limits();
-    ctx->io_in = nullptr;
-    if ((uintptr_t)d_in & 15) {
-        // the text kernels read 16-byte vectors: an input that is not 16-byte aligned (a slice of a
-        // larger buffer) is first copied to the bottom of the workspace
-        rc = arena_reserve(ctx, workspace_bytes((size_t)len) + 2 * (size_t)len + 1024);
-        if (rc) return rc;
-        ctx->io_bytes = ((size_t)len + 255) & ~(size_t)255;
-        CK(cudaMemcpyAsync(ctx->arena, d_in, (size_t)len, cudaMemcpyDeviceToDevice, st));
-        d_in = ctx->arena;
-        ctx->io_in = ctx->arena;  // tells the cores to skip the I/O region of the arena
-    }
-    stats_begin(ctx, len, op_direction(op), st);
-    rc = run_core(ctx, op, (const u8 *)d_in, (u32)len, (u8 *)d_out, primary, st);
-    ctx->io_in = nullptr;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
-    return 0;
+    return run_text_device(ctx, d_in, len, op_direction(op), stream, [&](const u8 *d_text, cudaStream_t st) {
+        return run_core(ctx, op, d_text, (u32)len, (u8 *)d_out, primary, st);
+    });
 }
 
 extern "C" int bwts_b200_forward_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_out, void *stream)
@@ -1501,21 +1518,22 @@ extern "C" int bwts_b200_divbwt_inverse_device(bwts_b200_ctx *ctx, const void *d
 static std::mutex g_dev_mutex[MAX_DEV];
 static bwts_b200_ctx *g_dev_ctx[MAX_DEV];
 
-// host <-> device copies of the host-buffer entry points: pinned buffers go as one async copy,
-// pageable ones (the tools' mmap'ed input, map_file.c, and malloc'ed output) through the context's
-// ring of pinned chunks -- the memcpy into chunk c+1 runs while chunk c is on the bus, where a
-// pageable cudaMemcpy stages serially inside the driver.  Defined behind PinnedRing.
-static int stage_h2d(bwts_b200_ctx *ctx, u8 *d_dst, const u8 *src, size_t len, cudaStream_t st);
-static int stage_d2h(bwts_b200_ctx *ctx, u8 *dst, const u8 *d_src, size_t len, cudaStream_t st);
-
-// The per-device context behind the one-call entry points and the block dealer: nobody can ask it for
-// statistics, so it records no per-launch events (two cudaEventRecord per kernel are a quarter of a
-// small transform's time: ~120 launches for a 1 MiB input).  BWTS_B200_PROFILE=1 switches them back on.
-static bwts_b200_ctx *create_default_ctx(int device)
+// The per-device context behind the one-call entry points and the block dealer, created on first use and returned
+// with the device's mutex held in lock.  Nobody can ask it for statistics, so it records no per-launch events (two
+// cudaEventRecord per kernel are a quarter of a small transform's time: ~120 launches for a 1 MiB input).
+// BWTS_B200_PROFILE=1 switches them back on.
+static int default_ctx(int device, std::unique_lock<std::mutex> &lock, bwts_b200_ctx *&ctx)
 {
-    bwts_b200_ctx *ctx = bwts_b200_create(device);
-    if (ctx && !getenv("BWTS_B200_PROFILE") && !getenv("BWTS_B200_TRACE")) ctx->profile = false;
-    return ctx;
+    const int ndev = bwts_b200_device_count();
+    if (ndev == 0) return BWTS_B200_ENODEV;
+    if (device < 0 || device >= ndev || device >= MAX_DEV) return BWTS_B200_EINVAL;
+    lock = std::unique_lock<std::mutex>(g_dev_mutex[device]);
+    if (!g_dev_ctx[device]) {
+        g_dev_ctx[device] = bwts_b200_create(device);
+        if (g_dev_ctx[device] && !getenv("BWTS_B200_PROFILE") && !getenv("BWTS_B200_TRACE")) g_dev_ctx[device]->profile = false;
+    }
+    ctx = g_dev_ctx[device];
+    return ctx ? 0 : BWTS_B200_ENODEV;
 }
 
 static int run_host(bwts_b200_ctx *ctx, int op, const unsigned char *in, long len, unsigned char *out,
@@ -1525,32 +1543,14 @@ static int run_host(bwts_b200_ctx *ctx, int op, const unsigned char *in, long le
     int rc = check_len(in, len, out);
     if (!rc) rc = check_primary(op, len, primary);
     if (rc) return rc;
-    CK(cudaSetDevice(ctx->device));
-    // workspace first (it may have to be re-allocated), then the two I/O buffers in its first bytes
-    rc = arena_reserve(ctx, workspace_bytes((size_t)len) + 2 * (size_t)len + 1024);
-    if (rc) return rc;
-    ctx->io_bytes = ((size_t)len + 255) & ~(size_t)255;
-    ctx->io_in = nullptr;
-    u8 *d_in = ctx->arena, *d_out = ctx->arena + ctx->io_bytes;
-    cudaStream_t st = ctx->own_stream;
-    apply_device_limits();
-    CK(cudaEventRecord(ctx->ev_io0, st));
-    rc = stage_h2d(ctx, d_in, in, (size_t)len, st);
-    if (rc) return rc;
-    ctx->io_in = d_in;  // tells the cores to skip the I/O region of the arena
-    stats_begin(ctx, len, op_direction(op), st);
-    rc = run_core(ctx, op, d_in, (u32)len, d_out, primary, st);
-    ctx->io_in = nullptr;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    rc = stage_d2h(ctx, out, d_out, (size_t)len, st);
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev_io1, st));
-    CK(cudaStreamSynchronize(st));
-    float t = 0;
-    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
-    if (cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
-    return 0;
+    // the input and the output in front of the workspace
+    const size_t io = r256((size_t)len);
+    Frame f = {len, op_direction(op), workspace_bytes((size_t)len) + 2 * (size_t)len + 1024, 2 * io, true};
+    f.in[0] = {0, in, (size_t)len};
+    f.out[0] = {io, out, (size_t)len};
+    return run_frame(ctx, nullptr, f, [&](cudaStream_t st) {
+        return run_core(ctx, op, ctx->arena, (u32)len, ctx->arena + io, primary, st);
+    });
 }
 
 extern "C" int bwts_b200_forward_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, unsigned char *out)
@@ -1589,14 +1589,10 @@ static int with_default_ctx(int device, int op, const unsigned char *in, long le
 {
     int rc = check_len(in, len, out);
     if (!rc) rc = check_primary(op, len, primary);
-    if (rc) return rc;
-    const int ndev = bwts_b200_device_count();
-    if (ndev == 0) return BWTS_B200_ENODEV;
-    if (device < 0 || device >= ndev || device >= MAX_DEV) return BWTS_B200_EINVAL;
-    std::lock_guard<std::mutex> lock(g_dev_mutex[device]);
-    if (!g_dev_ctx[device]) g_dev_ctx[device] = create_default_ctx(device);
-    if (!g_dev_ctx[device]) return BWTS_B200_ENODEV;
-    return run_host(g_dev_ctx[device], op, in, len, out, primary);
+    std::unique_lock<std::mutex> lock;
+    bwts_b200_ctx *ctx = nullptr;
+    if (!rc) rc = default_ctx(device, lock, ctx);
+    return rc ? rc : run_host(ctx, op, in, len, out, primary);
 }
 
 extern "C" int bwts_b200_forward(const unsigned char *in, long len, unsigned char *out, int device)
@@ -1790,12 +1786,10 @@ static int run_blocks_on_device(int op, const u8 *in, long len, long block_len, 
     std::vector<long> mine;
     for (long b = first; b < nblocks; b += stride) mine.push_back(b);
     if (mine.empty()) return 0;
-    if (dev >= MAX_DEV) return BWTS_B200_EINVAL;
     // the device's cached context (and its workspace) serves all blocks of this call
-    std::lock_guard<std::mutex> lock(g_dev_mutex[dev]);
-    if (!g_dev_ctx[dev]) g_dev_ctx[dev] = create_default_ctx(dev);
-    bwts_b200_ctx *ctx = g_dev_ctx[dev];
-    if (!ctx) return BWTS_B200_ENODEV;
+    std::unique_lock<std::mutex> lock;
+    bwts_b200_ctx *ctx = nullptr;
+    if (const int rc = default_ctx(dev, lock, ctx)) return rc;
     if (cudaSetDevice(dev) != cudaSuccess) return BWTS_B200_ECUDA;
     auto blk_off = [&](long b) { return b * block_len; };
     auto blk_len = [&](long b) { return (blk_off(b) + block_len <= len) ? block_len : len - blk_off(b); };
@@ -1997,64 +1991,25 @@ static int run_sa_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d
     int rc = check_sa_args(d_in, len, d_sa, d_lcp, want_lcp);
     if (rc) return rc;
     if (((uintptr_t)d_sa & 3) || ((uintptr_t)d_lcp & 3)) return BWTS_B200_EINVAL;
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    apply_device_limits();
-    ctx->io_in = nullptr;
-    if ((uintptr_t)d_in & 15) {  // as run_device: an unaligned slice is copied to the bottom of the workspace
-        rc = arena_reserve(ctx, workspace_bytes((size_t)len) + 2 * (size_t)len + 1024);
-        if (rc) return rc;
-        ctx->io_bytes = ((size_t)len + 255) & ~(size_t)255;
-        CK(cudaMemcpyAsync(ctx->arena, d_in, (size_t)len, cudaMemcpyDeviceToDevice, st));
-        d_in = ctx->arena;
-        ctx->io_in = ctx->arena;
-    }
-    stats_begin(ctx, len, 0, st);
-    rc = forward_core(ctx, (const u8 *)d_in, (u32)len, nullptr, (i32 *)d_sa, FWD_SA, st, nullptr,
-                      want_lcp ? (i32 *)d_lcp : nullptr);
-    ctx->io_in = nullptr;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
-    return 0;
+    return run_text_device(ctx, d_in, len, 0, stream, [&](const u8 *d_text, cudaStream_t st) {
+        return forward_core(ctx, d_text, (u32)len, nullptr, (i32 *)d_sa, FWD_SA, st, nullptr, want_lcp ? (i32 *)d_lcp : nullptr);
+    });
 }
 
 // host buffers: the text, the suffix array and the LCP array (if wanted) in the I/O region in front of the
 // workspace, 1 + 4 + 4 bytes per input byte; arguments already checked
 static int run_sa_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa, int *lcp)
 {
-    CK(cudaSetDevice(ctx->device));
-    const size_t io = ((size_t)len + 255) & ~(size_t)255;
-    const size_t sa_bytes = ((size_t)len * 4 + 255) & ~(size_t)255;
+    const size_t io = r256((size_t)len), sa_bytes = r256((size_t)len * 4);
     const size_t out_bytes = lcp ? 2 * sa_bytes : sa_bytes;
-    int rc = arena_reserve(ctx, workspace_bytes((size_t)len) + io + out_bytes + 1024);
-    if (rc) return rc;
-    // forward_core skips 2 * io_bytes of the arena: the I/O region
-    ctx->io_bytes = ((io + out_bytes + 1) / 2 + 255) & ~(size_t)255;
-    ctx->io_in = nullptr;
-    u8 *d_in = ctx->arena;
-    i32 *d_sa = (i32 *)(ctx->arena + io), *d_lcp = lcp ? (i32 *)(ctx->arena + io + sa_bytes) : nullptr;
-    cudaStream_t st = ctx->own_stream;
-    apply_device_limits();
-    CK(cudaEventRecord(ctx->ev_io0, st));
-    rc = stage_h2d(ctx, d_in, in, (size_t)len, st);
-    if (rc) return rc;
-    ctx->io_in = d_in;
-    stats_begin(ctx, len, 0, st);
-    rc = forward_core(ctx, d_in, (u32)len, nullptr, d_sa, FWD_SA, st, nullptr, d_lcp);
-    ctx->io_in = nullptr;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    rc = stage_d2h(ctx, (u8 *)sa, (const u8 *)d_sa, (size_t)len * 4, st);
-    if (!rc && lcp) rc = stage_d2h(ctx, (u8 *)lcp, (const u8 *)d_lcp, (size_t)len * 4, st);
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev_io1, st));
-    CK(cudaStreamSynchronize(st));
-    float t = 0;
-    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
-    if (cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
-    return 0;
+    Frame f = {len, 0, workspace_bytes((size_t)len) + io + out_bytes + 1024, io + out_bytes, true};
+    f.in[0] = {0, in, (size_t)len};
+    f.out[0] = {io, sa, (size_t)len * 4};
+    if (lcp) f.out[1] = {io + sa_bytes, lcp, (size_t)len * 4};
+    return run_frame(ctx, nullptr, f, [&](cudaStream_t st) {
+        return forward_core(ctx, ctx->arena, (u32)len, nullptr, (i32 *)(ctx->arena + io), FWD_SA, st, nullptr,
+                            lcp ? (i32 *)(ctx->arena + io + sa_bytes) : nullptr);
+    });
 }
 
 extern "C" int bwts_b200_sa_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *sa)
@@ -2080,29 +2035,25 @@ extern "C" int bwts_b200_sa_lcp_device(bwts_b200_ctx *ctx, const void *d_in, lon
 }
 
 // the one-call forms, on the per-device context of the other one-call functions; n == 0 returns 0
-static int sa_default_ctx(const unsigned char *T, int *SA, int *LCP, int n, int device)
-{
-    const int ndev = bwts_b200_device_count();
-    if (ndev == 0) return BWTS_B200_ENODEV;
-    if (device < 0 || device >= ndev || device >= MAX_DEV) return BWTS_B200_EINVAL;
-    std::lock_guard<std::mutex> lock(g_dev_mutex[device]);
-    if (!g_dev_ctx[device]) g_dev_ctx[device] = create_default_ctx(device);
-    if (!g_dev_ctx[device]) return BWTS_B200_ENODEV;
-    return run_sa_host(g_dev_ctx[device], T, n, SA, LCP);
-}
 // libdivsufsort's seam
 extern "C" int bwts_b200_divsufsort(const unsigned char *T, int *SA, int n, int device)
 {
     if (!T || !SA || n < 0) return BWTS_B200_EINVAL;
     if (n == 0) return 0;
-    return sa_default_ctx(T, SA, nullptr, n, device);
+    std::unique_lock<std::mutex> lock;
+    bwts_b200_ctx *ctx = nullptr;
+    const int rc = default_ctx(device, lock, ctx);
+    return rc ? rc : run_sa_host(ctx, T, n, SA, nullptr);
 }
 extern "C" int bwts_b200_sa_lcp(const unsigned char *T, int *SA, int *LCP, int n, int device)
 {
     if (!T || !SA || !LCP || n < 0) return BWTS_B200_EINVAL;
     if (n == 0) return 0;
-    const int rc = check_sa_args(T, n, SA, LCP, true);
-    return rc ? rc : sa_default_ctx(T, SA, LCP, n, device);
+    int rc = check_sa_args(T, n, SA, LCP, true);
+    std::unique_lock<std::mutex> lock;
+    bwts_b200_ctx *ctx = nullptr;
+    if (!rc) rc = default_ctx(device, lock, ctx);
+    return rc ? rc : run_sa_host(ctx, T, n, SA, LCP);
 }
 
 // ---- longest-previous-factor array and LZ77 parse ---------------------------------------------------------------
@@ -2127,27 +2078,9 @@ static int check_lz_args(const bwts_b200_ctx *ctx, const void *in, long len, con
 
 static int run_lz_device(bwts_b200_ctx *ctx, const void *d_in, long len, LzOut *lz, void *stream)
 {
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    apply_device_limits();
-    ctx->io_in = nullptr;
-    int rc;
-    if ((uintptr_t)d_in & 15) {  // as run_device: an unaligned slice is copied to the bottom of the workspace
-        rc = arena_reserve(ctx, workspace_bytes((size_t)len) + 2 * (size_t)len + 1024);
-        if (rc) return rc;
-        ctx->io_bytes = ((size_t)len + 255) & ~(size_t)255;
-        CK(cudaMemcpyAsync(ctx->arena, d_in, (size_t)len, cudaMemcpyDeviceToDevice, st));
-        d_in = ctx->arena;
-        ctx->io_in = ctx->arena;
-    }
-    stats_begin(ctx, len, 0, st);
-    rc = forward_core(ctx, (const u8 *)d_in, (u32)len, nullptr, nullptr, FWD_LZ, st, nullptr, nullptr, lz);
-    ctx->io_in = nullptr;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
-    return 0;
+    return run_text_device(ctx, d_in, len, 0, stream, [&](const u8 *d_text, cudaStream_t st) {
+        return forward_core(ctx, d_text, (u32)len, nullptr, nullptr, FWD_LZ, st, nullptr, nullptr, lz);
+    });
 }
 
 // host buffers: the text and LPF + PREV, or up to n factor pairs, in the I/O region in front of the workspace,
@@ -2155,43 +2088,22 @@ static int run_lz_device(bwts_b200_ctx *ctx, const void *d_in, long len, LzOut *
 static int run_lz_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *lpf, int *prev, int *factors,
                        long cap, long *z)
 {
-    CK(cudaSetDevice(ctx->device));
-    const size_t io = ((size_t)len + 255) & ~(size_t)255;
-    const size_t w_bytes = ((size_t)len * 4 + 255) & ~(size_t)255;
-    int rc = arena_reserve(ctx, workspace_bytes((size_t)len) + io + 2 * w_bytes + 1024);
-    if (rc) return rc;
-    ctx->io_bytes = ((io + 2 * w_bytes + 1) / 2 + 255) & ~(size_t)255;  // forward_core skips 2 * io_bytes
-    ctx->io_in = nullptr;
-    u8 *d_in = ctx->arena;
-    i32 *d_a = (i32 *)(ctx->arena + io), *d_b = (i32 *)(ctx->arena + io + w_bytes);
-    LzOut o;
-    if (lpf) { o.lpf = d_a; o.prev = d_b; }
-    else { o.factors = d_a; o.cap = cap; }
-    cudaStream_t st = ctx->own_stream;
-    apply_device_limits();
-    CK(cudaEventRecord(ctx->ev_io0, st));
-    rc = stage_h2d(ctx, d_in, in, (size_t)len, st);
-    if (rc) return rc;
-    ctx->io_in = d_in;
-    stats_begin(ctx, len, 0, st);
-    rc = forward_core(ctx, d_in, (u32)len, nullptr, nullptr, FWD_LZ, st, nullptr, nullptr, &o);
-    ctx->io_in = nullptr;
-    if (z && o.z >= 0) *z = o.z;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
+    const size_t io = r256((size_t)len), w_bytes = r256((size_t)len * 4);
+    Frame f = {len, 0, workspace_bytes((size_t)len) + io + 2 * w_bytes + 1024, io + 2 * w_bytes, true};
+    f.in[0] = {0, in, (size_t)len};
     if (lpf) {
-        rc = stage_d2h(ctx, (u8 *)lpf, (const u8 *)d_a, (size_t)len * 4, st);
-        if (!rc) rc = stage_d2h(ctx, (u8 *)prev, (const u8 *)d_b, (size_t)len * 4, st);
-    } else if (o.z > 0) {
-        rc = stage_d2h(ctx, (u8 *)factors, (const u8 *)d_a, (size_t)o.z * 8, st);
+        f.out[0] = {io, lpf, (size_t)len * 4};
+        f.out[1] = {io + w_bytes, prev, (size_t)len * 4};
     }
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev_io1, st));
-    CK(cudaStreamSynchronize(st));
-    float t = 0;
-    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
-    if (cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
-    return 0;
+    return run_frame(ctx, nullptr, f, [&](cudaStream_t st) {
+        LzOut o;
+        if (lpf) { o.lpf = (i32 *)(ctx->arena + io); o.prev = (i32 *)(ctx->arena + io + w_bytes); }
+        else { o.factors = (i32 *)(ctx->arena + io); o.cap = cap; }
+        const int rc = forward_core(ctx, ctx->arena, (u32)len, nullptr, nullptr, FWD_LZ, st, nullptr, nullptr, &o);
+        if (z && o.z >= 0) *z = o.z;
+        if (!lpf && o.z > 0) f.out[0] = {io, factors, (size_t)o.z * 8};
+        return rc;
+    });
 }
 
 extern "C" int bwts_b200_lpf_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int *lpf, int *prev)
@@ -2240,7 +2152,6 @@ struct bwts_b200_fm {
     FmView v;
 };
 
-static size_t r256(size_t b) { return (b + 255) & ~(size_t)255; }
 static size_t fm_layout(u32 n, u32 sg, u32 sample, size_t off[9])
 {
     const size_t sz[8] = {(size_t)n, 4ull * sg * ((n >> 16) + 1), 2ull * sg * ((n >> 8) + 1), 4ull * ((n + 31ull) / 32),
@@ -2253,23 +2164,21 @@ static bool fm_sample_ok(int sample) { return sample >= 1 && sample <= 1024 && (
 
 // The build: the byte histogram (C, the symbol map, sg, and so the index's size), the FWD_FM sort -- divbwt bytes
 // into the index's U, the suffix array into the I/O region -- then the checkpoints, marks, directory and samples.
-// d_text lies at the bottom of the arena, in an I/O region of io bytes reserved by the caller.
-static int fm_build_core(bwts_b200_ctx *ctx, const u8 *d_text, u32 n, u32 sample, size_t io, bwts_b200_fm **out,
-                         cudaStream_t st)
+// The text lies at the bottom of the arena, in the I/O region (fm_build_io) the caller reserved.  *out is set once
+// every launch is queued.
+static int fm_build_core(bwts_b200_ctx *ctx, u32 n, u32 sample, bwts_b200_fm **out, cudaStream_t st)
 {
     const u32 nb = (n >> 8) + 1, ns = (n >> 16) + 1;
     const u32 nt = cdiv(nb, SC_TILE);
+    const u8 *d_text = ctx->arena;
     u8 *p = ctx->arena + r256(n);
     i32 *d_sa = (i32 *)p;            p += r256(4ull * n);
     u32 *dircnt = (u32 *)p;          p += r256(4ull * nb);
     u32 *tiles = (u32 *)p;           p += r256(4ull * (nt + 1));
     u32 *hist = (u32 *)p;            p += 1024;
     u8 *syms = p;                    p += 256;
-    if ((size_t)(p - ctx->arena) > io) return BWTS_B200_EINTERNAL;
-    ctx->io_bytes = (io + 1) / 2;    // forward_core skips 2 io_bytes (+ up to 511) of the arena
-    ctx->io_in = (u8 *)d_text;
+    if ((size_t)(p - ctx->arena) > ctx->io_end) return BWTS_B200_EINTERNAL;
 
-    stats_begin(ctx, n, 0, st);
     ctx->phase = 3;
     CK(cudaMemsetAsync(hist, 0, 1024, st));
     LAUNCH(KC_EMIT, 1.0 * n, k_fm_hist, min(cdiv(n, 256), (u32)ctx->sm_count * 8), 256, d_text, n, hist);
@@ -2327,10 +2236,7 @@ static int fm_build_core(bwts_b200_ctx *ctx, const u8 *d_text, u32 n, u32 sample
                samples);
         return 0;
     }();
-    ctx->io_in = nullptr;
     if (rc) return fail(rc);
-    stats_end(ctx, st);
-    FCK(cudaGetLastError());
 #undef FCK
     fm->v.U = U; fm->v.S = S; fm->v.B = B; fm->v.marks = marks; fm->v.dir = dir; fm->v.samples = samples;
     fm->v.C = dC; fm->v.map = dmap;
@@ -2354,43 +2260,28 @@ static int fm_build_args(bwts_b200_ctx *ctx, const void *in, long len, int sampl
     if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
     return 0;
 }
-static int fm_build(bwts_b200_ctx *ctx, const void *src, long len, int sample, bwts_b200_fm **fm, cudaStream_t st,
-                    bool host)
+// the device form copies the text next to the suffix array whatever its alignment: one n-byte copy
+static int fm_build(bwts_b200_ctx *ctx, const void *src, long len, int sample, bwts_b200_fm **fm, void *stream, bool host)
 {
-    CK(cudaSetDevice(ctx->device));
     const size_t io = fm_build_io((size_t)len);
-    int rc = arena_reserve(ctx, workspace_bytes((size_t)len) + io + 1024);
-    if (rc) return rc;
-    apply_device_limits();
-    ctx->io_in = nullptr;
-    if (host) {
-        CK(cudaEventRecord(ctx->ev_io0, st));
-        rc = stage_h2d(ctx, ctx->arena, (const u8 *)src, (size_t)len, st);
-        if (rc) return rc;
-    } else {  // the text is copied next to the suffix array whatever its alignment: one n-byte copy
-        CK(cudaMemcpyAsync(ctx->arena, src, (size_t)len, cudaMemcpyDeviceToDevice, st));
-    }
-    rc = fm_build_core(ctx, ctx->arena, (u32)len, (u32)sample, io, fm, st);
-    ctx->io_in = nullptr;
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    if (host) {
-        float t = 0;
-        if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
-    }
-    return 0;
+    Frame f = {len, 0, workspace_bytes((size_t)len) + io + 1024, io, host};
+    f.in[0] = {0, src, (size_t)len};
+    const int rc = run_frame(ctx, stream, f, [&](cudaStream_t st) { return fm_build_core(ctx, (u32)len, (u32)sample, fm, st); });
+    if (rc && *fm) { bwts_b200_fm_free(*fm); *fm = nullptr; }
+    return rc;
 }
 
 extern "C" int bwts_b200_fm_build_host(bwts_b200_ctx *ctx, const unsigned char *in, long len, int sample,
                                        bwts_b200_fm **fm)
 {
     const int rc = fm_build_args(ctx, in, len, sample, fm);
-    return rc ? rc : fm_build(ctx, in, len, sample, fm, ctx->own_stream, true);
+    return rc ? rc : fm_build(ctx, in, len, sample, fm, nullptr, true);
 }
 extern "C" int bwts_b200_fm_build_device(bwts_b200_ctx *ctx, const void *d_in, long len, int sample, bwts_b200_fm **fm,
                                          void *stream)
 {
     const int rc = fm_build_args(ctx, d_in, len, sample, fm);
-    return rc ? rc : fm_build(ctx, d_in, len, sample, fm, stream ? (cudaStream_t)stream : ctx->own_stream, false);
+    return rc ? rc : fm_build(ctx, d_in, len, sample, fm, stream, false);
 }
 extern "C" void bwts_b200_fm_free(bwts_b200_fm *fm)
 {
@@ -2406,23 +2297,18 @@ extern "C" long bwts_b200_fm_bytes(const bwts_b200_fm *fm)
 
 // Queries run on the context's arena: 64 bytes of counters at its start, then (host forms) the staged arrays.
 // direction 1, phase 2 ("Walk sublists"): the searches and walks in class inv_walk, the checks and the offsets
-// scan in class inv_scan.
-static int fm_query_ctx(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, size_t arena_bytes, cudaStream_t st)
+// scan in class inv_scan.  f: the staged arrays and the arena they need.
+template <typename Core>
+static int run_fm_query(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, void *stream, Frame &f, Core &&core)
 {
     if (ctx->device != fm->device) return BWTS_B200_EINVAL;
-    CK(cudaSetDevice(ctx->device));
-    int rc = arena_reserve(ctx, max(arena_bytes, (size_t)4096));
-    if (rc) return rc;
-    stats_begin(ctx, fm->n, 1, st);
-    ctx->phase = 2;
-    return 0;
-}
-static int fm_query_end(bwts_b200_ctx *ctx, cudaStream_t st)
-{
-    stats_end(ctx, st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
-    return 0;
+    f.len = fm->n;
+    f.direction = 1;
+    f.arena = max(f.arena, (size_t)4096);
+    return run_frame(ctx, stream, f, [&](cudaStream_t st) {
+        ctx->phase = 2;
+        return core(st);
+    });
 }
 static u64 h_small_u64(const bwts_b200_ctx *ctx, int w) { return (u64)ctx->h_small[w] | ((u64)ctx->h_small[w + 1] << 32); }
 
@@ -2465,19 +2351,14 @@ extern "C" int bwts_b200_fm_count_host(bwts_b200_ctx *ctx, const bwts_b200_fm *f
     if (!fm_off_ok(off, npat, pat_len)) return BWTS_B200_EINVAL;
     if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
     const size_t a_pat = 256, a_off = a_pat + r256((size_t)pat_len), a_range = a_off + r256(8 * ((size_t)npat + 1));
-    cudaStream_t st = ctx->own_stream;
-    int rc = fm_query_ctx(ctx, fm, a_range + r256(8 * (size_t)npat), st);
-    if (rc) return rc;
-    u8 *d_pat = ctx->arena + a_pat;
-    long long *d_off = (long long *)(ctx->arena + a_off);
-    i32 *d_range = (i32 *)(ctx->arena + a_range);
-    if (pat_len) { rc = stage_h2d(ctx, d_pat, pat, (size_t)pat_len, st); if (rc) return rc; }
-    rc = stage_h2d(ctx, (u8 *)d_off, (const u8 *)off, 8 * ((size_t)npat + 1), st);
-    if (!rc) rc = fm_count_core(ctx, fm, d_pat, pat_len, d_off, npat, d_range, total, false, st);
-    if (!rc) rc = stage_d2h(ctx, (u8 *)range, (const u8 *)d_range, 8 * (size_t)npat, st);
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    CK(cudaStreamSynchronize(st));
-    return fm_query_end(ctx, st);
+    Frame f = {0, 0, a_range + r256(8 * (size_t)npat), 0, true};
+    f.in[0] = {a_pat, pat, (size_t)pat_len};
+    f.in[1] = {a_off, off, 8 * ((size_t)npat + 1)};
+    f.out[0] = {a_range, range, 8 * (size_t)npat};
+    return run_fm_query(ctx, fm, nullptr, f, [&](cudaStream_t st) {
+        return fm_count_core(ctx, fm, ctx->arena + a_pat, pat_len, (const long long *)(ctx->arena + a_off), npat,
+                             (i32 *)(ctx->arena + a_range), total, false, st);
+    });
 }
 extern "C" int bwts_b200_fm_count_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_pat, long pat_len,
                                          const void *d_off, long npat, void *d_range, long *total, void *stream)
@@ -2487,12 +2368,11 @@ extern "C" int bwts_b200_fm_count_device(bwts_b200_ctx *ctx, const bwts_b200_fm 
     if (!d_off || !d_range || (pat_len > 0 && !d_pat)) return BWTS_B200_EINVAL;
     if (((uintptr_t)d_off & 7) || ((uintptr_t)d_range & 3)) return BWTS_B200_EINVAL;
     if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    int rc = fm_query_ctx(ctx, fm, 4096, st);
-    if (!rc) rc = fm_count_core(ctx, fm, (const u8 *)d_pat, pat_len, (const long long *)d_off, npat, (i32 *)d_range, total,
-                                true, st);
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    return fm_query_end(ctx, st);
+    Frame f = {0, 0, 4096, 0, false};
+    return run_fm_query(ctx, fm, stream, f, [&](cudaStream_t st) {
+        return fm_count_core(ctx, fm, (const u8 *)d_pat, pat_len, (const long long *)d_off, npat, (i32 *)d_range, total,
+                             true, st);
+    });
 }
 
 // offsets of the ranges at arena + 256 (nrange + 1 u64); a bad range or a total above cap is EINVAL, nothing written
@@ -2534,16 +2414,12 @@ extern "C" int bwts_b200_fm_locate_host(bwts_b200_ctx *ctx, const bwts_b200_fm *
     }
     if (tot > (u64)cap) return BWTS_B200_EINVAL;
     const size_t a_range = 256 + r256(8 * ((size_t)nrange + 1)), a_pos = a_range + r256(8 * (size_t)nrange);
-    cudaStream_t st = ctx->own_stream;
-    int rc = fm_query_ctx(ctx, fm, a_pos + r256(4 * tot), st);
-    if (rc) return rc;
-    i32 *d_range = (i32 *)(ctx->arena + a_range), *d_pos = (i32 *)(ctx->arena + a_pos);
-    rc = stage_h2d(ctx, (u8 *)d_range, (const u8 *)range, 8 * (size_t)nrange, st);
-    if (!rc) rc = fm_locate_core(ctx, fm, d_range, nrange, d_pos, cap, total, st);
-    if (!rc && tot) rc = stage_d2h(ctx, (u8 *)pos, (const u8 *)d_pos, 4 * tot, st);
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    CK(cudaStreamSynchronize(st));
-    return fm_query_end(ctx, st);
+    Frame f = {0, 0, a_pos + r256(4 * tot), 0, true};
+    f.in[0] = {a_range, range, 8 * (size_t)nrange};
+    f.out[0] = {a_pos, pos, 4 * tot};
+    return run_fm_query(ctx, fm, nullptr, f, [&](cudaStream_t st) {
+        return fm_locate_core(ctx, fm, (const i32 *)(ctx->arena + a_range), nrange, (i32 *)(ctx->arena + a_pos), cap, total, st);
+    });
 }
 extern "C" int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_range, long nrange,
                                           void *d_pos, long cap, long *total, void *stream)
@@ -2552,15 +2428,14 @@ extern "C" int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm
     if (nrange == 0) { if (total) *total = 0; return 0; }
     if (!d_range || !d_pos || ((uintptr_t)d_range & 3) || ((uintptr_t)d_pos & 3)) return BWTS_B200_EINVAL;
     if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    int rc = fm_query_ctx(ctx, fm, 256 + r256(8 * ((size_t)nrange + 1)), st);
-    if (!rc) rc = fm_locate_core(ctx, fm, (const i32 *)d_range, nrange, (i32 *)d_pos, cap, total, st);
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    return fm_query_end(ctx, st);
+    Frame f = {0, 0, 256 + r256(8 * ((size_t)nrange + 1)), 0, false};
+    return run_fm_query(ctx, fm, stream, f, [&](cudaStream_t st) {
+        return fm_locate_core(ctx, fm, (const i32 *)d_range, nrange, (i32 *)d_pos, cap, total, st);
+    });
 }
 
 // ---- LZ77 decoding (lzd.cuh) -----------------------------------------------------------------------------------
-// Scratch at the arena's offset `at`: the words v, the starts p (z <= n), the two live lists, 4 n bytes each; the
+// Scratch from the end of the I/O region on: the words v, the starts p (z <= n), the two live lists, 4 n bytes each; the
 // tile sums, 8 per 4096 factors; 256 bytes of counters.
 static size_t lzd_scratch_bytes(size_t n)
 {
@@ -2578,17 +2453,16 @@ static int check_lzd_args(const bwts_b200_ctx *ctx, const void *factors, long z,
 // d_f: z pairs on the device, 4-byte aligned; d_out: n bytes.  The content rules are checked before anything is
 // written to d_out.  Direction 1: the checks and the scan in class inv_scan / phase 0, the chunks in inv_walk / 2,
 // the global rounds in inv_jump / 3, the bytes in inv_place / 4.
-static int lzd_core(bwts_b200_ctx *ctx, const i32 *d_f, u32 z, u8 *d_out, u32 n, size_t at, cudaStream_t st)
+static int lzd_core(bwts_b200_ctx *ctx, const i32 *d_f, u32 z, u8 *d_out, u32 n, cudaStream_t st)
 {
     const u32 nt = cdiv(z, LZD_TILE);
-    u8 *a = ctx->arena + at;
+    u8 *a = ctx->arena + ctx->io_end;
     u32 *v = (u32 *)a;                a += r256(4ull * n);
     u32 *p = (u32 *)a;                a += r256(4ull * n);
     u32 *live[2] = {(u32 *)a, nullptr}; a += r256(4ull * n);
     live[1] = (u32 *)a;               a += r256(4ull * n);
     u64 *tsum = (u64 *)a;             a += r256(8ull * (nt + 1));
     u32 *cnt = (u32 *)a;  // [0] bad, [2..3] the sum of max(1, len_k), [4] / [5] the live counts
-    stats_begin(ctx, n, 1, st);
     ctx->stats.factors = z;
     CK(cudaMemsetAsync(cnt, 0, 32, st));
     // pairs 8 per factor (twice), p 4, tile sums
@@ -2632,27 +2506,14 @@ extern "C" int bwts_b200_lz77_decode_host(bwts_b200_ctx *ctx, const int *factors
     int rc = check_lzd_args(ctx, factors, z, out, len);
     if (rc) return rc;
     if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
-    CK(cudaSetDevice(ctx->device));
     // I/O region: the pairs, then the text
     const size_t fb = r256(8 * (size_t)z), io = fb + r256((size_t)len);
-    rc = arena_reserve(ctx, io + lzd_scratch_bytes((size_t)len));
-    if (rc) return rc;
-    i32 *d_f = (i32 *)ctx->arena;
-    u8 *d_out = ctx->arena + fb;
-    cudaStream_t st = ctx->own_stream;
-    CK(cudaEventRecord(ctx->ev_io0, st));
-    rc = stage_h2d(ctx, (u8 *)d_f, (const u8 *)factors, 8 * (size_t)z, st);
-    if (!rc) rc = lzd_core(ctx, d_f, (u32)z, d_out, (u32)len, io, st);
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    rc = stage_d2h(ctx, out, d_out, (size_t)len, st);
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev_io1, st));
-    CK(cudaStreamSynchronize(st));
-    float t = 0;
-    if (cudaEventElapsedTime(&t, ctx->ev_io0, ctx->ev_begin) == cudaSuccess) ctx->stats.h2d_ms = t;
-    if (cudaEventElapsedTime(&t, ctx->ev_end, ctx->ev_io1) == cudaSuccess) ctx->stats.d2h_ms = t;
-    return 0;
+    Frame f = {len, 1, io + lzd_scratch_bytes((size_t)len), io, true};
+    f.in[0] = {0, factors, 8 * (size_t)z};
+    f.out[0] = {fb, out, (size_t)len};
+    return run_frame(ctx, nullptr, f, [&](cudaStream_t st) {
+        return lzd_core(ctx, (const i32 *)ctx->arena, (u32)z, ctx->arena + fb, (u32)len, st);
+    });
 }
 extern "C" int bwts_b200_lz77_decode_device(bwts_b200_ctx *ctx, const void *d_factors, long z, void *d_out, long len,
                                             void *stream)
@@ -2661,16 +2522,10 @@ extern "C" int bwts_b200_lz77_decode_device(bwts_b200_ctx *ctx, const void *d_fa
     if (rc) return rc;
     if ((uintptr_t)d_factors & 3) return BWTS_B200_EINVAL;
     if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
-    CK(cudaSetDevice(ctx->device));
-    rc = arena_reserve(ctx, lzd_scratch_bytes((size_t)len));
-    if (rc) return rc;
-    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->own_stream;
-    rc = lzd_core(ctx, (const i32 *)d_factors, (u32)z, (u8 *)d_out, (u32)len, 0, st);
-    if (rc) { cudaStreamSynchronize(st); cudaGetLastError(); return rc; }
-    stats_end(ctx, st);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ctx->last_cuda = (int)e; return BWTS_B200_ECUDA; }
-    return 0;
+    Frame f = {len, 1, lzd_scratch_bytes((size_t)len), 0, false};
+    return run_frame(ctx, stream, f, [&](cudaStream_t st) {
+        return lzd_core(ctx, (const i32 *)d_factors, (u32)z, (u8 *)d_out, (u32)len, st);
+    });
 }
 
 // ---- introspection --------------------------------------------------------------------------------------
