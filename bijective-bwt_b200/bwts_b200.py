@@ -35,6 +35,7 @@ EXPORTS = [
     "bwts_b200_sa_host", "bwts_b200_sa_device", "bwts_b200_sa_lcp_host", "bwts_b200_sa_lcp_device", "bwts_b200_sa_lcp",
     "bwts_b200_fm_build_host", "bwts_b200_fm_build_device", "bwts_b200_fm_free", "bwts_b200_fm_bytes",
     "bwts_b200_fm_count_host", "bwts_b200_fm_count_device", "bwts_b200_fm_locate_host", "bwts_b200_fm_locate_device",
+    "bwts_b200_fm_extract_host", "bwts_b200_fm_extract_device",
     "bwts_b200_lpf_host", "bwts_b200_lpf_device", "bwts_b200_lz77_host", "bwts_b200_lz77_device",
     "bwts_b200_lz77_decode_host", "bwts_b200_lz77_decode_device",
 ]
@@ -133,6 +134,8 @@ def lib():
     L.bwts_b200_fm_count_device.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp, vp]
     L.bwts_b200_fm_locate_host.argtypes = [vp, vp, vp, cl, vp, cl, vp]
     L.bwts_b200_fm_locate_device.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp]
+    L.bwts_b200_fm_extract_host.argtypes = [vp, vp, vp, cl, vp, cl, vp]
+    L.bwts_b200_fm_extract_device.argtypes = [vp, vp, vp, cl, vp, cl, vp, vp]
     L.bwts_b200_lpf_host.argtypes = [vp, vp, cl, vp, vp]
     L.bwts_b200_lpf_device.argtypes = [vp, vp, cl, vp, vp, vp]
     L.bwts_b200_lz77_host.argtypes = [vp, vp, cl, vp, cl, ctypes.POINTER(cl)]
@@ -624,6 +627,28 @@ class Context:
         total = ctypes.c_long()
         _check(lib().bwts_b200_fm_locate_device(self._h, fm.handle, d_range, nrange, d_pos, cap, ctypes.byref(total),
                                                 stream), "bwts_b200_fm_locate_device")
+        return total.value
+
+    def fm_extract_host(self, fm, a, b):
+        """-> (bytes uint8, offsets int64 of len(a) + 1): the text's T[a[k]:b[k]] is bytes[offsets[k]:offsets[k+1]]"""
+        a = np.asarray(a, dtype=np.int32)
+        b = np.asarray(b, dtype=np.int32)
+        rng = np.empty(2 * len(a), dtype=np.int32)
+        rng[0::2], rng[1::2] = a, b
+        off = np.zeros(len(a) + 1, dtype=np.int64)
+        np.cumsum(b.astype(np.int64) - a, out=off[1:])
+        cap = max(int(off[-1]), 0)
+        out = np.empty(max(cap, 1), dtype=np.uint8)
+        total = ctypes.c_long()
+        _check(lib().bwts_b200_fm_extract_host(self._h, fm.handle, rng.ctypes.data, len(a), out.ctypes.data, cap,
+                                               ctypes.byref(total)), "bwts_b200_fm_extract_host")
+        return out[:total.value], off
+
+    def fm_extract_device(self, fm, d_range, nrange, d_out, cap, stream=None):
+        """device arrays: int32 ranges (2 nrange, 4-byte aligned), output bytes (cap, any address) -> bytes written"""
+        total = ctypes.c_long()
+        _check(lib().bwts_b200_fm_extract_device(self._h, fm.handle, d_range, nrange, d_out, cap, ctypes.byref(total),
+                                                 stream), "bwts_b200_fm_extract_device")
         return total.value
 
     def stats(self):

@@ -2434,6 +2434,82 @@ extern "C" int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm
     });
 }
 
+// Extract's scratch from the arena's start: 256 bytes of counters, the byte offsets and the segment offsets of the
+// ranges (nrange + 1 u64 each) and the inverse table of the samples (ceil(n / sample) + 1 u32).  A host form stages
+// its ranges and output above fm_extract_scratch.
+static size_t fm_extract_scratch(const bwts_b200_fm *fm, long nrange)
+{
+    const size_t nsamp = ((size_t)fm->n + fm->sample - 1) / fm->sample;
+    return 256 + 2 * r256(8 * ((size_t)nrange + 1)) + r256(4 * (nsamp + 1));
+}
+
+// The checks and byte offsets of k_fm_range_scan, then -- when some range is non-empty -- the segment offsets, the
+// inverse table and the walk; a bad range or a total above cap is EINVAL with nothing written
+static int fm_extract_core(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const i32 *d_range, long nrange, u8 *d_out, long cap,
+                           long *total, cudaStream_t st)
+{
+    u32 *flags = (u32 *)ctx->arena;  // [0] bad range, [1] over cap, [2..3] total, [4..5] bytes read
+    unsigned long long *offs = (unsigned long long *)(ctx->arena + 256);
+    unsigned long long *segs = (unsigned long long *)(ctx->arena + 256 + r256(8 * ((size_t)nrange + 1)));
+    u32 *isa = (u32 *)(ctx->arena + 256 + 2 * r256(8 * ((size_t)nrange + 1)));
+    const u32 sh = (u32)__builtin_ctz(fm->sample), nsamp = cdiv(fm->n, fm->sample), nblk = cdiv(fm->n, FM_BLOCK);
+    CK(cudaMemsetAsync(flags, 0, 64, st));
+    LAUNCH(KC_INV_SCAN, 16.0 * nrange, k_fm_range_scan, 1, 1024, d_range, (u64)nrange, fm->n, (u64)cap, offs, flags);
+    int rc = readback(ctx, st, flags, 16);
+    if (rc) return rc;
+    if (ctx->h_small[0] || ctx->h_small[1]) return BWTS_B200_EINVAL;
+    const u64 tot = h_small_u64(ctx, 2);
+    if (tot) {
+        LAUNCH(KC_INV_SCAN, 16.0 * nrange, k_fm_seg_scan, 1, 1024, d_range, (u64)nrange, sh, segs);
+        // marks and directory, the samples read and the table written
+        LAUNCH(KC_INV_SCAN, fm->n / 8.0 + 4.0 * nblk + 8.0 * nsamp, k_fm_isa, cdiv(nblk, 8), 256, fm->v, sh, isa);
+        // every segment holds at least one output byte, so at most tot half-warps have work
+        LAUNCH(KC_INV_WALK, 1.0 * tot, k_fm_extract, (u32)min((tot + 15) / 16, (u64)ctx->sm_count * 64), 256, fm->v, isa,
+               sh, d_range, (u64)nrange, offs, segs, d_out, (unsigned long long *)(flags + 4));
+        const size_t rec = ctx->recs.size() - 1;
+        rc = readback(ctx, st, flags, 24);
+        if (rc) return rc;
+        ctx->recs[rec].bytes += (double)h_small_u64(ctx, 4);
+    }
+    if (total) *total = (long)tot;
+    return 0;
+}
+
+extern "C" int bwts_b200_fm_extract_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const int *range, long nrange,
+                                         unsigned char *out, long cap, long *total)
+{
+    if (!ctx || !fm || nrange < 0 || cap < 0) return BWTS_B200_EINVAL;
+    if (nrange == 0) { if (total) *total = 0; return 0; }
+    if (!range || !out) return BWTS_B200_EINVAL;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    u64 tot = 0;
+    for (long k = 0; k < nrange; k++) {
+        const int lo = range[2 * k], hi = range[2 * k + 1];
+        if (lo < 0 || lo > hi || (u32)hi > fm->n) return BWTS_B200_EINVAL;
+        tot += (u64)(hi - lo);
+    }
+    if (tot > (u64)cap) return BWTS_B200_EINVAL;
+    const size_t a_range = fm_extract_scratch(fm, nrange), a_out = a_range + r256(8 * (size_t)nrange);
+    Frame f = {0, 0, a_out + r256(tot), 0, true};
+    f.in[0] = {a_range, range, 8 * (size_t)nrange};
+    f.out[0] = {a_out, out, tot};
+    return run_fm_query(ctx, fm, nullptr, f, [&](cudaStream_t st) {
+        return fm_extract_core(ctx, fm, (const i32 *)(ctx->arena + a_range), nrange, ctx->arena + a_out, cap, total, st);
+    });
+}
+extern "C" int bwts_b200_fm_extract_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_range, long nrange,
+                                           void *d_out, long cap, long *total, void *stream)
+{
+    if (!ctx || !fm || nrange < 0 || cap < 0) return BWTS_B200_EINVAL;
+    if (nrange == 0) { if (total) *total = 0; return 0; }
+    if (!d_range || !d_out || ((uintptr_t)d_range & 3)) return BWTS_B200_EINVAL;
+    if (bwts_b200_device_count() == 0) return BWTS_B200_ENODEV;
+    Frame f = {0, 0, fm_extract_scratch(fm, nrange), 0, false};
+    return run_fm_query(ctx, fm, stream, f, [&](cudaStream_t st) {
+        return fm_extract_core(ctx, fm, (const i32 *)d_range, nrange, (u8 *)d_out, cap, total, st);
+    });
+}
+
 // ---- LZ77 decoding (lzd.cuh) -----------------------------------------------------------------------------------
 // Scratch from the end of the I/O region on: the words v, the starts p (z <= n), the two live lists, 4 n bytes each; the
 // tile sums, 8 per 4096 factors; 256 bytes of counters.

@@ -1,4 +1,4 @@
-// fm.cuh -- FM-index over libdivsufsort's BWT: the build kernels after the FWD_FM sort and the count / locate
+// fm.cuh -- FM-index over libdivsufsort's BWT: the build kernels after the FWD_FM sort and the count / locate / extract
 // queries (DESIGN.md section 4.9).
 //
 // Rows are those of T$: row 0 is the end-of-text suffix, row i >= 1 is SA row i-1.  The L column is the divbwt
@@ -308,6 +308,116 @@ __global__ void __launch_bounds__(256) k_fm_locate(FmView f, const i32 *__restri
         if (hl == 0) {
             pos[p] = (i32)(__ldg(f.samples + fm_mark_rank(f.marks, f.dir, r)) + steps);
             rd += 4 + 4 + 32 + 4;
+        }
+    }
+    if (lane == 0 || lane == 16) {
+        if (rd) atomicAdd(cnt, (unsigned long long)rd);
+    }
+}
+
+// ---- extract ---------------------------------------------------------------------------------------------
+// The inverse of the samples, derived per call: isa[v >> sh] = FM row of text position v for every sampled v
+// (sample = 2^sh), and isa[ceil(n / sample)] = 0, the $ row, which is the row of position n.  Segment q of the text
+// is [q << sh, min((q + 1) << sh, n)); it is decoded from the row isa[q + 1] of its end by LF steps, each giving
+// the byte before the current position: T[p - 1] = L[row].
+
+// One warp per 256-row block of the marks: lane l takes rows 8l .. 8l + 7 of the block, its marked rows' ranks
+// follow from dir and a warp scan, and each marked row r with value v = samples[rank] sets isa[v >> sh] = r + 1.
+__global__ void __launch_bounds__(256) k_fm_isa(FmView f, u32 sh, u32 *__restrict__ isa)
+{
+    const u32 b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = lane_id();
+    if (blockIdx.x == 0 && threadIdx.x == 0) isa[(f.n + (1u << sh) - 1) >> sh] = 0;
+    if ((u64)b * FM_BLOCK >= f.n) return;
+    const u32 w = b * 8 + (lane >> 2);
+    const u32 bits = w < (f.n + 31) / 32 ? (__ldg(f.marks + w) >> ((lane & 3) * 8)) & 0xffu : 0u;
+    const u32 c = __popc(bits);
+    u32 rank = __ldg(f.dir + b) + warp_incl_sum(c) - c;
+    for (u32 m = bits; m; m &= m - 1) {
+        const u32 r = b * FM_BLOCK + lane * 8 + (__ffs(m) - 1);
+        isa[__ldg(f.samples + rank++) >> sh] = r + 1;
+    }
+}
+
+static __device__ __forceinline__ u64 fm_warp_incl_u64(u64 v)
+{
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const u64 y = __shfl_up_sync(FULL_MASK, v, o);
+        if (lane_id() >= (u32)o) v += y;
+    }
+    return v;
+}
+
+// One CTA, after k_fm_range_scan accepted the ranges: segs[k] = exclusive 64-bit prefix of the segment counts
+// ceil(b_k / s) - floor(a_k / s) (0 for an empty range), segs[nrange] = the number of segments.
+__global__ void __launch_bounds__(1024) k_fm_seg_scan(const i32 *__restrict__ range, u64 nrange, u32 sh,
+                                                      unsigned long long *__restrict__ segs)
+{
+    __shared__ u64 ws[33];
+    const u32 lane = lane_id(), warp = threadIdx.x >> 5;
+    u64 carry = 0;
+    for (u64 base = 0; base < nrange; base += 1024) {
+        const u64 k = base + threadIdx.x;
+        u64 v = 0;
+        if (k < nrange) {
+            const u32 a = (u32)range[2 * k], b = (u32)range[2 * k + 1];
+            v = a < b ? (u64)(((b - 1) >> sh) - (a >> sh) + 1) : 0u;
+        }
+        const u64 incl = fm_warp_incl_u64(v);
+        if (lane == 31) ws[warp] = incl;
+        __syncthreads();
+        if (warp == 0) {
+            const u64 x = ws[lane], xi = fm_warp_incl_u64(x);
+            ws[lane] = xi - x;
+            if (lane == 31) ws[32] = xi;
+        }
+        __syncthreads();
+        if (k < nrange) segs[k] = carry + ws[warp] + incl - v;
+        carry += ws[32];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) segs[nrange] = carry;
+}
+
+// Extract, one half-warp per segment (grid-stride): the range k with segs[k] <= g < segs[k+1] by binary search,
+// its segment q = a_k / s + g - segs[k], then LF from isa[q + 1] down to position max(a_k, q s); the bytes at
+// positions inside [a_k, b_k) go to out[offs[k] + p - a_k].  A walk stops at position >= 0 before reading row
+// primary, so the $ is never read.  cnt[0] += bytes read.
+__global__ void __launch_bounds__(256) k_fm_extract(FmView f, const u32 *__restrict__ isa, u32 sh,
+                                                    const i32 *__restrict__ range, u64 nrange,
+                                                    const unsigned long long *__restrict__ offs,
+                                                    const unsigned long long *__restrict__ segs, u8 *__restrict__ out,
+                                                    unsigned long long *__restrict__ cnt)
+{
+    __shared__ u32 sC[257];
+    __shared__ u8 smap[256];
+    for (u32 t = threadIdx.x; t < 257; t += 256) sC[t] = f.C[t];
+    smap[threadIdx.x] = f.map[threadIdx.x];
+    __syncthreads();
+    const u32 lane = lane_id(), hl = lane & 15, hmask = lane < 16 ? 0x0000ffffu : 0xffff0000u;
+    const u64 halves = (u64)gridDim.x * 16, nseg = segs[nrange];
+    u64 rd = 0;
+    for (u64 g = (u64)blockIdx.x * 16 + (threadIdx.x >> 4); g < nseg; g += halves) {
+        u64 lo = 0, hi = nrange;  // largest k with segs[k] <= g: the non-empty range after any empty ones
+        while (hi - lo > 1) {
+            const u64 mid = (lo + hi) >> 1;
+            if (segs[mid] <= g) lo = mid; else hi = mid;
+            rd += 8;
+        }
+        const u32 a = (u32)range[2 * lo], b = (u32)range[2 * lo + 1];
+        const u32 q = (a >> sh) + (u32)(g - segs[lo]);
+        const u32 first = max(a, q << sh);
+        const u64 base = offs[lo] - a;  // out[base + p] holds T[p]
+        u32 p = min((q + 1) << sh, f.n);
+        u32 i = __ldg(isa + q + 1);
+        rd += 8 + 8 + 8 + 4;  // segs[k], offs[k], the range, the start row
+        for (;;) {
+            const u32 c = __ldg(f.U + (i - (i > f.primary)));
+            rd += 1;
+            p--;
+            if (hl == 0 && p < b) out[base + p] = (u8)c;
+            if (p == first) break;
+            i = sC[c] + fm_occ(f, sC, smap, c, i, hl, hmask, &rd);
         }
     }
     if (lane == 0 || lane == 16) {

@@ -21,7 +21,7 @@
  *                       additive: the suffix array and the LCP array on the context, device and
  *                       one-call entry points (see the section below).
  *   bwts_b200_fm_*      additive: an FM-index over the divbwt output, counting and locating many
- *                       patterns on the GPU (see the section below).
+ *                       patterns and extracting ranges of the text on the GPU (see the section below).
  *   bwts_b200_lpf_*, bwts_b200_lz77_*
  *                       additive: the longest-previous-factor array and the greedy LZ77 parse,
  *                       from the suffix array and LCP array on the GPU (see the last section).
@@ -307,7 +307,7 @@ int bwts_b200_sa_lcp_host(bwts_b200_ctx *ctx, const unsigned char *in, long len,
 int bwts_b200_sa_lcp_device(bwts_b200_ctx *ctx, const void *d_in, long len, void *d_sa, void *d_lcp, void *stream);
 int bwts_b200_sa_lcp(const unsigned char *T, int *SA, int *LCP, int n, int device);   /* divsufsort-shaped */
 
-/* ---- FM-index: count and locate over libdivsufsort's BWT ----------------------------------- */
+/* ---- FM-index: count, locate and extract over libdivsufsort's BWT ------------------------- */
 /* Bytes compare as unsigned char and the end of text is smaller than every byte (the order of
  * bwts_b200_divsufsort and bwts_b200_sa_*); SA is the suffix array of the text T, n = len,
  * 1 <= len <= BWTS_B200_MAX_LEN.  An index is built once from T and answers batches of patterns.
@@ -369,6 +369,32 @@ int bwts_b200_fm_locate_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const i
                              int *pos, long cap, long *total);
 int bwts_b200_fm_locate_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_range, long nrange,
                                void *d_pos, long cap, long *total, void *stream);
+
+/* Extract: the text back from its index, so a caller need not keep T beside it.  range holds int32 pairs
+ * (a_k, b_k) with 0 <= a_k <= b_k <= n; out = T[a_0..b_0) . T[a_1..b_1) . ..., in range order; ranges may
+ * overlap and repeat.  *total (may be NULL) = the sum of b_k - a_k; out[0 .. cap) must hold it.
+ *     banana       [0,6) -> banana   [1,4) -> ana   [5,6) -> a   [3,3) and [6,6) -> nothing
+ *     mississippi  [2,6) -> ssis
+ *     aaaa         [1,3) -> aa
+ * Arguments as locate: a NULL ctx, fm or array, nrange < 0 or cap < 0 is BWTS_B200_EINVAL; nrange == 0 returns 0
+ * with *total = 0; a bad range or a total above cap is BWTS_B200_EINVAL and nothing is written to out.  The host
+ * form checks the ranges on the host, the device form on the GPU (the validation kernel of locate) before any other
+ * work.  Device ranges must be 4-byte aligned; d_out may lie at any address.  Without a device both calls return
+ * BWTS_B200_ENODEV after the checks that need no index; an index from another device is BWTS_B200_EINVAL.
+ * GPU path (DESIGN.md section 4.9): each call inverts the samples into a table of the rows of the text positions
+ * k * sample, then decodes every segment [k sample, (k+1) sample) that a range touches by at most `sample` LF steps
+ * from the row of its end, one half-warp per segment.  The index is only read, so its size and layout are those
+ * of count and locate, and threads with their own contexts may extract from one index at once.
+ * Device memory, from the context's workspace (which never shrinks): 256 bytes of counters, the byte offsets and the
+ * segment offsets of the ranges (8 (nrange + 1) bytes each) and 4 (ceil(n / sample) + 1) bytes of table, each
+ * rounded up to 256; the host form adds 8 nrange bytes of ranges and the total bytes of output.  Offsets are 64-bit:
+ * a total may exceed 2^32.
+ * Statistics: direction 1, phase 2; the range checks, the scans and the table in class "inv_scan", the walk
+ * (k_fm_extract) in class "inv_walk". */
+int bwts_b200_fm_extract_host(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const int *range, long nrange,
+                              unsigned char *out, long cap, long *total);
+int bwts_b200_fm_extract_device(bwts_b200_ctx *ctx, const bwts_b200_fm *fm, const void *d_range, long nrange,
+                                void *d_out, long cap, long *total, void *stream);
 
 /* ---- longest-previous-factor array and greedy LZ77 parse ------------------------------------ */
 /* Bytes compare as unsigned char and the end of text is smaller than every byte (the order of
